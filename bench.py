@@ -1,7 +1,7 @@
 #!/usr/bin/env python3
 """bench.py -- aligned reads/s through score + pileup + consensus (BASELINE.json metric), one JSON line.
 
-    python bench.py [--gpus N --steps K --warmup W] [--impl reference] [--reads R --alleles A]
+    python bench.py [--gpus N --steps K --warmup W] [--impl reference] [--reads R --alleles A] [--dump-outputs DIR]
 
 Workload (N=1): BASELINE.json configs[1] -- one sample of 10 M x 150 bp reads, K=4 alignments per read (40 M BAM
 records, coordinate-sorted), against the synthetic E. coli + S. aureus + K. pneumoniae schemes (21 loci x 1024
@@ -68,7 +68,12 @@ def parse():
     ap.add_argument("--e2e-plain-pileup", action="store_true", help="`e2e` leg: ship the chosen contigs' pileup records plain instead of as DEFLATE blocks")
     ap.add_argument("--e2e-lanes", type=int, default=3, help="samples in flight in the `e2e` leg (api.SampleLanes); 1, 2 and 3 are always timed and reported beside it")
     ap.add_argument("--max-depth", type=int, default=8000, help="htslib pileup depth cap of the main workload (0 = uncapped; profiling aid)")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None, help="after the timed passes, write what the last one returned (chosen alleles, "
+                    "consensus, holes, SNPs, read counters) as DIR/<name>.npy in float64, to compare two builds output for output")
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    return args
 
 
 ORGS = ("ecoli", "saureus", "kpneumoniae")
@@ -196,6 +201,21 @@ def event_ms(pairs):
     return [a.elapsed_time(b) for a, b in pairs]
 
 
+def dump_outputs(out_dir, result, total_reads, ignored_reads, name_to_tid):
+    """One pass's result ({species: [(contig, consensus, holes, snps)]} in the reference's dict order, totalReads, ignoredReads)
+    as float64 arrays, one entry per chosen locus in that order; every value is an integer well below 2**53, so nothing is rounded."""
+    rows = [(c, s, h, n) for sp in result for (c, s, h, n) in result[sp]]
+    arrays = {"allele": [name_to_tid[c] for c, _s, _h, _n in rows],
+              "consensus_len": [len(s) for _c, s, _h, _n in rows],
+              "consensus": np.frombuffer("".join(s for _c, s, _h, _n in rows).encode("latin-1"), np.uint8),
+              "holes": [h for _c, _s, h, _n in rows],
+              "snps": [n for _c, _s, _h, n in rows],
+              "reads": [total_reads, ignored_reads]}
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), np.asarray(a, dtype=np.float64))
+
+
 # ----------------------------------------------------------------------------------------------------------------
 def cpu_port_run(w, args, threads, steps=1, warmup=0):
     """The oracle's C port (oracle/cpu_path.py over oracle/c) on the host cores over the WHOLE sample `w`: score of every record,
@@ -237,7 +257,9 @@ def run_reference(args):
     dev = "cuda:%d" % int(os.environ.get("LOCAL_RANK", "0")) if torch.cuda.is_available() else "cpu"
     w = cpu_workload(db, args, dev)
     steps = max(1, args.steps)
-    rate, dt, _res, sample, phases = cpu_port_run(w, args, threads, steps=steps, warmup=min(max(args.warmup, 0), 2))
+    rate, dt, res, sample, phases = cpu_port_run(w, args, threads, steps=steps, warmup=min(max(args.warmup, 0), 2))
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, res["result"], int(res["counters"][0]), int(res["counters"][1]), {n: i for i, n in enumerate(db.ref_names())})
     cfg = workload_config(args, 1)
     line = {"impl": "reference", "metric": "aligned reads/s (score+pileup+consensus)", "value": rate, "unit": "records/s", "n_gpus": args.gpus,
             "steps": steps, "warmup": args.warmup, "ms_per_step": dt * 1e3, "higher_is_better": True, "scaling": "weak",
@@ -442,6 +464,8 @@ def main():
     outs_serial = [p.collect() for p in pipes]
     out = outs_serial[0]
     assert outs_serial == results, "results changed between steps"
+    k = (args.steps - 1) % n_samples
+    last = (outs_serial[k], pipes[k].total_reads, pipes[k].ignored_reads)
     serial_ms = e0.elapsed_time(e1) / args.steps
     serial_launches = sum(p.launches for p in pipes)
     # the same serial passes alternating between TWO samples only: both score streams (2 x 121 MB) still exceed the L2 and are streamed from HBM every
@@ -479,10 +503,15 @@ def main():
         lanes.join()
         e1.record()
         barrier()
-        assert lanes.collect() == want, "cohort-mode results differ from the serial pass"
+        outs_lanes = lanes.collect()
+        assert outs_lanes == want, "cohort-mode results differ from the serial pass"
+        k = (args.steps - 1) % args.lanes
+        last = (outs_lanes[k], lanes.pipes[k].total_reads, lanes.pipes[k].ignored_reads)
     if prof:
         torch.cuda.profiler.stop()
     assert out == result, "results changed between steps"
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, *last, index.name_to_tid)
     launches = lanes.launches if lanes is not None else serial_launches
     # per-kernel durations: 20 back-to-back launches of each kernel of the same pass between two CUDA events on the
     # launching stream (events are not graph-capturable; a single launch would carry the event/launch gap)

@@ -1,6 +1,6 @@
 import os, sys
 import numpy as np
-ROOT = "/root/repo"
+ROOT = os.path.dirname(os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 sys.path.insert(0, ROOT); sys.path.insert(0, os.path.join(ROOT, "profiles", "tools"))
 import torch
 sys.argv = sys.argv[:1]

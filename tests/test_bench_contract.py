@@ -5,6 +5,8 @@ import os
 import subprocess
 import sys
 
+import numpy as np
+
 from conftest import ROOT
 
 REQUIRED = {"impl", "metric", "value", "unit", "n_gpus", "steps", "warmup", "ms_per_step", "higher_is_better", "scaling", "vs_baseline", "dtype",
@@ -36,3 +38,27 @@ def test_reference_arm_prints_one_json_line_with_the_contract_keys():
 
 def test_reference_arm_other_ranks_exit_silently():
     assert _run({"RANK": "1", "WORLD_SIZE": "2", "LOCAL_RANK": "1"}).strip() == ""
+
+
+DUMPED = ("allele", "consensus_len", "consensus", "holes", "snps", "reads")
+
+
+def _load_dump(d):
+    assert sorted(os.listdir(d)) == sorted(n + ".npy" for n in DUMPED)
+    out = {n: np.load(os.path.join(d, n + ".npy")) for n in DUMPED}
+    assert all(a.dtype == np.float64 and a.ndim == 1 for a in out.values())
+    assert sum(a.nbytes for a in out.values()) <= 64 << 20
+    return out
+
+
+def test_dump_outputs_is_deterministic_and_self_consistent(tmp_path):
+    a, b = tmp_path / "a", tmp_path / "b"
+    _run(args=("--dump-outputs", str(a)))
+    _run(args=("--steps", "2", "--dump-outputs", str(b)))
+    da, db = _load_dump(a), _load_dump(b)
+    for n in DUMPED:
+        assert np.array_equal(da[n], db[n]), n
+    n_loci = len(da["allele"])
+    assert n_loci > 0 and len(da["holes"]) == len(da["snps"]) == len(da["consensus_len"]) == n_loci
+    assert da["consensus_len"].sum() == len(da["consensus"]) and set(np.unique(da["consensus"]).tolist()) <= set(map(float, b"ACGTNacgtn"))
+    assert da["reads"][0] == 2000 * 4 and 0 <= da["reads"][1] <= da["reads"][0]
