@@ -165,7 +165,8 @@ int mmlst_coverage_dev(const uint32_t* tid, const int16_t* as0, const uint8_t* x
 
 /* ---------------------------------------------------------------------------------------------------------------
  * Stage 2 -- pileup base counts.  Replaces cmseq/cmseq.py:527-548 (+ htslib pileup rules H1-H3 applied at unpack).
- *   chunks[c]: a run of consecutive pileup-stream records of ONE chosen contig; its columns live at
+ *   chunks[c]: a run of consecutive pileup-stream records of ONE chosen contig, of any length (the library's own rule,
+ *   mmlst_chunk_records, gives <= 63 tiles of 512 records); its columns live at
  *   counts[col_base .. col_base+contig_len); plane_delta is added (mod 2^32) to row_off of its records so that a
  *   caller may upload only the chosen contigs' plane ranges.  A base counts as its letter when V=1 and the record
  *   passes as_named >= minscore && xm_named <= max_xm (metaMLST_functions.py:259), else as N.

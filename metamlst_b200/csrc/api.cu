@@ -453,8 +453,6 @@ extern "C" int mmlst_coverage(mmlst_ctx* c, const mmlst_soa* soa, const uint64_t
 }
 
 // ---------------------------------------------------------------------------------------------------------------
-static const uint32_t kMaxChunkRecords = 63 * 512;  // bit-sliced counters hold < 2^10 records per lane (pileup_bitsliced.cu)
-
 // Chunk length (records) for a launch over n_rec records: two chunks per SM (one resident wave of the bit-sliced kernel --
 // every (chunk, column word) pair costs one cross-lane flush, so chunks are as long as a full wave allows), whole
 // 512-record tiles.

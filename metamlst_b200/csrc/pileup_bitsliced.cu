@@ -7,7 +7,8 @@
 // are counted per LOP3 with carry-save adders (Harley-Seal), the same trick as a vertical popcount.
 //
 // Mapping
-//   CTA      : persistent over chunks (<= 63 tiles of one contig); tile = 512 consecutive coordinate-sorted records.
+//   CTA      : persistent over chunks (records of one contig, any length; the library builds <= 63 tiles); tile = 512 consecutive
+//              coordinate-sorted records.
 //              Their plane rows are ONE contiguous global range and their 16-byte records another, so a tile is two
 //              cp.async.bulk (TMA 1-D, SASS UBLKCP) into a double-buffered shared-memory stage, completion on one
 //              mbarrier; thread 0 issues tile t+1 before tile t is counted.  No per-thread global loads at all.
@@ -19,7 +20,8 @@
 //              five 1-bit planes (counted, ok, ok&B0, ok&B1, ok&B0&B1) and a 16-input Harley-Seal block (30 LOP3
 //              per 16 inputs per counter) into private bit-sliced counters ones/twos/fours/eights, the sixteens
 //              plane rippled into 6 upper planes once per tile.
-//   flush    : when the warp's word changes or the chunk ends: bit-sliced add across the 32 lanes (shuffle butterfly
+//   flush    : when the warp's word changes, after 63 tiles on the same word (63 x 16 = 1008 records per lane; one more tile
+//              could reach 1024, which 10 planes cannot hold) or when the chunk ends: bit-sliced add across the 32 lanes (shuffle butterfly
 //              over only as many planes as the tiles accumulated so far can have set), lane i extracts column i,
 //              converts to A/C/G/T/N and issues 5 coalesced RED.ADD.
 #include <stdlib.h>
@@ -32,8 +34,9 @@ constexpr int TR = 512;         // records per tile
 constexpr int NWARP = 8;        // column words in the window
 constexpr int NTHREADS = NWARP * 32;
 constexpr int LOWP = 4;         // ones, twos, fours, eights
-constexpr int UPP = 6;          // 16s .. 512s  => < 1024 records per lane between flushes (63 tiles x 16)
+constexpr int UPP = 6;          // 16s .. 512s  => < 1024 records per lane between flushes: a warp flushes after 63 tiles on one word
 constexpr int NP = LOWP + UPP;  // planes per lane counter
+constexpr uint32_t kMaxAccTiles = ((1u << NP) - 1u) / 16u;   // 63 tiles of 16 records per lane fit the NP planes
 constexpr int NPR = NP + 5;     // planes after the 32-lane reduction
 constexpr uint32_t FULL = 0xffffffffu;
 
@@ -260,7 +263,8 @@ __global__ void __launch_bounds__(NTHREADS, 2) pileup_bitsliced_kernel(const Pil
                 // the word of this window that this warp owns: w == wid (mod NWARP)
                 const int w = wlo + ((int(wid) - wlo) & (NWARP - 1));
                 if (w > whi) continue;
-                if (w != cur_w) {
+                // same word for kMaxAccTiles tiles: flush anyway, the next tile could carry out of the top plane (chunks of any length)
+                if (w != cur_w || acc_tiles == kMaxAccTiles) {
                     if (cur_w != INT_MIN) flush_word(acc, cur_w, ck, a.counts, acc_tiles);
                     acc.clear();
                     cur_w = w;
