@@ -583,8 +583,10 @@ void mmlst_bam_free(mmlst_bam* bam);
  * inflated by the hardware decompression engine (cuMemBatchDecompressAsync, DEFLATE), records are chained, parsed, put in
  * `samtools sort` order, depth-capped and packed by kernels, and the result stays in HBM.
  *   bam / n_bytes : the whole BAM file in HOST memory (page-locked memory from mmlst_pinned_alloc makes the copy one async DMA)
- *   opts          : as mmlst_bam_unpack (n_threads, pinned ignored; check_crc not supported on the device: the engine verifies the
- *                   DEFLATE stream and the ISIZE of every block, not the CRC32)
+ *   opts          : as mmlst_bam_unpack (n_threads, pinned ignored).  The engine verifies the DEFLATE stream and a kernel the ISIZE of
+ *                   every block; check_crc = 1 also checks every non-empty block's CRC32 against its trailer (MMLST_E_BAM, "CRC mismatch
+ *                   in BGZF block k", k counting non-empty blocks as mmlst_bam_unpack does; its time is part of seconds[1]).  With
+ *                   opts == NULL check_crc is 0, unlike mmlst_bam_unpack's default of 1.
  *   stream        : cudaStream_t the work is queued on (NULL = the default stream); the call returns after the last kernel finished
  * Every pointer of mmlst_dev_bam_info_t except contig_start / ref_len / ref_names / header_text is a DEVICE pointer owned by the
  * handle.  MMLST_E_CUDA when the device has no hardware DEFLATE (then use mmlst_bam_unpack).

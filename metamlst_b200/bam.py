@@ -174,12 +174,13 @@ def read_pinned(path: str, pool: Optional[PinnedPool] = None):
 
 
 def ingest_bam(source, device=0, minqual: int = packing.DEFAULT_MINQUAL, max_depth: Optional[int] = packing.DEFAULT_MAX_DEPTH,
-               presorted: bool = False, want_qhash: bool = True, sentinel_nodes: int = 1):
+               presorted: bool = False, want_qhash: bool = True, sentinel_nodes: int = 1, check_crc: bool = False):
     """BAM -> streams.DeviceStreams WITHOUT the sample ever being unpacked on the host: the compressed file crosses PCIe, the
     hardware decompression engine inflates the BGZF blocks, kernels chain / parse / sort / depth-cap / pack the records
     (csrc/ingest.cu).  `source`: a path, or a uint8 torch tensor / numpy array holding the file's bytes (page-locked for an
     asynchronous copy: `read_pinned`).  Same streams, same refusals as `unpack_bam`; raises MmlstError(MMLST_E_CUDA) on a device
-    without hardware DEFLATE."""
+    without hardware DEFLATE.  `check_crc`: also check every BGZF block's CRC32 against its trailer on the device, as `unpack_bam`
+    always does (MmlstError(MMLST_E_BAM) "CRC mismatch in BGZF block k"); without it the DEFLATE stream and ISIZE are still checked."""
     import torch
     from . import streams
     dev = torch.device("cuda", device) if isinstance(device, int) else torch.device(device)
@@ -187,7 +188,8 @@ def ingest_bam(source, device=0, minqual: int = packing.DEFAULT_MINQUAL, max_dep
     addr = data.data_ptr() if hasattr(data, "data_ptr") else data.ctypes.data
     nbytes = int(data.numel() if hasattr(data, "numel") else data.size)
     lib = native.lib()
-    o = UnpackOpts(int(minqual), int(max_depth or 0), int(sentinel_nodes), 0, 1, 1 if presorted else 0, 1 if want_qhash else 0, 0, 0)
+    o = UnpackOpts(int(minqual), int(max_depth or 0), int(sentinel_nodes), 0, 1, 1 if presorted else 0, 1 if want_qhash else 0,
+                  1 if check_crc else 0, 0)
     h = C.c_void_p()
     with torch.cuda.device(dev):
         stream = torch.cuda.current_stream(dev).cuda_stream

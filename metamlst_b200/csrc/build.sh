@@ -8,7 +8,7 @@ SRCS="api.cu select.cu score.cu score_runs.cu coverage.cu pileup_atomic.cu pileu
 OBJS=""
 for s in $SRCS; do
   o="${s%.cu}.o"
-  if [ ! -f "$o" ] || [ "$s" -nt "$o" ] || [ common.cuh -nt "$o" ] || [ pileup.cuh -nt "$o" ] || [ score_runs_kernels.cuh -nt "$o" ] || [ ingest_core.cuh -nt "$o" ] || [ de.h -nt "$o" ] || [ ../../include/mmlst.h -nt "$o" ]; then
+  if [ ! -f "$o" ] || [ "$s" -nt "$o" ] || [ common.cuh -nt "$o" ] || [ pileup.cuh -nt "$o" ] || [ score_runs_kernels.cuh -nt "$o" ] || [ ingest_core.cuh -nt "$o" ] || [ bgzf_crc.cuh -nt "$o" ] || [ de.h -nt "$o" ] || [ ../../include/mmlst.h -nt "$o" ]; then
     $NVCC $FLAGS -c "$s" -o "$o" 2> "${s%.cu}.ptxas.log" || { cat "${s%.cu}.ptxas.log"; exit 1; }
   fi
   OBJS="$OBJS $o"

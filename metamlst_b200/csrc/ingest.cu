@@ -9,6 +9,7 @@
 //   DE     raw DEFLATE of every block by Blackwell's hardware decompression engine: cuMemBatchDecompressAsync,
 //          CU_MEM_DECOMPRESS_ALGORITHM_DEFLATE (measured 132 GB/s of output on B200, byte-identical to zlib:
 //          profiles/r2a_de_probe.json) -- BGZF blocks are independent raw-deflate streams, exactly its batch shape
+//   CRC    opts.check_crc: CRC-32 of every inflated block against its trailer, a CTA per block at a time (bgzf_crc.cuh)
 //   K1     record chain: a BAM record only says where the NEXT one starts.  One thread per BGZF block guesses the first record
 //          boundary at or after its block start (htslib never splits a record across blocks, so the guess is offset 0 there;
 //          otherwise the first offset passing a strict plausibility test) and walks the chain to the block end; the guesses are
@@ -24,6 +25,7 @@
 #include <cuda.h>
 #include <cub/cub.cuh>
 
+#include <algorithm>
 #include <chrono>
 #include <cstdio>
 #include <cstring>
@@ -32,6 +34,7 @@
 #include <string>
 #include <vector>
 
+#include "bgzf_crc.cuh"
 #include "common.cuh"
 #include "de.h"
 #include "ingest_core.cuh"
@@ -209,6 +212,52 @@ __global__ void __launch_bounds__(kT) chain_offsets_kernel(const ChainArgs a, co
 __global__ void __launch_bounds__(kT) check_isize_kernel(const uint32_t* act, const uint32_t* isize, uint32_t n_blocks, unsigned long long* err) {
     const uint32_t b = blockIdx.x * kT + threadIdx.x;
     if (b < n_blocks && act[b] != isize[b]) report(err, b, E_CHAIN);
+}
+
+// ---- BGZF CRC-32 (opts.check_crc) ------------------------------------------------------------------------------------------
+// A CTA per block, looping over blocks so that the tables are built once per CTA: 8 KB of slice-by-8 tables and the byte tables of
+// the kCrcLevels combine operators (32 KB) in shared memory.  Thread t takes segment t of the block's frame (bgzf_crc.cuh); the
+// segments are combined by five shuffle levels inside a warp and three across the warps.
+struct CrcArgs {
+    const uint8_t* u; const uint64_t* uoff; const uint32_t* isize;
+    const uint32_t* want;                             // [b] trailer CRC ^ crc32(0^isize): the block's raw CRC
+    uint32_t n_blocks;
+    uint32_t ops[bgzf_crc::kCrcLevels][32];           // bgzf_crc::make_ops
+};
+
+__global__ void __launch_bounds__(bgzf_crc::kCrcThreads, 4) crc_kernel(const CrcArgs a, unsigned long long* err) {
+    namespace bc = bgzf_crc;
+    constexpr uint32_t kWarps = bc::kCrcThreads / 32;
+    static_assert(kWarps <= 32 && (1u << bc::kCrcLevels) == bc::kCrcThreads && bc::kCrcThreads == 256, "one table entry per thread");
+    __shared__ uint32_t T[8][256];
+    __shared__ uint32_t O[bc::kCrcLevels][4][256];
+    __shared__ uint32_t warp_r[kWarps];
+    const uint32_t t = threadIdx.x, lane = t & 31u, warp = t >> 5;
+    T[0][t] = bc::t0_entry(t);
+#pragma unroll 1
+    for (uint32_t k = 0; k < bc::kCrcLevels; ++k)
+#pragma unroll 1
+        for (uint32_t j = 0; j < 4; ++j) O[k][j][t] = bc::op_entry(a.ops[k], j, t);
+    __syncthreads();
+    uint32_t c = T[0][t];
+    for (int k = 1; k < 8; ++k) { c = bc::zero_byte(c, T[0]); T[k][t] = c; }
+    __syncthreads();
+    for (uint32_t b = blockIdx.x; b < a.n_blocks; b += gridDim.x) {
+        const uint8_t* blk = a.u + a.uoff[b];
+        const uint32_t n = a.isize[b];
+        uint32_t r = bc::segment(blk, n, t, T);
+#pragma unroll
+        for (uint32_t k = 0; k < 5; ++k) r = bc::shift(r, O[k]) ^ __shfl_down_sync(0xffffffffu, r, 1u << k);
+        if (lane == 0) warp_r[warp] = r;
+        __syncthreads();
+        if (warp == 0) {
+            r = lane < kWarps ? warp_r[lane] : 0u;
+#pragma unroll
+            for (uint32_t k = 5; k < bc::kCrcLevels; ++k) r = bc::shift(r, O[k]) ^ __shfl_down_sync(0xffffffffu, r, 1u << (k - 5));
+            if (lane == 0 && !bc::matches(r, a.want[b], blk, n, T[0])) report(err, b, E_CRC);
+        }
+        __syncthreads();   // warp_r is rewritten by the next block
+    }
 }
 
 // ---- K2: per record ---------------------------------------------------------------------------------------------------------
@@ -453,6 +502,7 @@ const char* err_text(uint32_t code) {
         case E_NAMED: return "record enters the pileup without integer AS:i / XM:i tags (pysam get_tag KeyError, cmseq/cmseq.py:545)";
         case E_NOQUAL: return "record has no base qualities: query_qualities is None (TypeError at cmseq/cmseq.py:538)";
         case E_QLEN: return "read longer than 65535 bases (len(SEQ) is carried as 16 bits)";
+        case E_CRC: return "CRC mismatch in BGZF block";
         default: return "hardware decompression produced a block of the wrong size / record chain broken";
     }
 }
@@ -525,10 +575,11 @@ extern "C" int mmlst_dev_bam_info(const mmlst_dev_bam* b, mmlst_dev_bam_info_t* 
 
 #define ING_TRY(expr) do { int _r = (expr); if (_r != MMLST_OK) return _r; } while (0)
 
-static int fetch_error(unsigned long long* d_err, cudaStream_t st, const char* what) {
+static int fetch_error(unsigned long long* d_err, cudaStream_t st, const char* what, unsigned long long* got = nullptr) {
     unsigned long long e = kNoErr;
     CUDA_TRY(cudaMemcpyAsync(&e, d_err, 8, cudaMemcpyDeviceToHost, st));
     CUDA_TRY(cudaStreamSynchronize(st));
+    if (got) *got = e;
     if (e == kNoErr) return MMLST_OK;
     const uint32_t code = static_cast<uint32_t>(e & 0xff);
     mmlst_set_error("%s: record %llu: %s", what, static_cast<unsigned long long>(e >> 8), err_text(code));
@@ -549,7 +600,7 @@ extern "C" int mmlst_bam_ingest(int device, const uint8_t* bam, size_t n_bytes, 
         if (rc != MMLST_OK) { mmlst_set_error("mmlst_bam_ingest: %s; use mmlst_bam_unpack", mmlst_last_error()); return rc; }
     }
     // ---- host: BGZF block table
-    struct Blk { uint64_t coff; uint32_t clen, isize; uint64_t uoff; };
+    struct Blk { uint64_t coff; uint32_t clen, isize, crc; uint64_t uoff; };
     std::vector<Blk> blocks;
     uint64_t usize = 0;
     for (size_t p = 0; p < n_bytes;) {
@@ -571,6 +622,7 @@ extern "C" int mmlst_bam_ingest(int device, const uint8_t* bam, size_t n_bytes, 
         Blk b;
         b.coff = p + 12 + xlen;
         b.clen = static_cast<uint32_t>(total - 12 - xlen - 8);
+        b.crc = h_rd32(&bam[p + total - 8]);
         b.isize = h_rd32(&bam[p + total - 4]);
         b.uoff = usize;
         if (b.isize > 65536) { mmlst_set_error("mmlst_bam_ingest: BGZF block with ISIZE %u > 64 KiB at %zu", b.isize, p); return MMLST_E_BAM; }
@@ -588,13 +640,14 @@ extern "C" int mmlst_bam_ingest(int device, const uint8_t* bam, size_t n_bytes, 
     auto mark = [&]() { cudaEventRecord(ev[evn++], st); };
 
     // ---- H2D + hardware inflate
-    DBuf d_comp, d_u, d_act, d_isize, d_uoff, d_err;
+    DBuf d_comp, d_u, d_act, d_isize, d_uoff, d_err, d_crc;
     ING_TRY(d_comp.alloc(n_bytes + 64));
     ING_TRY(d_u.alloc(usize + 64));
     ING_TRY(d_act.alloc(static_cast<size_t>(nb) * 4));
     ING_TRY(d_isize.alloc(static_cast<size_t>(nb) * 4));
     ING_TRY(d_uoff.alloc((static_cast<size_t>(nb) + 1) * 8));
     ING_TRY(d_err.alloc(8 + 32));
+    if (o.check_crc) ING_TRY(d_crc.alloc(static_cast<size_t>(nb) * 4));
     unsigned long long* err = d_err.as<unsigned long long>();
     uint32_t* d_flags = reinterpret_cast<uint32_t*>(err + 1);   // [0] sortedness, [1] repair counter, [2] uniform qlen, [3] max row words, [4] records with the unmapped flag
     CUDA_TRY(cudaMemsetAsync(err, 0xff, 8, st));
@@ -606,6 +659,13 @@ extern "C" int mmlst_bam_ingest(int device, const uint8_t* bam, size_t n_bytes, 
     h_uoff[nb] = usize;
     CUDA_TRY(cudaMemcpyAsync(d_isize.p, h_isize.data(), static_cast<size_t>(nb) * 4, cudaMemcpyHostToDevice, st));
     CUDA_TRY(cudaMemcpyAsync(d_uoff.p, h_uoff.data(), (static_cast<size_t>(nb) + 1) * 8, cudaMemcpyHostToDevice, st));
+    std::vector<uint32_t> h_want;
+    if (o.check_crc) {   // the raw CRC each block must have: trailer ^ crc32(0^isize)
+        static const std::vector<uint32_t> zeros = [] { std::vector<uint32_t> z(65537); bgzf_crc::make_zeros(z.data(), 65536); return z; }();
+        h_want.resize(nb);
+        for (uint32_t b = 0; b < nb; ++b) h_want[b] = blocks[b].crc ^ zeros[blocks[b].isize];
+        CUDA_TRY(cudaMemcpyAsync(d_crc.p, h_want.data(), static_cast<size_t>(nb) * 4, cudaMemcpyHostToDevice, st));
+    }
     mark();  // 1
     std::vector<CUmemDecompressParams> prm(nb);
     memset(prm.data(), 0, sizeof(CUmemDecompressParams) * nb);
@@ -626,6 +686,17 @@ extern "C" int mmlst_bam_ingest(int device, const uint8_t* bam, size_t n_bytes, 
     }
     check_isize_kernel<<<(nb + kT - 1) / kT, kT, 0, st>>>(d_act.as<uint32_t>(), d_isize.as<uint32_t>(), nb, err);
     CUDA_TRY(cudaGetLastError());
+    if (o.check_crc) {
+        static const CrcArgs proto = [] { CrcArgs c{}; bgzf_crc::make_ops(c.ops); return c; }();
+        CrcArgs ca = proto;
+        ca.u = d_u.as<uint8_t>(); ca.uoff = d_uoff.as<uint64_t>(); ca.isize = d_isize.as<uint32_t>(); ca.want = d_crc.as<uint32_t>(); ca.n_blocks = nb;
+        int sms = 0, per_sm = 0;
+        CUDA_TRY(cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, device));
+        CUDA_TRY(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, crc_kernel, bgzf_crc::kCrcThreads, 0));
+        const uint32_t grid = std::min<uint32_t>(nb, static_cast<uint32_t>(std::max(sms, 1) * std::max(per_sm, 1)));
+        crc_kernel<<<grid, bgzf_crc::kCrcThreads, 0, st>>>(ca, err);
+        CUDA_TRY(cudaGetLastError());
+    }
     mark();  // 2
     // ---- header (first bytes of the inflated stream come back to the host)
     std::unique_ptr<mmlst_dev_bam> B(new mmlst_dev_bam());
@@ -642,8 +713,14 @@ extern "C" int mmlst_bam_ingest(int device, const uint8_t* bam, size_t n_bytes, 
             head = hb;
             CUDA_TRY(cudaMemcpyAsync(hb, d_u.p, want, cudaMemcpyDeviceToHost, st));
             {
-                const int rc = fetch_error(err, st, "mmlst_bam_ingest (inflate)");
-                if (rc != MMLST_OK) { mmlst_set_error("mmlst_bam_ingest: a BGZF block did not inflate to its ISIZE (corrupt file?)"); return MMLST_E_BAM; }
+                unsigned long long e = kNoErr;
+                const int rc = fetch_error(err, st, "mmlst_bam_ingest (inflate)", &e);
+                if (rc != MMLST_OK) {
+                    // block k counts the non-empty blocks, as the host unpacker's message does
+                    if (e != kNoErr && (e & 0xff) == E_CRC) mmlst_set_error("mmlst_bam_ingest: CRC mismatch in BGZF block %llu", e >> 8);
+                    else mmlst_set_error("mmlst_bam_ingest: a BGZF block did not inflate to its ISIZE (corrupt file?)");
+                    return MMLST_E_BAM;
+                }
             }
             if (round == 0 && want >= 12 && want < usize && memcmp(head, "BAM\1", 4) == 0) {
                 const int32_t lt = static_cast<int32_t>(h_rd32(&head[4]));

@@ -33,7 +33,8 @@ enum Err : uint32_t {
     E_NAMED = 12,       // record enters the pileup without integer AS:i / XM:i (cmseq/cmseq.py:545)
     E_NOQUAL = 13,      // record enters the pileup without base qualities (cmseq/cmseq.py:538)
     E_CHAIN = 14,       // record chain could not be established (internal)
-    E_QLEN = 15         // read longer than 65535 bases (len(SEQ) is carried as 16 bits)
+    E_QLEN = 15,        // read longer than 65535 bases (len(SEQ) is carried as 16 bits)
+    E_CRC = 16          // inflated BGZF block does not match its trailer's CRC-32 (index = block, opts.check_crc)
 };
 
 ING_HD uint32_t rd16(const uint8_t* p) { return static_cast<uint32_t>(p[0]) | (static_cast<uint32_t>(p[1]) << 8); }

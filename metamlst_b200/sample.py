@@ -173,7 +173,9 @@ class SampleTyper:
                  min_accuracy: float = 0.90, penalty: int = 100, nloci: int = 100, species_filter: Optional[str] = None,
                  write_known: bool = False, log: bool = False, presorted: bool = False, debug: bool = False,
                  unpack_threads: int = 0, ctx: Optional[native.Context] = None, engine: str = "device", group=None,
-                 ingest: str = "host"):
+                 ingest: str = "host", check_crc: bool = False):
+        """check_crc: with ingest="device", also check every BGZF block's CRC32 on the GPU (bam.ingest_bam); the host unpacker
+        (ingest="host") always checks it."""
         if not os.path.isfile(db_path):
             raise IOError("Failed to connect to the database: please check your database file!")  # metamlst.py:72-73
         if engine not in ("device", "host", "onecall"):
@@ -186,7 +188,7 @@ class SampleTyper:
         self.device = int(device)
         self._ctx = ctx
         self._own_ctx = ctx is None
-        self.engine, self.group, self.ingest = engine, group, ingest
+        self.engine, self.group, self.ingest, self.check_crc = engine, group, ingest, bool(check_crc)
         self.minscore, self.max_xM, self.min_read_len = int(minscore), int(max_xM), int(min_read_len)
         self.min_accuracy, self.penalty, self.nloci = float(min_accuracy), int(penalty), int(nloci)
         self.species_filter, self.write_known, self.log, self.presorted, self.debug = species_filter, write_known, log, presorted, debug
@@ -254,7 +256,7 @@ class SampleTyper:
         in HBM (csrc/ingest.cu).  A host-unpacked sample passes through."""
         if hasattr(loaded, "c_struct"):
             return loaded
-        st = bam.ingest_bam(loaded, self.device, presorted=self.presorted, want_qhash=want_qhash)
+        st = bam.ingest_bam(loaded, self.device, presorted=self.presorted, want_qhash=want_qhash, check_crc=self.check_crc)
         bam.POOL.put(loaded)  # the call is synchronous: the staging buffer has been consumed
         return st
 
