@@ -231,11 +231,15 @@ int mmlst_consensus_dev(const uint32_t* counts, const uint8_t* dbseq, const uint
  *   scratch: >= 12*n_loci + 16 bytes, 8-byte aligned.  flags: MMLST_SELECT_CONSUME = the call resets what it has read
  *   (sum_as / n_hit / first_idx of every hit row, counters) so the next pass needs no memset of the score tables;
  *   MMLST_SELECT_SCRATCH_CLEAN = the caller zeroed the scratch once and every call since ran to completion (the
- *   call leaves it zeroed), so the 4-byte ticket memset is skipped.
+ *   call leaves its ticket at zero; the per-locus results before it are scratch), so the 4-byte ticket memset is skipped.
  *   Outputs: header[0]=n_chosen [1]=n_chunks [2]=total columns [3]=error bits (1: "Database is broken", 2: chunk list
  *   overflow) [4]=records per chunk [6,7]=counters[0] (totalReads) [8,9]=counters[1] (ignoredReads) when `counters` is
  *   given; chosen_tid / chosen_species / col_off / db_start per chosen locus in output order; chunks for
  *   mmlst_pileup_indirect_dev.  header needs 16 words.
+ *   Range: n_loci <= 8192, n_species <= 4096, and the finalizing CTA keeps 4 (11 n_loci + 1 + 4 n_species) + 16 bytes in shared memory, which
+ *   must fit the current device's opt-in maximum per block (cudaDevAttrMaxSharedMemoryPerBlockOptin, about 227 KB on sm_100, less the kernel's
+ *   static shared memory): about 5000 loci at 7 loci per species, 3800 at 4096 species.  An index past either bound is refused with
+ *   MMLST_E_RANGE before any launch, and the message names both sizes; mmlst_index_upload applies the same check.
  * --------------------------------------------------------------------------------------------------------------- */
 /* Finalization of the selection (gate, dict order, column layout, chunk list) by ONE warp with shuffles instead of the whole last CTA with barriers, when
  * n_loci <= 32 and n_species <= 32 (larger index sets always take the CTA-wide form).  1 = on, 0 = off, other = query; returns the previous value;
@@ -423,6 +427,7 @@ int mmlst_score(mmlst_ctx* ctx, const mmlst_soa* soa, const uint8_t* allow, cons
  *   species_of_locus[n_loci], genes_in_db[n_species] = rows of `genes` per organism (metamlst.py:184),
  *   db_ascii / db_off[n_ref+1]: the DB sequence of every row (metaMLST_functions.py:260-276 compares against it),
  *   bam_ln[n_ref]: @SQ LN of every reference.
+ *   An index the selection cannot serve (see the range of mmlst_select_dev) is refused by mmlst_index_upload with MMLST_E_RANGE.
  * mmlst_sample_result: caller-allocated arrays sized for n_loci entries (col_off: n_loci + 1), cons for cons_capacity bytes;
  *   sum_as / n_hit / first_idx optional (all three or none).  Output order = the reference's dict order (H5).
  *   error_bits & 1: "Database is broken" (metamlst.py:188-190), nothing piled up.  MMLST_E_RANGE + bad_len_tid: a chosen reference

@@ -685,6 +685,7 @@ extern "C" int mmlst_index_upload(mmlst_ctx* c, const mmlst_index* ix) {
     const uint32_t nr = ix->n_ref, nl = ix->n_loci, ns = ix->n_species;
     if (nr == 0 || nl == 0 || ns == 0) { mmlst_set_error("mmlst_index_upload: empty index"); return MMLST_E_ARG; }
     if (nl > 8192 || ns > 4096) { mmlst_set_error("mmlst_index_upload: more than 8192 loci / 4096 species"); return MMLST_E_RANGE; }
+    TRY(mmlst_select_fits(nl, ns, "mmlst_index_upload"));   // refused here, not by the first mmlst_sample
     // allele rows grouped by locus (counting sort, stable: ascending row inside a locus)
     std::vector<uint32_t> start(nl + 1, 0), rows(nr);
     for (uint32_t t = 0; t < nr; ++t) {

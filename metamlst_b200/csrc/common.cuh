@@ -46,6 +46,10 @@ int mmlst_cuda_fail(cudaError_t e, const char* what);
 
 int mmlst_num_sms();
 
+// MMLST_OK when the selection launch of mmlst_select_dev for n_loci / n_species fits the current device's shared memory per block (the opt-in
+// maximum less the kernel's static part), else MMLST_E_RANGE with a message that names both sizes (`who` = the refusing call)
+int mmlst_select_fits(uint32_t n_loci, uint32_t n_species, const char* who);
+
 // MMLST_TRACE=1: host wall-clock marks inside the host-buffer calls, printed to stderr when the call returns (profiles/tools/e2e_trace.py)
 void mmlst_trace_mark(const char* label);
 void mmlst_trace_flush(const char* call);

@@ -493,6 +493,34 @@ extern "C" int mmlst_set_select_warp_finalize(int on) {
     return prev;
 }
 
+// Dynamic shared memory of one selection launch: the finalization arrays (10 n_loci + 1 + 3 n_species words, see the kernel) + the prefetched
+// species_of_locus / genes_in_db, and never less than the 193 words the one-warp finalizer lays out whatever n_loci is.
+static size_t select_smem_bytes(uint32_t n_loci, uint32_t n_species) {
+    const size_t smem = sizeof(uint32_t) * (static_cast<size_t>(n_loci) * 11 + 1 + 4 * static_cast<size_t>(n_species)) + 16;
+    return smem < 200 * sizeof(uint32_t) ? 200 * sizeof(uint32_t) : smem;
+}
+
+// see common.cuh
+int mmlst_select_fits(uint32_t n_loci, uint32_t n_species, const char* who) {
+    static int max_dynamic_by_device[MMLST_MAX_DEVICES] = {0};   // 0 = not asked yet
+    int& max_dynamic = max_dynamic_by_device[mmlst_current_device()];
+    if (max_dynamic == 0) {
+        int dev = 0, optin = 0;
+        CUDA_TRY(cudaGetDevice(&dev));
+        CUDA_TRY(cudaDeviceGetAttribute(&optin, cudaDevAttrMaxSharedMemoryPerBlockOptin, dev));
+        cudaFuncAttributes fa;
+        CUDA_TRY(cudaFuncGetAttributes(&fa, sel_locus));
+        max_dynamic = optin - static_cast<int>(fa.sharedSizeBytes);   // the kernel's static shared memory counts against the same per-block limit
+    }
+    const size_t smem = select_smem_bytes(n_loci, n_species);
+    if (smem > static_cast<size_t>(max_dynamic)) {
+        mmlst_set_error("%s: %u loci / %u species need %zu bytes of shared memory per block for the selection, the device allows %d", who, n_loci,
+                        n_species, smem, max_dynamic);
+        return MMLST_E_RANGE;
+    }
+    return MMLST_OK;
+}
+
 // see include/mmlst.h
 extern "C" int mmlst_select_dev(int64_t* sum_as, uint32_t* n_hit, uint32_t* first_idx, const uint32_t* locus_rows,
                                 const uint32_t* locus_start, const uint32_t* allele_num, uint32_t n_ref,
@@ -509,6 +537,7 @@ extern "C" int mmlst_select_dev(int64_t* sum_as, uint32_t* n_hit, uint32_t* firs
     }
     if (n_loci == 0) { mmlst_set_error("mmlst_select_dev: no loci"); return MMLST_E_ARG; }
     if (n_loci > 8192 || n_species > 4096) { mmlst_set_error("mmlst_select_dev: more than 8192 loci / 4096 species"); return MMLST_E_RANGE; }
+    if (const int rc = mmlst_select_fits(n_loci, n_species, "mmlst_select_dev")) return rc;
     const size_t need = static_cast<size_t>(n_loci) * 12 + 16;
     if (scratch_bytes < need || (reinterpret_cast<uintptr_t>(scratch) & 7)) { mmlst_set_error("mmlst_select_dev: scratch needs %zu bytes, 8-byte aligned", need); return MMLST_E_ARG; }
     cudaStream_t s = static_cast<cudaStream_t>(stream);
@@ -532,12 +561,14 @@ extern "C" int mmlst_select_dev(int64_t* sum_as, uint32_t* n_hit, uint32_t* firs
     a.tl = mmlst_timeline_buffer();
     a.warp_final = select_warp() ? 1u : 0u;
     if (!(flags & MMLST_SELECT_SCRATCH_CLEAN)) CUDA_TRY(cudaMemsetAsync(a.done, 0, 4, s));
-    // finalization arrays (10 n_loci + 1 + 3 n_species words, see the kernel) + the prefetched species_of_locus / genes_in_db
-    size_t smem = sizeof(uint32_t) * (static_cast<size_t>(n_loci) * 11 + 1 + 4 * static_cast<size_t>(n_species)) + 16;
-    if (smem < 200 * sizeof(uint32_t)) smem = 200 * sizeof(uint32_t);   // the one-warp finalizer lays out 193 words whatever n_loci is
-    static size_t configured_by_device[MMLST_MAX_DEVICES] = {0};  // 0 = the 48 KB every kernel starts with
+    const size_t smem = select_smem_bytes(n_loci, n_species);
+    static size_t configured_by_device[MMLST_MAX_DEVICES] = {0};  // 0 = not asked yet
     size_t& configured = configured_by_device[mmlst_current_device()];
-    if (configured == 0) configured = 48 * 1024;
+    if (configured == 0) {   // what every kernel starts with: 48 KB less its static shared memory
+        cudaFuncAttributes fa;
+        CUDA_TRY(cudaFuncGetAttributes(&fa, sel_locus));
+        configured = fa.maxDynamicSharedSizeBytes;
+    }
     if (smem > configured) {
         CUDA_TRY(cudaFuncSetAttribute(sel_locus, cudaFuncAttributeMaxDynamicSharedMemorySize, static_cast<int>(smem)));
         configured = smem;
