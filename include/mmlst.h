@@ -219,6 +219,46 @@ int mmlst_consensus_dev(const uint32_t* counts, const uint8_t* dbseq, const uint
                         uint32_t mincov, uint8_t* cons, uint32_t* holes, uint32_t* snps, void* stream);
 
 /* ---------------------------------------------------------------------------------------------------------------
+ * cmseq contig statistics over a BATCH of contigs (metamlst_b200/cmseq_api.py, the BamFile *_all methods).  Replaces the column
+ * loops of cmseq/cmseq.py:507-569 (get_base_stats: column recorded iff A+C+G+T >= min_read_depth; binomial test only where
+ * max/sum < dominant_frq_thrsh), :226-241 (reference_free_consensus), :430-456 (polymorphism_rate) and :459-490
+ * (breadth_and_depth_of_coverage: window [trunc, len - trunc) when len > 2 trunc).  The ratios, p-values and distributions stay on
+ * the host, computed from what this returns.
+ *   counts[total_cols][5], col_off[n+1] (col_off[0] = 0, ascending; contigs of length 0 allowed): the batch's count tensor
+ *   selected column    : inside the contig's window and A+C+G+T >= mincov
+ *   low-dominance      : selected and (double)max(A,C,G,T) / (double)(A+C+G+T) < dominant_frq_thrsh (IEEE division, strict <)
+ *   sel_off / low_off / depth_off [n+1]: prefix over the batch's contigs of the number of selected columns, of low-dominance
+ *                        columns and of the sum of A+C+G+T over selected columns (contig i: [i+1] - [i])
+ *   compacted columns  : ascending column inside a contig, contigs in batch order (positions from scans, never from atomics);
+ *                        out_col = column inside the contig (0-based), out_val = `width` u32 per column:
+ *                        MMLST_STATS_COLUMNS every selected column, width 5 (A, C, G, T, N)       -- get_base_stats
+ *                        MMLST_STATS_DEPTH   every selected column, width 1 (A+C+G+T)            -- breadth_and_depth_of_coverage
+ *                        MMLST_STATS_LOWDOM  low-dominance columns, width 2 (max, A+C+G+T)       -- polymorphism_rate, consensus
+ *                        capacity: sel_off[n] (low_off[n] for LOWDOM) <= total_cols entries
+ *   cons[total_cols] (or NULL): the majority call (first maximum in the order A, C, G, N, T, H8: the column rule of the consensus
+ *                        kernel) of every selected column, none_char elsewhere
+ *   scratch            : mmlst_contig_stats_scratch_bytes(total_cols) bytes, 16-byte aligned
+ *   flags              : MMLST_CONSENSUS_CONSUME = zero the counts it read (the next batch accumulates from zero, no memset)
+ * Range: total_cols <= MMLST_CONTIG_STATS_MAX_COLS (the kernels index counts and out_val with 5 * column in 32 bits), else
+ * MMLST_E_RANGE before any launch.  Three launches (tile sums, one-CTA scan, emit); 20 B / column in.
+ * --------------------------------------------------------------------------------------------------------------- */
+#define MMLST_STATS_COLUMNS 0u
+#define MMLST_STATS_DEPTH 1u
+#define MMLST_STATS_LOWDOM 2u
+#define MMLST_CONTIG_STATS_MAX_COLS 858993459u   /* floor((2^32 - 1) / 5) */
+typedef struct {
+    uint32_t mode;               /* MMLST_STATS_* */
+    uint32_t mincov;             /* >= 1 */
+    uint32_t trunc;              /* 0 = whole contig */
+    uint32_t none_char;          /* byte of unselected columns in cons, 0..255 */
+    double dominant_frq_thrsh;
+} mmlst_contig_stats_params;
+size_t mmlst_contig_stats_scratch_bytes(uint32_t total_cols);
+int mmlst_contig_stats_dev(uint32_t* counts, const uint32_t* col_off, uint32_t n, uint32_t total_cols, const mmlst_contig_stats_params* prm,
+                           void* scratch, size_t scratch_bytes, uint32_t* sel_off, uint32_t* low_off, uint64_t* depth_off,
+                           uint32_t* out_col, uint32_t* out_val, uint8_t* cons, uint32_t flags, void* stream);
+
+/* ---------------------------------------------------------------------------------------------------------------
  * Best-allele selection on the device: no host round trip between stage 1 and stage 2.  Replaces metamlst.py:133-151
  * (maxLen, penalty, round(avg,1) -- computed exactly as integer tenths from the IEEE double quotient, H6), :184-206
  * (--nloci gate), :213-220 + :244 (alleles whose rounded average equals the locus maximum, lowest int(allele)), and the
@@ -462,6 +502,25 @@ int mmlst_coverage(mmlst_ctx* ctx, const mmlst_soa* soa, const uint64_t* qhash, 
 int mmlst_pileup_consensus(mmlst_ctx* ctx, const mmlst_soa* soa, const uint32_t* chosen_tid, uint32_t n_loci,
                            const uint8_t* dbseq, const uint32_t* col_off, int minscore, int max_xm, uint32_t mincov,
                            int impl, uint32_t* counts, uint8_t* cons, uint32_t* holes, uint32_t* snps);
+
+/* seam S2' bulk (cmseq_api.BamFile *_all methods): mmlst_contig_stats_dev over a batch of contigs of a pileup stream, host buffers.
+ * The records and plane rows of the contigs (consecutive contigs are one contiguous range of the sorted stream and cross the bus as
+ * one copy) -> mmlst_pileup_dev (library chunk rule) ->
+ * mmlst_contig_stats_dev -> the [n+1] prefixes, then the compacted prefix they size, back to the host.  tid[n] ascending,
+ * col_off[n+1] = prefix of the contigs' lengths (host).  Range: col_off[n] <= MMLST_CONTIG_STATS_MAX_COLS, else MMLST_E_RANGE
+ * (checked before anything else).  out->capacity = entries of out_col (out_val holds width x as many); out->n_out = entries written. */
+typedef struct {
+    uint32_t* sel_off;           /* [n+1] */
+    uint32_t* low_off;           /* [n+1] */
+    uint64_t* depth_off;         /* [n+1] */
+    uint32_t* out_col;           /* [capacity] */
+    uint32_t* out_val;           /* [capacity * width] */
+    uint8_t* cons;               /* [col_off[n]] or NULL */
+    uint64_t capacity;
+    uint64_t n_out;
+} mmlst_contig_stats_out;
+int mmlst_contig_stats(mmlst_ctx* ctx, const mmlst_soa* soa, const uint32_t* tid, uint32_t n, const uint32_t* col_off, int minscore,
+                       int max_xm, const mmlst_contig_stats_params* prm, mmlst_contig_stats_out* out);
 
 /* seam S3 (metamlst-merge.py:177-181): DB planes stay resident in the context across calls / samples. */
 int mmlst_db_upload(mmlst_ctx* ctx, const uint32_t* db_hi, const uint32_t* db_lo, const uint16_t* row_len,

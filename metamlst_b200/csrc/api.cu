@@ -127,6 +127,7 @@ struct mmlst_ctx {
     DevBuf qhash, cov_table, cov;
     // pileup stream (chosen contigs only)
     DevBuf p_recs, planes, chunks, counts, dbseq, col_off, cons, holes, snps;
+    DevBuf cs_scratch, cs_off, cs_out;   // contig statistics (mmlst_contig_stats): tile sums, the three prefixes, compacted columns
     // hamming
     DevBuf db_hi, db_lo, db_len, q_hi, q_lo, q_len, blocks, best;
     DevBuf xr_ids, xr_x, xr_bytes, xq_ids, xq_x, xq_bytes;  // flagged (non-ACGT) rows / queries, H9
@@ -173,7 +174,7 @@ struct mmlst_ctx {
                        &db_lo, &db_len, &q_hi, &q_lo, &q_len, &blocks, &best, &qhash, &cov_table, &cov, &xr_ids, &xr_x, &xr_bytes, &xq_ids, &xq_x, &xq_bytes,
                        &run_tid, &run_start, &chunk_run, &chunk_qlen, &prof_start, &prof_allele, &st_q, &st_qn, &st_count, &st_best, &st_nbest, &st_out,
                        &first_row, &row_key, &zbuf, &zact, &zpbuf, &zpact, &ix_locus_of, &ix_locus_rows, &ix_locus_start, &ix_allele_num, &ix_species_of_locus, &ix_genes_in_db, &ix_db_ascii,
-                       &ix_db_off, &ix_bam_ln, &ix_zero64, &ix_scratch, &ix_out, &ix_db_start, &ix_chunks};
+                       &ix_db_off, &ix_bam_ln, &ix_zero64, &ix_scratch, &ix_out, &ix_db_start, &ix_chunks, &cs_scratch, &cs_off, &cs_out};
         for (DevBuf* b : l) all[n_all++] = b;
     }
 };
@@ -513,15 +514,22 @@ extern "C" int mmlst_pileup_consensus_indirect_dev(const mmlst_prec* recs, const
 
 // The pileup records and plane rows of the chosen contigs (contiguous ranges of the coordinate-sorted stream) host -> device, packed one after the
 // other, plus the chunk list over them.  The copies are dealt over the context's copy lanes; `s` continues when all of them have landed.
+// `runs`: a run of consecutive tids is one record range and one plane range of the stream and crosses the bus as one copy of each (plain
+// stream only; its chunks share the run's plane_delta).
 static int upload_chosen_contigs(mmlst_ctx* c, const mmlst_soa* soa, const uint32_t* chosen_tid, uint32_t n_loci, const uint32_t* col_off,
-                                 std::vector<mmlst_chunk>& chunks, bool use_zp = false) {
+                                 std::vector<mmlst_chunk>& chunks, bool use_zp = false, bool runs = false) {
     cudaStream_t s = c->stream;
     auto row_end = [&](uint64_t r) { return soa->p_recs[r].row_off + mmlst_row_words(soa->p_recs[r].nw); };
+    // end of the run that starts at chosen_tid[l] (exclusive index into chosen_tid)
+    auto run_end = [&](uint32_t l) { uint32_t e = l + 1; while (runs && e < n_loci && chosen_tid[e] == chosen_tid[e - 1] + 1) ++e; return e; };
     size_t n_rec = 0, n_words = 0;
     for (uint32_t l = 0; l < n_loci; ++l) {
         const uint32_t t = chosen_tid[l];
         if (t >= soa->n_ref) { mmlst_set_error("chosen_tid[%u]=%u out of range", l, t); return MMLST_E_ARG; }
-        const uint64_t r0 = soa->contig_start[t], r1 = soa->contig_start[t + 1];
+    }
+    for (uint32_t l = 0, e; l < n_loci; l = e) {
+        e = run_end(l);
+        const uint64_t r0 = soa->contig_start[chosen_tid[l]], r1 = soa->contig_start[chosen_tid[e - 1] + 1];
         if (r1 <= r0) continue;
         n_rec += r1 - r0;
         n_words += (size_t)row_end(r1 - 1) - soa->p_recs[r0].row_off + 4;  // +4: every range starts 16-byte aligned on the device
@@ -610,9 +618,9 @@ static int upload_chosen_contigs(mmlst_ctx* c, const mmlst_soa* soa, const uint3
     const uint32_t kChunkRecords = mmlst_chunk_records(n_rec);
     size_t rbase = 0, wbase = 0;
     int k = 0;
-    for (uint32_t l = 0; l < n_loci; ++l) {
-        const uint32_t t = chosen_tid[l];
-        const uint64_t r0 = soa->contig_start[t], r1 = soa->contig_start[t + 1];
+    for (uint32_t l = 0, e; l < n_loci; l = e) {
+        e = run_end(l);
+        const uint64_t r0 = soa->contig_start[chosen_tid[l]], r1 = soa->contig_start[chosen_tid[e - 1] + 1];
         const size_t nr = r1 - r0;
         if (nr == 0) continue;
         const uint32_t w0 = soa->p_recs[r0].row_off, w1 = row_end(r1 - 1);
@@ -620,14 +628,17 @@ static int upload_chosen_contigs(mmlst_ctx* c, const mmlst_soa* soa, const uint3
         k = (k + 1) % mmlst_ctx::kLanes;
         CUDA_TRY(cudaMemcpyAsync(c->planes.as<uint32_t>() + wbase, soa->planes + w0, (size_t)(w1 - w0) * 4, cudaMemcpyHostToDevice, c->lane[k]));
         k = (k + 1) % mmlst_ctx::kLanes;
-        for (size_t b = 0; b < nr; b += kChunkRecords) {
-            mmlst_chunk ck{};
-            ck.rec_begin = (uint32_t)(rbase + b);
-            ck.rec_end = (uint32_t)(rbase + std::min(nr, b + kChunkRecords));
-            ck.col_base = col_off[l];
-            ck.contig_len = col_off[l + 1] - col_off[l];
-            ck.plane_delta = (uint32_t)wbase - w0;
-            chunks.push_back(ck);
+        for (uint32_t m = l; m < e; ++m) {
+            const uint64_t q0 = soa->contig_start[chosen_tid[m]], q1 = soa->contig_start[chosen_tid[m] + 1];
+            for (uint64_t b = q0; b < q1; b += kChunkRecords) {
+                mmlst_chunk ck{};
+                ck.rec_begin = (uint32_t)(rbase + (b - r0));
+                ck.rec_end = (uint32_t)(rbase + (std::min<uint64_t>(q1, b + kChunkRecords) - r0));
+                ck.col_base = col_off[m];
+                ck.contig_len = col_off[m + 1] - col_off[m];
+                ck.plane_delta = (uint32_t)wbase - w0;
+                chunks.push_back(ck);
+            }
         }
         rbase += nr;
         wbase += (size_t)(w1 - w0);
@@ -671,6 +682,61 @@ extern "C" int mmlst_pileup_consensus(mmlst_ctx* c, const mmlst_soa* soa, const 
     CUDA_TRY(cudaStreamSynchronize(s));
     mmlst_trace_mark("sync");
     mmlst_trace_flush("mmlst_pileup_consensus");
+    return MMLST_OK;
+}
+
+extern "C" int mmlst_contig_stats(mmlst_ctx* c, const mmlst_soa* soa, const uint32_t* tid, uint32_t n, const uint32_t* col_off, int minscore,
+                                  int max_xm, const mmlst_contig_stats_params* prm, mmlst_contig_stats_out* out) {
+    if (!soa || !tid || !col_off || !prm || !out || !out->sel_off || !out->low_off || !out->depth_off) { mmlst_set_error("mmlst_contig_stats: null pointer"); return MMLST_E_ARG; }
+    if (col_off[0] != 0) { mmlst_set_error("mmlst_contig_stats: col_off[0] = %u, not 0", col_off[0]); return MMLST_E_ARG; }
+    for (uint32_t i = 0; i < n; ++i) {
+        if (col_off[i + 1] < col_off[i]) { mmlst_set_error("mmlst_contig_stats: col_off not ascending at %u", i); return MMLST_E_ARG; }
+        if (i && tid[i] <= tid[i - 1]) { mmlst_set_error("mmlst_contig_stats: tid not ascending at %u", i); return MMLST_E_ARG; }
+    }
+    const uint32_t total_cols = col_off[n];
+    if (total_cols > MMLST_CONTIG_STATS_MAX_COLS) {
+        mmlst_set_error("mmlst_contig_stats: %u columns in one batch, at most %u (5 * column in 32 bits)", total_cols, (uint32_t)MMLST_CONTIG_STATS_MAX_COLS);
+        return MMLST_E_RANGE;
+    }
+    if (prm->mode > MMLST_STATS_LOWDOM || prm->mincov == 0 || prm->none_char > 255) { mmlst_set_error("mmlst_contig_stats: mode %u / mincov %u / none_char %u out of range", prm->mode, prm->mincov, prm->none_char); return MMLST_E_ARG; }
+    const uint32_t width = prm->mode == MMLST_STATS_COLUMNS ? 5u : prm->mode == MMLST_STATS_DEPTH ? 1u : 2u;
+    if (out->capacity && (!out->out_col || !out->out_val)) { mmlst_set_error("mmlst_contig_stats: null pointer"); return MMLST_E_ARG; }
+    out->n_out = 0;
+    if (n == 0) { out->sel_off[0] = 0; out->low_off[0] = 0; out->depth_off[0] = 0; return MMLST_OK; }
+    CTX_ENTER(c);
+    cudaStream_t s = c->stream;
+    mmlst_trace_mark("enter");
+    std::vector<mmlst_chunk> chunks;
+    TRY(upload_chosen_contigs(c, soa, tid, n, col_off, chunks, false, true));
+    TRY(h2d(c->col_off, col_off, (size_t)n + 1, s));
+    const size_t scratch = mmlst_contig_stats_scratch_bytes(total_cols);
+    TRY(c->counts.reserve((size_t)total_cols * 20 + 16)); TRY(c->cs_scratch.reserve(scratch));
+    TRY(c->cs_off.reserve(((size_t)n + 1) * 16 + 16)); TRY(c->cs_out.reserve((size_t)total_cols * 4 * (1 + width) + 16));
+    if (out->cons) TRY(c->cons.reserve((size_t)total_cols + 16));
+    uint32_t* d_sel = c->cs_off.as<uint32_t>(); uint32_t* d_low = d_sel + n + 1;
+    uint64_t* d_dep = reinterpret_cast<uint64_t*>(c->cs_off.as<uint8_t>() + (((size_t)n + 1) * 8 + 15) / 16 * 16);
+    uint32_t* d_col = c->cs_out.as<uint32_t>(); uint32_t* d_val = d_col + total_cols;
+    CUDA_TRY(cudaMemsetAsync(c->counts.p, 0, (size_t)total_cols * 20, s));
+    TRY(mmlst_pileup_dev(c->p_recs.as<mmlst_prec>(), c->planes.as<uint32_t>(), c->chunks.as<mmlst_chunk>(), (uint32_t)chunks.size(),
+                         soa->max_row_words, minscore, max_xm, c->counts.as<uint32_t>(), total_cols, 0, s));
+    TRY(mmlst_contig_stats_dev(c->counts.as<uint32_t>(), c->col_off.as<uint32_t>(), n, total_cols, prm, c->cs_scratch.p, scratch, d_sel, d_low, d_dep,
+                               d_col, d_val, out->cons ? c->cons.as<uint8_t>() : nullptr, 0, s));
+    CUDA_TRY(cudaMemcpyAsync(out->sel_off, d_sel, ((size_t)n + 1) * 4, cudaMemcpyDeviceToHost, s));
+    CUDA_TRY(cudaMemcpyAsync(out->low_off, d_low, ((size_t)n + 1) * 4, cudaMemcpyDeviceToHost, s));
+    CUDA_TRY(cudaMemcpyAsync(out->depth_off, d_dep, ((size_t)n + 1) * 8, cudaMemcpyDeviceToHost, s));
+    if (out->cons && total_cols) CUDA_TRY(cudaMemcpyAsync(out->cons, c->cons.p, total_cols, cudaMemcpyDeviceToHost, s));
+    mmlst_trace_mark("summaries_enqueued");
+    CUDA_TRY(cudaStreamSynchronize(s));
+    const uint64_t n_out = prm->mode == MMLST_STATS_LOWDOM ? out->low_off[n] : out->sel_off[n];
+    if (n_out > out->capacity) { mmlst_set_error("mmlst_contig_stats: %llu compacted columns, capacity %llu", (unsigned long long)n_out, (unsigned long long)out->capacity); return MMLST_E_ARG; }
+    if (n_out) {
+        CUDA_TRY(cudaMemcpyAsync(out->out_col, d_col, n_out * 4, cudaMemcpyDeviceToHost, s));
+        CUDA_TRY(cudaMemcpyAsync(out->out_val, d_val, n_out * 4 * width, cudaMemcpyDeviceToHost, s));
+        CUDA_TRY(cudaStreamSynchronize(s));
+    }
+    out->n_out = n_out;
+    mmlst_trace_mark("sync");
+    mmlst_trace_flush("mmlst_contig_stats");
     return MMLST_OK;
 }
 

@@ -4,7 +4,7 @@ set -e
 cd "$(dirname "$0")"
 NVCC=${NVCC:-/usr/local/cuda/bin/nvcc}
 FLAGS="-gencode arch=compute_100a,code=sm_100a -O3 -lineinfo -std=c++17 -Xcompiler -fPIC,-O3,-Wall -Xptxas -v"
-SRCS="api.cu select.cu score.cu score_runs.cu coverage.cu pileup_atomic.cu pileup_bitsliced.cu consensus.cu hamming.cu hamming_exact.cu hamming_tc.cu st_match.cu ingest.cu de.cu allreduce.cu exchange.cu"
+SRCS="api.cu select.cu score.cu score_runs.cu coverage.cu pileup_atomic.cu pileup_bitsliced.cu consensus.cu contig_stats.cu hamming.cu hamming_exact.cu hamming_tc.cu st_match.cu ingest.cu de.cu allreduce.cu exchange.cu"
 OBJS=""
 for s in $SRCS; do
   o="${s%.cu}.o"

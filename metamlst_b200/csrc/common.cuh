@@ -94,6 +94,17 @@ __device__ __forceinline__ void tl_mark(unsigned long long* tl, uint32_t base, u
 
 __device__ __forceinline__ uint32_t lane_id() { return threadIdx.x & 31u; }
 
+// cmseq's majority call of a recorded column (cmseq/cmseq.py:202-209): max(sorted(freq), key=freq.get) is the first maximum in the
+// order A, C, G, N, T, and N competes with the bases (H8).  The consensus kernels and the contig statistics share it.
+__device__ __forceinline__ uint8_t mmlst_majority_call(uint32_t A, uint32_t C, uint32_t G, uint32_t T, uint32_t N) {
+    uint32_t best = A; uint8_t call = 'A';
+    if (C > best) { best = C; call = 'C'; }
+    if (G > best) { best = G; call = 'G'; }
+    if (N > best) { best = N; call = 'N'; }
+    if (T > best) { best = T; call = 'T'; }
+    return call;
+}
+
 // streaming 128-bit load: read once, do not pollute L1
 __device__ __forceinline__ uint4 ld_stream_u4(const void* p) {
     uint4 r;

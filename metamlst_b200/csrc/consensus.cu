@@ -28,15 +28,7 @@ __global__ void __launch_bounds__(CONS_THREADS) consensus_kernel(uint32_t* __res
         uint32_t* c = counts + static_cast<size_t>(col) * 5;
         const uint32_t A = c[0], C = c[1], G = c[2], T = c[3], N = c[4];
         if (CONSUME) { c[0] = 0; c[1] = 0; c[2] = 0; c[3] = 0; c[4] = 0; }  // the next pass accumulates from zero without a memset
-        uint8_t call = 'N';
-        if (A + C + G + T >= mincov && (A | C | G | T | N)) {
-            // max(sorted(freq), key=freq.get): first maximum in the order A, C, G, N, T (H8)
-            uint32_t best = A; call = 'A';
-            if (C > best) { best = C; call = 'C'; }
-            if (G > best) { best = G; call = 'G'; }
-            if (N > best) { best = N; call = 'N'; }
-            if (T > best) { best = T; call = 'T'; }
-        }
+        const uint8_t call = (A + C + G + T >= mincov && (A | C | G | T | N)) ? mmlst_majority_call(A, C, G, T, N) : 'N';
         const uint8_t db = db_base[col];
         uint8_t out;
         if (call == 'N') { out = (db >= 'A' && db <= 'Z') ? db + 32 : db; ++h; }

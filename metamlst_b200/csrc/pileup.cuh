@@ -29,14 +29,7 @@ __device__ __forceinline__ void consensus_of_locus(uint32_t* counts, const uint8
         uint32_t* c = counts + static_cast<size_t>(col) * 5;
         const uint32_t A = __ldcg(c + 0), C = __ldcg(c + 1), G = __ldcg(c + 2), T = __ldcg(c + 3), N = __ldcg(c + 4);
         if (consume) { c[0] = 0; c[1] = 0; c[2] = 0; c[3] = 0; c[4] = 0; }
-        uint8_t call = 'N';
-        if (A + C + G + T >= mincov && (A | C | G | T | N)) {
-            uint32_t best = A; call = 'A';   // first maximum in the order A, C, G, N, T (H8)
-            if (C > best) { best = C; call = 'C'; }
-            if (G > best) { best = G; call = 'G'; }
-            if (N > best) { best = N; call = 'N'; }
-            if (T > best) { best = T; call = 'T'; }
-        }
+        const uint8_t call = (A + C + G + T >= mincov && (A | C | G | T | N)) ? mmlst_majority_call(A, C, G, T, N) : 'N';
         const uint8_t db = db_base[col];
         uint8_t out;
         if (call == 'N') { out = (db >= 'A' && db <= 'Z') ? db + 32 : db; ++h; }

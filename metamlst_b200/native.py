@@ -65,6 +65,19 @@ class SampleResult(C.Structure):   # mmlst_sample_result
                 ("sum_as", C.c_void_p), ("n_hit", C.c_void_p), ("first_idx", C.c_void_p)]
 
 
+class ContigStatsParams(C.Structure):   # mmlst_contig_stats_params
+    _fields_ = [("mode", C.c_uint32), ("mincov", C.c_uint32), ("trunc", C.c_uint32), ("none_char", C.c_uint32), ("dominant_frq_thrsh", C.c_double)]
+
+
+class ContigStatsOut(C.Structure):   # mmlst_contig_stats_out
+    _fields_ = [("sel_off", C.c_void_p), ("low_off", C.c_void_p), ("depth_off", C.c_void_p), ("out_col", C.c_void_p), ("out_val", C.c_void_p),
+                ("cons", C.c_void_p), ("capacity", C.c_uint64), ("n_out", C.c_uint64)]
+
+
+STATS_COLUMNS, STATS_DEPTH, STATS_LOWDOM = 0, 1, 2   # include/mmlst.h MMLST_STATS_*
+CONTIG_STATS_MAX_COLS = 858993459                     # MMLST_CONTIG_STATS_MAX_COLS
+
+
 EXPORTS = {
     # name: (restype, argtypes)
     "mmlst_last_error": (C.c_char_p, []),
@@ -117,6 +130,11 @@ EXPORTS = {
     "mmlst_pileup_consensus_indirect_dev": (C.c_int, [C.c_void_p] * 4 + [C.c_uint32, C.c_int, C.c_int, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_uint32,
                                                       C.c_uint32, C.c_void_p, C.c_void_p, C.c_void_p, C.c_uint32, C.c_void_p, C.c_void_p]),
     "mmlst_chunk_records": (C.c_uint32, [C.c_uint64]),
+    "mmlst_contig_stats_scratch_bytes": (C.c_size_t, [C.c_uint32]),
+    "mmlst_contig_stats_dev": (C.c_int, [C.c_void_p, C.c_void_p, C.c_uint32, C.c_uint32, C.POINTER(ContigStatsParams), C.c_void_p, C.c_size_t]
+                               + [C.c_void_p] * 6 + [C.c_uint32, C.c_void_p]),
+    "mmlst_contig_stats": (C.c_int, [C.c_void_p, C.POINTER(Soa), C.c_void_p, C.c_uint32, C.c_void_p, C.c_int, C.c_int,
+                                     C.POINTER(ContigStatsParams), C.POINTER(ContigStatsOut)]),
     "mmlst_xchg_publish_dev": (C.c_int, [C.c_void_p, C.c_uint32, C.c_void_p, C.c_uint32, C.c_uint32, C.c_uint64, C.c_uint64, C.c_uint64,
                                          C.c_void_p, C.c_void_p]),
     "mmlst_xchg_await_dev": (C.c_int, [C.c_void_p, C.c_uint32, C.c_uint32, C.c_uint64, C.c_uint64, C.c_uint64, C.c_void_p, C.c_void_p,
