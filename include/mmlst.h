@@ -155,13 +155,29 @@ int mmlst_expand_runs_dev(const uint32_t* run_tid, const uint32_t* run_start, ui
  *   table           : device scratch of 24 * table_slots bytes, 16-byte aligned, ZEROED by the caller;
  *                     table_slots = mmlst_coverage_table_slots(upper bound on passing records), a power of two
  *   cov[n_loci]     : ACCUMULATED (caller zeroes); shards that hold whole loci (contig-aligned, SURVEY.md 8e) add up
+ *   file index      : orig_idx[i] when given, else idx_base + i; idx_base + n_rec must stay below 2^48 (MMLST_E_RANGE)
  * Same filter as mmlst_score_dev (allow, minscore, max_xm, min_read_len).
+ * mmlst_coverage_dev = mmlst_coverage_insert_dev then mmlst_coverage_sum_dev (same arguments; the insert pass ignores cov).
+ * Shards that cut through loci (record ranges) run the passes apart and, in between, mmlst_coverage_merge_dev with the
+ * occupied slots of every other shard's table (keys[m][2] = the 16-byte key words, vals[m] = the value words, both as
+ * the table holds them; {0,0} keys are skipped): a local slot whose key is listed takes the larger value word, absent
+ * keys are ignored.  Then only the shard holding the globally last record of a name adds it, and the shards' cov add up.
  * --------------------------------------------------------------------------------------------------------------- */
 uint64_t mmlst_coverage_table_slots(uint64_t n_names_upper_bound);
 int mmlst_coverage_dev(const uint32_t* tid, const int16_t* as0, const uint8_t* xm3, const uint16_t* qlen,
                        const uint32_t* orig_idx, const uint64_t* qhash, uint64_t n_rec, uint64_t idx_base,
                        const uint8_t* allow, const uint32_t* locus_of, uint32_t n_ref, int minscore, int max_xm,
                        int min_read_len, void* table, uint64_t table_slots, uint64_t* cov, void* stream);
+int mmlst_coverage_insert_dev(const uint32_t* tid, const int16_t* as0, const uint8_t* xm3, const uint16_t* qlen,
+                              const uint32_t* orig_idx, const uint64_t* qhash, uint64_t n_rec, uint64_t idx_base,
+                              const uint8_t* allow, const uint32_t* locus_of, uint32_t n_ref, int minscore, int max_xm,
+                              int min_read_len, void* table, uint64_t table_slots, uint64_t* cov, void* stream);
+int mmlst_coverage_sum_dev(const uint32_t* tid, const int16_t* as0, const uint8_t* xm3, const uint16_t* qlen,
+                           const uint32_t* orig_idx, const uint64_t* qhash, uint64_t n_rec, uint64_t idx_base,
+                           const uint8_t* allow, const uint32_t* locus_of, uint32_t n_ref, int minscore, int max_xm,
+                           int min_read_len, void* table, uint64_t table_slots, uint64_t* cov, void* stream);
+int mmlst_coverage_merge_dev(const uint64_t* keys, const uint64_t* vals, uint64_t m, void* table, uint64_t table_slots,
+                             void* stream);
 
 /* ---------------------------------------------------------------------------------------------------------------
  * Stage 2 -- pileup base counts.  Replaces cmseq/cmseq.py:527-548 (+ htslib pileup rules H1-H3 applied at unpack).

@@ -10,6 +10,9 @@
 //   pass 1  insert_kernel : every passing record -> claim/find its (locus, name) slot, atomicMax the value
 //   pass 2  sum_kernel    : every passing record looks its slot up again; the one record whose index IS the maximum
 //                           adds its len(SEQ) to cov[locus] (warp-aggregated when the warp is on one locus)
+// Record shards that cut through loci (a contiguous range of the sorted stream per rank) run the passes apart: between
+// them every rank raises its own slots to the maximum any rank holds for the key (merge_kernel over the other ranks'
+// occupied slots), so that only the rank holding the globally last record of a name adds it.
 // Random 32-byte sector traffic, not a streaming kernel: it is off the headline pass and run only when the coverage
 // column is wanted.
 #include "common.cuh"
@@ -18,6 +21,7 @@ namespace {
 
 constexpr int kThreads = 256;
 constexpr uint32_t FULL = 0xffffffffu;
+constexpr uint64_t kMaxIdx = (1ull << 48) - 1;  // value word: (file index + 1) << 16 | len(SEQ)
 
 struct __align__(16) Key128 { unsigned long long lo, hi; };
 
@@ -65,8 +69,11 @@ __device__ __forceinline__ Rec load_rec(const CovArgs& a, uint64_t i) {
     r.locus = a.locus_of[t];
     r.ql = static_cast<uint32_t>(ql);
     r.key.lo = a.qhash[2 * i];
-    r.key.hi = a.qhash[2 * i + 1] ^ (static_cast<unsigned long long>(r.locus + 1u) * 0x9E3779B97F4A7C15ull);  // one set per locus
-    if ((r.key.lo | r.key.hi) == 0ull) r.key.lo = 1ull;  // {0,0} is the empty slot
+    const unsigned long long fold = static_cast<unsigned long long>(r.locus + 1u) * 0x9E3779B97F4A7C15ull;  // one set per locus
+    r.key.hi = a.qhash[2 * i + 1] ^ fold;
+    // {0,0} is the empty slot: remap it to {1, fold}, the key of the hash {1, 0} on the SAME locus (a collision of the 128-bit
+    // hash, like any other), never to a key shared by every locus.  fold != 0: locus + 1 < 2^32 times an odd constant.
+    if ((r.key.lo | r.key.hi) == 0ull) { r.key.lo = 1ull; r.key.hi = fold; }
     const unsigned long long idx = a.orig_idx ? static_cast<unsigned long long>(a.orig_idx[i]) : (a.idx_base + i);
     r.val = ((idx + 1ull) << 16) | static_cast<unsigned long long>(r.ql);
     r.slot = mix64(r.key.lo ^ mix64(r.key.hi)) & a.mask;
@@ -125,6 +132,75 @@ __global__ void __launch_bounds__(kThreads) cov_sum_kernel(const CovArgs a) {
     }
 }
 
+__global__ void __launch_bounds__(kThreads) cov_merge_kernel(const Key128* __restrict__ in_keys, const unsigned long long* __restrict__ in_vals,
+                                                             uint64_t m, Key128* keys, unsigned long long* vals, uint64_t mask) {
+    const uint64_t stride = static_cast<uint64_t>(gridDim.x) * blockDim.x;
+    for (uint64_t j = static_cast<uint64_t>(blockIdx.x) * blockDim.x + threadIdx.x; j < m; j += stride) {
+        const Key128 k = in_keys[j];
+        if ((k.lo | k.hi) == 0ull) continue;  // padding / empty slot of the sender
+        uint64_t s = mix64(k.lo ^ mix64(k.hi)) & mask;
+        for (uint64_t probe = 0; probe <= mask; ++probe, s = (s + 1) & mask) {
+            const Key128 cur = ld128(keys + s);
+            if (cur.lo == k.lo && cur.hi == k.hi) {
+                atomicMax(vals + s, in_vals[j]);
+                break;
+            }
+            if ((cur.lo | cur.hi) == 0ull) break;  // no local record has the name: nothing to decide here
+        }
+    }
+}
+
+uint32_t grid_for(uint64_t n) {
+    const uint64_t want = (n + kThreads - 1) / kThreads;
+    const uint64_t cap = static_cast<uint64_t>(mmlst_num_sms()) * 16u;
+    return static_cast<uint32_t>(want < cap ? want : cap);
+}
+
+int check_table(const char* who, const void* table, uint64_t table_slots) {
+    if (!table) {
+        mmlst_set_error("%s: null pointer", who);
+        return MMLST_E_ARG;
+    }
+    if (table_slots < 2 || (table_slots & (table_slots - 1)) || (reinterpret_cast<uintptr_t>(table) & 15)) {
+        mmlst_set_error("%s: table_slots must be a power of two and the table 16-byte aligned", who);
+        return MMLST_E_ARG;
+    }
+    return MMLST_OK;
+}
+
+// pass: 1 = insert, 2 = sum, 3 = both
+int coverage_passes(const char* who, int pass, const uint32_t* tid, const int16_t* as0, const uint8_t* xm3, const uint16_t* qlen,
+                    const uint32_t* orig_idx, const uint64_t* qhash, uint64_t n_rec, uint64_t idx_base, const uint8_t* allow,
+                    const uint32_t* locus_of, uint32_t n_ref, int minscore, int max_xm, int min_read_len, void* table,
+                    uint64_t table_slots, uint64_t* cov, void* stream) {
+    if (n_rec == 0) return MMLST_OK;
+    if (!tid || !as0 || !xm3 || !qlen || !qhash || !allow || !locus_of || ((pass & 2) && !cov)) {
+        mmlst_set_error("%s: null pointer", who);
+        return MMLST_E_ARG;
+    }
+    if (int rc = check_table(who, table, table_slots)) return rc;
+    if (!orig_idx && (idx_base >= kMaxIdx || n_rec > kMaxIdx - idx_base)) {  // (idx + 1) << 16 must not lose bits
+        mmlst_set_error("%s: idx_base + n_rec = %llu exceeds the 48-bit file index of the value word", who,
+                        static_cast<unsigned long long>(idx_base + n_rec));
+        return MMLST_E_RANGE;
+    }
+    CovArgs a{tid, as0, xm3, qlen, orig_idx, reinterpret_cast<const unsigned long long*>(qhash), n_rec, idx_base, allow, locus_of, n_ref,
+              minscore, max_xm, min_read_len, static_cast<Key128*>(table),
+              reinterpret_cast<unsigned long long*>(static_cast<uint8_t*>(table) + 16 * table_slots), table_slots - 1,
+              reinterpret_cast<unsigned long long*>(cov)};
+    cudaStream_t s = static_cast<cudaStream_t>(stream);
+    const uint32_t grid = grid_for(n_rec);
+    if (pass & 1) {
+        cov_insert_kernel<<<grid, kThreads, 0, s>>>(a);
+        if (int rc = mmlst_cuda_fail(cudaGetLastError(), "cov_insert_kernel")) return rc;
+    }
+    if (pass & 2) {
+        cov_sum_kernel<<<grid, kThreads, 0, s>>>(a);
+        if (int rc = mmlst_cuda_fail(cudaGetLastError(), "cov_sum_kernel")) return rc;
+    }
+    return MMLST_OK;
+}
+
 }  // namespace
 
 extern "C" uint64_t mmlst_coverage_table_slots(uint64_t n_names_upper_bound) {
@@ -137,24 +213,36 @@ extern "C" int mmlst_coverage_dev(const uint32_t* tid, const int16_t* as0, const
                                   const uint32_t* orig_idx, const uint64_t* qhash, uint64_t n_rec, uint64_t idx_base,
                                   const uint8_t* allow, const uint32_t* locus_of, uint32_t n_ref, int minscore, int max_xm,
                                   int min_read_len, void* table, uint64_t table_slots, uint64_t* cov, void* stream) {
-    if (n_rec == 0) return MMLST_OK;
-    if (!tid || !as0 || !xm3 || !qlen || !qhash || !allow || !locus_of || !table || !cov) {
-        mmlst_set_error("mmlst_coverage_dev: null pointer");
+    return coverage_passes("mmlst_coverage_dev", 3, tid, as0, xm3, qlen, orig_idx, qhash, n_rec, idx_base, allow, locus_of, n_ref,
+                           minscore, max_xm, min_read_len, table, table_slots, cov, stream);
+}
+
+extern "C" int mmlst_coverage_insert_dev(const uint32_t* tid, const int16_t* as0, const uint8_t* xm3, const uint16_t* qlen,
+                                         const uint32_t* orig_idx, const uint64_t* qhash, uint64_t n_rec, uint64_t idx_base,
+                                         const uint8_t* allow, const uint32_t* locus_of, uint32_t n_ref, int minscore, int max_xm,
+                                         int min_read_len, void* table, uint64_t table_slots, uint64_t* cov, void* stream) {
+    return coverage_passes("mmlst_coverage_insert_dev", 1, tid, as0, xm3, qlen, orig_idx, qhash, n_rec, idx_base, allow, locus_of, n_ref,
+                           minscore, max_xm, min_read_len, table, table_slots, cov, stream);
+}
+
+extern "C" int mmlst_coverage_sum_dev(const uint32_t* tid, const int16_t* as0, const uint8_t* xm3, const uint16_t* qlen,
+                                      const uint32_t* orig_idx, const uint64_t* qhash, uint64_t n_rec, uint64_t idx_base,
+                                      const uint8_t* allow, const uint32_t* locus_of, uint32_t n_ref, int minscore, int max_xm,
+                                      int min_read_len, void* table, uint64_t table_slots, uint64_t* cov, void* stream) {
+    return coverage_passes("mmlst_coverage_sum_dev", 2, tid, as0, xm3, qlen, orig_idx, qhash, n_rec, idx_base, allow, locus_of, n_ref,
+                           minscore, max_xm, min_read_len, table, table_slots, cov, stream);
+}
+
+extern "C" int mmlst_coverage_merge_dev(const uint64_t* keys, const uint64_t* vals, uint64_t m, void* table, uint64_t table_slots,
+                                        void* stream) {
+    if (m == 0) return MMLST_OK;
+    if (!keys || !vals || (reinterpret_cast<uintptr_t>(keys) & 15)) {
+        mmlst_set_error("mmlst_coverage_merge_dev: keys must be non-null and 16-byte aligned, vals non-null");
         return MMLST_E_ARG;
     }
-    if (table_slots < 2 || (table_slots & (table_slots - 1)) || (reinterpret_cast<uintptr_t>(table) & 15)) {
-        mmlst_set_error("mmlst_coverage_dev: table_slots must be a power of two and the table 16-byte aligned");
-        return MMLST_E_ARG;
-    }
-    CovArgs a{tid, as0, xm3, qlen, orig_idx, reinterpret_cast<const unsigned long long*>(qhash), n_rec, idx_base, allow, locus_of, n_ref,
-              minscore, max_xm, min_read_len, static_cast<Key128*>(table),
-              reinterpret_cast<unsigned long long*>(static_cast<uint8_t*>(table) + 16 * table_slots), table_slots - 1,
-              reinterpret_cast<unsigned long long*>(cov)};
-    cudaStream_t s = static_cast<cudaStream_t>(stream);
-    const uint64_t want = (n_rec + kThreads - 1) / kThreads;
-    const uint32_t grid = static_cast<uint32_t>(want < static_cast<uint64_t>(mmlst_num_sms()) * 16u ? want : static_cast<uint64_t>(mmlst_num_sms()) * 16u);
-    cov_insert_kernel<<<grid, kThreads, 0, s>>>(a);
-    if (int rc = mmlst_cuda_fail(cudaGetLastError(), "cov_insert_kernel")) return rc;
-    cov_sum_kernel<<<grid, kThreads, 0, s>>>(a);
-    return mmlst_cuda_fail(cudaGetLastError(), "cov_sum_kernel");
+    if (int rc = check_table("mmlst_coverage_merge_dev", table, table_slots)) return rc;
+    cov_merge_kernel<<<grid_for(m), kThreads, 0, static_cast<cudaStream_t>(stream)>>>(
+        reinterpret_cast<const Key128*>(keys), reinterpret_cast<const unsigned long long*>(vals), m, static_cast<Key128*>(table),
+        reinterpret_cast<unsigned long long*>(static_cast<uint8_t*>(table) + 16 * table_slots), table_slots - 1);
+    return mmlst_cuda_fail(cudaGetLastError(), "cov_merge_kernel");
 }

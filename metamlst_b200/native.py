@@ -78,6 +78,9 @@ STATS_COLUMNS, STATS_DEPTH, STATS_LOWDOM = 0, 1, 2   # include/mmlst.h MMLST_STA
 CONTIG_STATS_MAX_COLS = 858993459                     # MMLST_CONTIG_STATS_MAX_COLS
 
 
+_COVERAGE_ARGS = [C.c_void_p] * 6 + [C.c_uint64, C.c_uint64, C.c_void_p, C.c_void_p, C.c_uint32, C.c_int, C.c_int, C.c_int, C.c_void_p,
+                                      C.c_uint64, C.c_void_p, C.c_void_p]   # mmlst_coverage_dev and its two passes
+
 EXPORTS = {
     # name: (restype, argtypes)
     "mmlst_last_error": (C.c_char_p, []),
@@ -108,8 +111,10 @@ EXPORTS = {
     "mmlst_set_pdl": (C.c_int, [C.c_int]),
     "mmlst_expand_runs_dev": (C.c_int, [C.c_void_p, C.c_void_p, C.c_uint32, C.c_void_p, C.c_uint64, C.c_void_p, C.c_void_p]),
     "mmlst_coverage_table_slots": (C.c_uint64, [C.c_uint64]),
-    "mmlst_coverage_dev": (C.c_int, [C.c_void_p] * 6 + [C.c_uint64, C.c_uint64, C.c_void_p, C.c_void_p, C.c_uint32, C.c_int, C.c_int,
-                                     C.c_int, C.c_void_p, C.c_uint64, C.c_void_p, C.c_void_p]),
+    "mmlst_coverage_dev": (C.c_int, _COVERAGE_ARGS),
+    "mmlst_coverage_insert_dev": (C.c_int, _COVERAGE_ARGS),
+    "mmlst_coverage_sum_dev": (C.c_int, _COVERAGE_ARGS),
+    "mmlst_coverage_merge_dev": (C.c_int, [C.c_void_p, C.c_void_p, C.c_uint64, C.c_void_p, C.c_uint64, C.c_void_p]),
     "mmlst_coverage": (C.c_int, [C.c_void_p, C.POINTER(Soa), C.c_void_p, C.c_void_p, C.c_void_p, C.c_uint32, C.POINTER(ScoreParams),
                                  C.c_uint32, C.c_void_p]),
     "mmlst_pileup_dev": (C.c_int, [C.c_void_p] * 3 + [C.c_uint32, C.c_uint32, C.c_int, C.c_int, C.c_void_p, C.c_uint32,

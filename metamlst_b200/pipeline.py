@@ -214,33 +214,100 @@ class DevicePipeline:
         if self.dist and not self.owner:
             dist.allreduce_score_block(self.zscore, self.first_idx, self.group)
 
-    def run_coverage(self, timed: bool = False):
-        """Coverage column (H7, metamlst.py:127,228) of the resident score stream: {'species_gene': bases}.  Needs streams
-        packed with the 128-bit QNAME keys.  Contig-aligned shards hold whole loci, so ranks just add their tables."""
+    # -- coverage column (H7, metamlst.py:127,228), csrc/coverage.cu.  run_coverage is the whole of it; the four steps below are
+    # what it runs on a record shard that cuts through loci, exposed so that shards can be driven one after another in one process.
+    def _cov_call(self, fn):
+        s = self.s
+        native.check(fn(native.ptr(s.tid), native.ptr(s.as0), native.ptr(s.xm3), native.ptr(s.qlen),
+                        native.ptr(getattr(s, "orig_idx", None)),  # file-order index per record, exactly as _score_call passes it
+                        native.ptr(s.qhash), int(s.tid.shape[0]), self.idx_base, native.ptr(self.allow), native.ptr(self.locus_of), self.n_ref,
+                        self.minscore, self.max_xM, self.min_read_len, native.ptr(self._cov_table), self._cov_slots, native.ptr(self._cov),
+                        self._stream()))
+
+    def _coverage_reset(self):
         s = self.s
         if getattr(s, "qhash", None) is None:
             raise ValueError("streams were packed without QNAME keys (want_qhash)")
-        n = int(s.tid.shape[0])
-        slots = int(self.lib.mmlst_coverage_table_slots(n))
-        if getattr(self, "_cov_table", None) is None or self._cov_table.shape[0] < slots * 3:
-            self._cov_table = torch.empty(slots * 3, dtype=torch.int64, device=self.dev)
+        self._cov_slots = int(self.lib.mmlst_coverage_table_slots(int(s.tid.shape[0])))
+        if getattr(self, "_cov_table", None) is None or self._cov_table.shape[0] < self._cov_slots * 3:
+            self._cov_table = torch.empty(self._cov_slots * 3, dtype=torch.int64, device=self.dev)
             self._cov = torch.zeros(self.index.n_loci, dtype=torch.int64, device=self.dev)
+        self._cov_table[: self._cov_slots * 3].zero_(); self._cov.zero_()
+
+    def coverage_insert(self, reset: bool = True):
+        """Zeroes the (locus, QNAME) table and the per-locus sums (unless `reset` is False), then inserts every passing record
+        of this shard: afterwards each slot holds the largest value word, (file index + 1) << 16 | len(SEQ), among this
+        shard's records of the name."""
+        if reset:
+            self._coverage_reset()
+        self._cov_call(self.lib.mmlst_coverage_insert_dev)
+        self.launches += 1
+
+    def coverage_entries(self) -> torch.Tensor:
+        """The occupied slots of the table as one int64 tensor [m][3]: key words (2) and value word."""
+        n = self._cov_slots
+        keys = self._cov_table[: 2 * n].view(n, 2)
+        occ = (keys != 0).any(1)
+        return torch.cat([keys[occ], self._cov_table[2 * n: 3 * n][occ].view(-1, 1)], 1)
+
+    def coverage_merge(self, entries: torch.Tensor):
+        """Raise this shard's slots to the value words of the same keys in `entries` (another shard's coverage_entries, any
+        number of rows; rows of zeros are skipped).  Keys this shard does not hold are ignored."""
+        m = int(entries.shape[0])
+        if m == 0:
+            return
+        keys = entries[:, :2].contiguous()
+        vals = entries[:, 2].contiguous()
+        native.check(self.lib.mmlst_coverage_merge_dev(native.ptr(keys), native.ptr(vals), m, native.ptr(self._cov_table), self._cov_slots,
+                                                       self._stream()))
+        self.launches += 1
+
+    def coverage_sum(self) -> torch.Tensor:
+        """Sum pass: every record that IS the last of its name (value word equal to its slot's) adds len(SEQ) to its locus.
+        Returns the per-locus sums of this shard (int64 [n_loci], on the device)."""
+        self._cov_call(self.lib.mmlst_coverage_sum_dev)
+        self.launches += 1
+        return self._cov
+
+    def _exchange_coverage_entries(self):
+        """Every rank's occupied slots to every rank (all-gather, padded with zero rows to the largest rank), merged here."""
+        mine = self.coverage_entries()
+        cnt = torch.tensor([int(mine.shape[0])], dtype=torch.int64, device=self.dev)
+        cnts = torch.zeros(self.world, dtype=torch.int64, device=self.dev)
+        torch.distributed.all_gather_into_tensor(cnts, cnt, group=self.group)
+        m = int(cnts.max().item())
+        if m == 0:
+            return
+        pad = torch.zeros((m, 3), dtype=torch.int64, device=self.dev)
+        pad[: mine.shape[0]] = mine
+        every = torch.zeros((self.world * m, 3), dtype=torch.int64, device=self.dev)
+        torch.distributed.all_gather_into_tensor(every, pad, group=self.group)
+        rank = torch.distributed.get_rank(self.group)
+        for r in range(self.world):
+            if r != rank:
+                self.coverage_merge(every[r * m:(r + 1) * m])
+
+    def run_coverage(self, timed: bool = False):
+        """Coverage column (H7, metamlst.py:127,228) of the resident score stream: {'species_gene': bases}.  Needs streams
+        packed with the 128-bit QNAME keys.  Owner-mode shards ("loci") hold whole loci, so ranks just add their sums.  Record
+        shards ("ranges") can split the records of one name over several ranks: between the insert and the sum pass every rank
+        merges the others' table entries, so that exactly one rank -- the one holding the name's last record in file order --
+        adds it, and the sums add up again."""
         ev = [torch.cuda.Event(enable_timing=True) for _ in range(3)]
         ev[0].record()
-        self._cov_table[: slots * 3].zero_(); self._cov.zero_()
+        self._coverage_reset()
         ev[1].record()
-        native.check(self.lib.mmlst_coverage_dev(native.ptr(s.tid), native.ptr(s.as0), native.ptr(s.xm3), native.ptr(s.qlen), 0, native.ptr(s.qhash),
-                                                 n, self.idx_base, native.ptr(self.allow), native.ptr(self.locus_of), self.n_ref, self.minscore,
-                                                 self.max_xM, self.min_read_len, native.ptr(self._cov_table), slots, native.ptr(self._cov),
-                                                 self._stream()))
+        self.coverage_insert(reset=False)
+        if self.dist and not self.owner:
+            self._exchange_coverage_entries()
+        self.coverage_sum()
         ev[2].record()
-        self.launches += 2
         if self.dist:
             torch.distributed.all_reduce(self._cov, group=self.group)
         cov = self._cov.cpu().numpy()
         out = {sp + "_" + g: int(cov[l]) for l, (sp, g) in enumerate(self.index.locus_names) if cov[l]}
         if timed:
-            return out, {"memset_ms": ev[0].elapsed_time(ev[1]), "kernels_ms": ev[1].elapsed_time(ev[2]), "table_bytes": slots * 24}
+            return out, {"memset_ms": ev[0].elapsed_time(ev[1]), "kernels_ms": ev[1].elapsed_time(ev[2]), "table_bytes": self._cov_slots * 24}
         return out
 
     def select(self):

@@ -7,7 +7,9 @@ shard a rank types:
   "ranges"  any record sharding (SURVEY.md 8e, north_star: "reads are sharded across the GPUs ... partial pileup-count and score
             tensors are allreduced"): rank r takes a contiguous range of the score stream (file-order indices kept through
             idx_base / orig_idx) and a contiguous range of the pileup stream.  The htslib depth cap was resolved at unpack over
-            the WHOLE sample, i.e. before sharding, so counts add up exactly.  Goes with exchange="allreduce".
+            the WHOLE sample, i.e. before sharding, so counts add up exactly.  Goes with exchange="allreduce".  The records of one
+            read name can fall on both sides of a cut: the coverage column merges the ranks' name tables before it adds their sums
+            (DevicePipeline.run_coverage).
   "loci"    contig-aligned shards: rank r takes the score-stream records of loci l with l % world == r (orig_idx made explicit)
             and keeps the whole (depth-capped, hence small) pileup stream; it only ever chooses -- and piles up -- contigs of
             its own loci.  Goes with the owner-mode exchanges ("p2p", "gather").
