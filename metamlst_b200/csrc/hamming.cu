@@ -227,6 +227,10 @@ extern "C" int mmlst_hamming_min_dev2(const uint32_t* db_hi, const uint32_t* db_
         mmlst_set_error("mmlst_hamming_min_dev: query planes must be 16-byte aligned");
         return MMLST_E_ARG;
     }
+    // 0 = not known: every block may span all rows / all queries (as the any-width path reads it).  A call whose blocks are all
+    // empty then launches CTAs that exit at once and leaves best[] at the caller's "no row" preset, instead of a grid of size 0.
+    if (max_block_rows == 0) max_block_rows = n_rows;
+    if (max_block_queries == 0) max_block_queries = n_q;
     cudaStream_t s = static_cast<cudaStream_t>(stream);
     for (uint32_t b0 = 0; b0 < n_blocks; b0 += 65535u) {   // gridDim.y holds 65535 blocks: more go out in slices
         const uint32_t nb = n_blocks - b0 < 65535u ? n_blocks - b0 : 65535u;

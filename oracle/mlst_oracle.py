@@ -400,27 +400,21 @@ class OracleDB:
 
     def define_profile(self, labels: Sequence[str]) -> List[Tuple[int, int]]:
         """metaMLST_functions.py:205-216 incl. its quirks (H11): unknown labels silently shrink the denominator;
-        `[(0,0)]` only when the LAST lookup failed."""
+        `[(0,0)]` only when the LAST lookup failed.  The ST statement is the reference's, verbatim: the order of tied profiles
+        (`ORDER BY T DESC` leaves them in descending profileCode order in SQLite 3.x) is whatever that statement returns, and the
+        merge takes the first of them."""
         recs = []
         result = None
         for label in labels:
             result = self.conn.execute("SELECT recID FROM alleles WHERE bacterium||'_'||gene||'_'||alleleVariant = ?", (label,)).fetchone()
             if result:
-                recs.append(int(result["recID"]))
+                recs.append(str(result["recID"]))
         if not result:
             return [(0, 0)]
-        counts: Dict[int, int] = {}
-        order: List[int] = []
-        q = "SELECT profileCode, alleleCode FROM profiles WHERE alleleCode IN (%s) ORDER BY profileCode" % ",".join(str(x) for x in recs)
-        for row in self.conn.execute(q):
-            if row["profileCode"] not in counts:
-                counts[row["profileCode"]] = 0
-                order.append(row["profileCode"])
-            counts[row["profileCode"]] += 1
-        if not counts:
-            return []
-        top = max(counts.values())
-        return [(pc, int((float(top) / float(len(recs))) * 100)) for pc in order if counts[pc] == top]
+        inl = ",".join(recs)
+        q = ("SELECT profileCode, COUNT(*) as T FROM profiles WHERE alleleCode IN (" + inl + ") GROUP BY profileCode HAVING T = "
+             "(SELECT COUNT(*) FROM profiles WHERE alleleCode IN (" + inl + ") GROUP BY profileCode ORDER BY COUNT(*) DESC LIMIT 1) ORDER BY T DESC")
+        return [(row[0], int((float(row[1]) / float(len(recs))) * 100)) for row in self.conn.execute(q)]
 
 
 def string_diff(s1: str, s2: str) -> int:
