@@ -693,6 +693,58 @@ void mmlst_dev_bam_free(mmlst_dev_bam* bam);
  * this gives the idle blocks back to the driver */
 int mmlst_ingest_trim(int device);
 
+/* ---------------------------------------------------------------------------------------------------------------
+ * ONE BAM over W ranks (metamlst_b200/bam.py ingest_bam_sharded drives these calls and the collectives between them).  The
+ * whole-file ingest above is split where the records are known:
+ *   front half (rank r): the rank's own contiguous range of BGZF blocks, followed by a HALO of the next blocks so that the last
+ *     record starting in its range can end there, is inflated (check_crc: the CRC32 of the own blocks); the record chain is walked
+ *     from an entry point the ranks agree on (rank r's entry = rank r-1's exit, by the guess-and-verify rule of the record chain);
+ *     the records that START in the own blocks are grouped by owner rank, stable in file order (the partition kernel).
+ *   exchange: per-destination counts, the raw record bytes, their lengths and shard-relative indices (all-to-all).
+ *   back half (owner): parse -> sort (stable by key, then file index) -> score stream -> depth cap -> plane rows, exactly the
+ *     whole-file ingest's; orig_idx is always the explicit file index, contig_start covers all n_ref contigs (those of other owners
+ *     are empty).
+ * Refusals are not raised by a front / back call alone: they come back as error words that the ranks reduce to their minimum
+ * (phase << 56 | index << 8 | code; phase 0 = BGZF block, 1 = record, 2 = --presorted order, 3 = plane array size, 4 = pileup
+ * record) before mmlst_ingest_refusal turns the winner into the whole-file ingest's code and text.
+ * --------------------------------------------------------------------------------------------------------------- */
+typedef struct mmlst_ingest_front mmlst_ingest_front;
+typedef struct {
+    uint64_t n_blocks, n_own_blocks;   /* non-empty blocks in the buffer / in the own range */
+    uint64_t own_inflated, inflated, compressed;   /* inflated bytes of the own blocks / of the whole buffer; compressed bytes of the buffer */
+    uint64_t block_error;              /* (block << 8 | code), block counted in the buffer; ~0 = none */
+    uint64_t entry, exit;              /* inflated offsets in the buffer: first record / where the chain leaves the own range; ~0 = broken */
+    uint64_t need;                     /* > inflated: the halo is too short, the last record needs a buffer of this many inflated bytes */
+    uint64_t n_rec;                    /* records starting in the own range */
+    uint64_t chain_error;              /* (shard record << 8 | code) of a malformed record; ~0 = none */
+    uint32_t repairs; int world;
+    const uint8_t* send;               /* DEVICE: records grouped by destination rank, file order inside a group */
+    const uint32_t* send_len;          /* DEVICE [n_rec]: byte length of every sent record */
+    const uint32_t* send_idx;          /* DEVICE [n_rec]: its index among the shard's records */
+    const uint64_t* dest_records;      /* HOST [world] */
+    const uint64_t* dest_bytes;        /* HOST [world] */
+    int unsorted;                      /* two neighbouring records of the shard out of coordinate order */
+    uint64_t first_key, last_key;      /* (tid << 32 | pos + 1) of the shard's first / last record */
+    double seconds[3];                 /* host wall time: open (H2D + inflate), walks, partition */
+} mmlst_ingest_front_info_t;
+typedef struct {
+    const uint32_t* ref_len; const char* ref_names; const char* header_text; int32_t n_ref;
+    int unsorted;                      /* the FILE is out of coordinate order (any shard, or across a shard boundary): --presorted refuses */
+} mmlst_ingest_back_args;
+/* comp: the rank's compressed bytes (own blocks, then the halo's) in host memory; n_own_bytes: how many of them are the own blocks */
+int mmlst_ingest_front_open(int device, const uint8_t* comp, size_t n_comp, size_t n_own_bytes, const uint32_t* ref_len, int32_t n_ref,
+                            int check_crc, void* stream, mmlst_ingest_front** out);
+/* entry: inflated offset in the buffer of the first record starting in the own range (may lie past it), ~0 = guess */
+int mmlst_ingest_front_walk(mmlst_ingest_front* front, uint64_t entry);
+/* owner[tid]: destination rank of the records of contig tid (records with tid outside the dictionary go to rank 0); world <= 256 */
+int mmlst_ingest_front_partition(mmlst_ingest_front* front, const int32_t* owner, int world);
+int mmlst_ingest_front_info(const mmlst_ingest_front* front, mmlst_ingest_front_info_t* info);
+void mmlst_ingest_front_free(mmlst_ingest_front* front);
+/* recs / rec_len / file_idx: DEVICE, the received records in file order and their file indices */
+int mmlst_bam_ingest_back(int device, const uint8_t* recs, const uint32_t* rec_len, const uint32_t* file_idx, uint64_t n,
+                          const mmlst_ingest_back_args* args, const mmlst_unpack_opts* opts, void* stream, mmlst_dev_bam** out, uint64_t* error_word);
+int mmlst_ingest_refusal(uint64_t error_word);
+
 #ifdef __cplusplus
 }
 #endif

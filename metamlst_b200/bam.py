@@ -182,7 +182,6 @@ def ingest_bam(source, device=0, minqual: int = packing.DEFAULT_MINQUAL, max_dep
     without hardware DEFLATE.  `check_crc`: also check every BGZF block's CRC32 against its trailer on the device, as `unpack_bam`
     always does (MmlstError(MMLST_E_BAM) "CRC mismatch in BGZF block k"); without it the DEFLATE stream and ISIZE are still checked."""
     import torch
-    from . import streams
     dev = torch.device("cuda", device) if isinstance(device, int) else torch.device(device)
     data = read_pinned(source) if isinstance(source, str) else source
     addr = data.data_ptr() if hasattr(data, "data_ptr") else data.ctypes.data
@@ -194,9 +193,15 @@ def ingest_bam(source, device=0, minqual: int = packing.DEFAULT_MINQUAL, max_dep
     with torch.cuda.device(dev):
         stream = torch.cuda.current_stream(dev).cuda_stream
         native.check(lib.mmlst_bam_ingest(dev.index or 0, addr, nbytes, C.byref(o), stream, C.byref(h)))
-    keep = _DevHandle(h)
+    return _dev_streams(_DevHandle(h), dev, want_qhash)
+
+
+def _dev_streams(keep, dev, want_qhash: bool):
+    """streams.DeviceStreams over the arrays of an mmlst_dev_bam handle (no copy: the handle stays alive with the streams)."""
+    import torch
+    from . import streams
     info = DevBamInfo()
-    native.check(lib.mmlst_dev_bam_info(h, C.byref(info)))
+    native.check(native.lib().mmlst_dev_bam_info(keep.h, C.byref(info)))
     n, P, n_ref, nr = int(info.n_rec), int(info.n_prec), int(info.n_ref), int(info.n_runs)
 
     def t(addr_, count, typestr, dtype):
@@ -229,3 +234,24 @@ def ingest_bam(source, device=0, minqual: int = packing.DEFAULT_MINQUAL, max_dep
     s.ingest_stats = {"bgzf_blocks": int(info.n_bgzf_blocks), "compressed_bytes": int(info.compressed_bytes), "inflated_bytes": int(info.inflated_bytes),
                       "boundary_repairs": int(info.boundary_repairs), "unmapped_flag": int(info.n_unmapped_flag)}
     return s
+
+
+def ingest_bam_sharded(path: str, device=0, group=None, locus_of=None, minqual: int = packing.DEFAULT_MINQUAL,
+                       max_depth: Optional[int] = packing.DEFAULT_MAX_DEPTH, presorted: bool = False, want_qhash: bool = True,
+                       sentinel_nodes: int = 1, check_crc: bool = False):
+    """One BAM ingested by every rank of a torch.distributed group (metamlst_b200/shard.py): this rank inflates and parses a 1/W share
+    of the BGZF blocks and returns its streams.DeviceStreams, the records of the loci it owns (locus_of[tid] % W == rank; default:
+    the loci of api.AlleleIndex over the header's reference names) -- what `DeviceStreams.from_soa(unpack_bam(path), mode="loci")`
+    gives, with orig_idx the explicit file index and the pileup stream of the owned contigs only.  Same options and the same refusals
+    as `ingest_bam`: every rank raises the refusal the whole file gives, after the ranks agreed on it."""
+    from . import shard
+    coll = shard.TorchCollective(group)
+    return coll.run(shard.ingest_steps(path, device, coll.rank, coll.world, locus_of=locus_of, minqual=minqual, max_depth=max_depth,
+                                       presorted=presorted, want_qhash=want_qhash, sentinel_nodes=sentinel_nodes, check_crc=check_crc))
+
+
+def ingest_bam_local(path: str, world: int, device=0, **kw):
+    """Every rank of a `world`-rank sharded ingest (ingest_bam_sharded) run in turn in this process on one device: the list of the
+    ranks' streams."""
+    from . import shard
+    return shard.run_local([shard.ingest_steps(path, device, r, world, **kw) for r in range(world)])

@@ -148,33 +148,52 @@ __device__ __forceinline__ void report(unsigned long long* err, uint64_t index, 
 }
 
 // ---- K1: record chain -------------------------------------------------------------------------------------------------------
+// first_record == kNoEntry: no record boundary is known inside the buffer (a shard that starts past the header): every block guesses.
+// uend: where the last block's records stop STARTING (usize, or the end of a shard's own blocks when a halo of the next shard's
+// bytes follows them so that its last record can end there).  need (optional) [b]: after a walk that met a record running past usize,
+// the buffer size that record needs (0 when the walk ended normally or the record is malformed).
+constexpr uint64_t kNoEntry = ~0ull;
 struct ChainArgs {
     const uint8_t* u; uint64_t usize; const uint64_t* uoff; uint32_t n_blocks; uint64_t first_record;
     int32_t n_ref; const uint32_t* ref_len;
     uint64_t* start; uint64_t* exit_; uint32_t* count; uint32_t* bad_walk;   // bad_walk[b] = 1: the walk from start[b] met a malformed record
+    uint64_t uend; uint64_t* need;
 };
 
+__device__ __forceinline__ uint64_t block_end(const ChainArgs& a, uint32_t b) { return (b + 1 < a.n_blocks) ? a.uoff[b + 1] : a.uend; }
+
 __device__ __forceinline__ void walk_block(const ChainArgs& a, uint32_t b, uint64_t s) {
-    const uint64_t bend = (b + 1 < a.n_blocks) ? a.uoff[b + 1] : a.usize;
-    uint64_t off = s;
+    const uint64_t bend = block_end(a, b);
+    uint64_t off = s, need = 0;
     uint32_t cnt = 0, bad = 0;
     while (off < bend) {
         const uint64_t nx = next_record(a.u, off, a.usize);
-        if (nx == 0) { bad = 1; off = a.usize; break; }
+        if (nx == 0) {
+            bad = 1;
+            if (off + 4 > a.usize) need = off + 4;
+            else { const int32_t bs = rdi32(a.u + off); need = bs >= 32 ? off + 4 + static_cast<uint64_t>(bs) : 0; }
+            off = a.usize;
+            break;
+        }
         ++cnt;
         off = nx;
     }
     a.start[b] = s; a.exit_[b] = off; a.count[b] = cnt; a.bad_walk[b] = bad;
+    if (a.need) a.need[b] = need;
 }
 
 __global__ void __launch_bounds__(kT) chain_guess_kernel(const ChainArgs a) {
     const uint32_t b = blockIdx.x * kT + threadIdx.x;
     if (b >= a.n_blocks) return;
     uint64_t s;
-    if (a.uoff[b] <= a.first_record) {
-        const uint64_t bend = (b + 1 < a.n_blocks) ? a.uoff[b + 1] : a.usize;
+    if (a.first_record != kNoEntry && a.uoff[b] <= a.first_record) {
+        const uint64_t bend = block_end(a, b);
         s = a.first_record < bend ? a.first_record : bend;   // header blocks hold no record start before first_record
-        if (a.first_record >= bend) { a.start[b] = bend; a.exit_[b] = bend; a.count[b] = 0; a.bad_walk[b] = 0; return; }
+        if (a.first_record >= bend) {
+            a.start[b] = bend; a.exit_[b] = bend; a.count[b] = 0; a.bad_walk[b] = 0;
+            if (a.need) a.need[b] = 0;
+            return;
+        }
     } else {
         s = a.uoff[b];
         const uint64_t lim = (s + (1ull << 20) < a.usize) ? s + (1ull << 20) : a.usize;
@@ -188,7 +207,7 @@ __global__ void __launch_bounds__(kT) chain_guess_kernel(const ChainArgs a) {
 __global__ void __launch_bounds__(kT) chain_repair_kernel(const ChainArgs a, uint32_t* changed) {
     const uint32_t b = blockIdx.x * kT + threadIdx.x;
     if (b == 0 || b >= a.n_blocks) return;
-    if (a.uoff[b] <= a.first_record) return;
+    if (a.first_record != kNoEntry && a.uoff[b] <= a.first_record) return;
     const uint64_t want = a.exit_[b - 1];
     if (a.start[b] == want) return;
     atomicAdd(changed, 1u);
@@ -198,7 +217,7 @@ __global__ void __launch_bounds__(kT) chain_repair_kernel(const ChainArgs a, uin
 __global__ void __launch_bounds__(kT) chain_offsets_kernel(const ChainArgs a, const uint32_t* base, uint64_t* roff, unsigned long long* err) {
     const uint32_t b = blockIdx.x * kT + threadIdx.x;
     if (b >= a.n_blocks) return;
-    const uint64_t bend = (b + 1 < a.n_blocks) ? a.uoff[b + 1] : a.usize;
+    const uint64_t bend = block_end(a, b);
     uint64_t off = a.start[b];
     uint64_t i = base[b];
     while (off < bend) {
@@ -260,18 +279,82 @@ __global__ void __launch_bounds__(bgzf_crc::kCrcThreads, 4) crc_kernel(const Crc
     }
 }
 
+// ---- shard front half: routing + partition of the raw records by destination rank ------------------------------------------
+// A shard's records go to the rank that owns their contig; a record whose refID is outside the dictionary goes to rank 0, where
+// its refusal is raised exactly as on the whole file.  ord_key is the sort key without its strand bit: what --presorted compares.
+constexpr int kMaxShardRanks = 256;
+
+__device__ __forceinline__ uint64_t ord_key(int32_t tid, int32_t pos) {
+    const uint64_t key = (static_cast<uint64_t>(static_cast<uint32_t>(tid)) << 33) | ((static_cast<uint64_t>(static_cast<uint32_t>(pos)) + 1ull) << 1);
+    return key >> 1;
+}
+
+// dest[i], rlen[i] = 4 + block_size, dcount[d] += records for d; flags[0] = 1 when two neighbours are out of coordinate order;
+// keys[0] / keys[1] = ord_key of the first / last record
+__global__ void __launch_bounds__(kT) route_kernel(const uint8_t* u, const uint64_t* roff, uint64_t n, int32_t n_ref, const int32_t* owner, int world,
+                                                   uint32_t* dest, uint32_t* rlen, unsigned long long* dcount, uint32_t* flags, uint64_t* keys) {
+    __shared__ unsigned long long h[kMaxShardRanks];
+    for (int d = threadIdx.x; d < world; d += kT) h[d] = 0;
+    __syncthreads();
+    const uint64_t i = static_cast<uint64_t>(blockIdx.x) * kT + threadIdx.x;
+    if (i < n) {
+        const uint8_t* r = u + roff[i];
+        const int32_t tid = rdi32(r + 4), pos = rdi32(r + 8);
+        const uint32_t d = (tid >= 0 && tid < n_ref) ? static_cast<uint32_t>(owner[tid]) : 0u;
+        dest[i] = d;
+        rlen[i] = 4u + rd32(r);
+        atomicAdd(&h[d], 1ull);
+        const uint64_t k = ord_key(tid, pos);
+        if (i > 0) {
+            const uint8_t* q = u + roff[i - 1];
+            if (k < ord_key(rdi32(q + 4), rdi32(q + 8))) atomicOr(flags, 1u);
+        }
+        if (i == 0) keys[0] = k;
+        if (i == n - 1) keys[1] = k;
+    }
+    __syncthreads();
+    for (int d = threadIdx.x; d < world; d += kT) if (h[d]) atomicAdd(&dcount[d], h[d]);
+}
+
+__global__ void __launch_bounds__(kT) part_len_kernel(const uint32_t* order, const uint32_t* rlen, uint64_t n, uint64_t* plen) {
+    const uint64_t j = static_cast<uint64_t>(blockIdx.x) * kT + threadIdx.x;
+    if (j < n) plen[j] = rlen[order[j]];
+    if (j == n) plen[j] = 0;
+}
+
+// one warp per record j of the partitioned order: its raw bytes to out + boff[j], its length and its index in the shard to the sidecars
+__global__ void __launch_bounds__(kT) partition_kernel(const uint8_t* u, const uint64_t* roff, const uint32_t* order, const uint32_t* rlen,
+                                                       const uint64_t* boff, uint64_t n, uint8_t* out, uint32_t* out_len, uint32_t* out_idx) {
+    const uint64_t j = (static_cast<uint64_t>(blockIdx.x) * kT + threadIdx.x) >> 5;
+    const uint32_t lane = threadIdx.x & 31u;
+    if (j >= n) return;
+    const uint32_t i = order[j], len = rlen[i];
+    const uint8_t* src = u + roff[i];
+    uint8_t* dst = out + boff[j];
+    for (uint32_t b = lane; b < len; b += 32) dst[b] = src[b];
+    if (lane == 0) { out_len[j] = len; out_idx[j] = i; }
+}
+
+__global__ void __launch_bounds__(kT) widen_kernel(const uint32_t* x, uint64_t n, uint64_t* y) {
+    const uint64_t i = static_cast<uint64_t>(blockIdx.x) * kT + threadIdx.x;
+    if (i < n) y[i] = x[i];
+    if (i == n) y[i] = 0;
+}
+
 // ---- K2: per record ---------------------------------------------------------------------------------------------------------
 struct ParseOut {
     uint64_t* key; uint16_t* reflen; int16_t* as0; int16_t* asn; uint16_t* qlen; uint8_t* xm3; uint8_t* xmn; uint8_t* bits; uint64_t* qh;
 };
 
-__global__ void __launch_bounds__(kT) parse_kernel(const uint8_t* u, const uint64_t* roff, uint64_t n, int32_t n_ref, ParseOut o, unsigned long long* err) {
+// gidx (shards): file index of record i, for the refusal text; nullptr = i
+__global__ void __launch_bounds__(kT) parse_kernel(const uint8_t* u, const uint64_t* roff, const uint32_t* gidx, uint64_t n, int32_t n_ref, ParseOut o,
+                                                   unsigned long long* err) {
     const uint64_t i = static_cast<uint64_t>(blockIdx.x) * kT + threadIdx.x;
     if (i >= n) return;
     Core c;
     uint64_t qh[2];
     const uint32_t e = parse_record(u, roff[i], n_ref, &c, o.qh ? qh : nullptr);
-    if (e != E_NONE) { report(err, i, e); o.key[i] = ~0ull; return; }
+    if (e != E_NONE) { report(err, gidx ? gidx[i] : i, e); o.key[i] = ~0ull; return; }
     o.key[i] = c.key; o.reflen[i] = static_cast<uint16_t>(c.reflen); o.as0[i] = c.as0; o.asn[i] = c.asn; o.qlen[i] = c.qlen;
     o.xm3[i] = c.xm3; o.xmn[i] = c.xmn; o.bits[i] = c.bits;
     if (o.qh) { o.qh[2 * i] = qh[0]; o.qh[2 * i + 1] = qh[1]; }
@@ -296,7 +379,7 @@ __global__ void __launch_bounds__(kT) iota_kernel(uint32_t* x, uint64_t n) {
 // ---- K3: score stream in sorted order ---------------------------------------------------------------------------------------
 struct GatherArgs {
     const uint64_t* key_sorted; const uint32_t* order;   // order == nullptr: identity
-    ParseOut in; const uint64_t* roff;
+    ParseOut in; const uint64_t* roff; const uint32_t* gidx;   // gidx: file index of record i (shards); nullptr = i
     uint32_t* tid; int16_t* as0; uint8_t* xm3; uint16_t* qlen; uint32_t* orig_idx; uint64_t* qhash;
     int32_t* s_pos; uint16_t* s_reflen; uint8_t* s_bits; int16_t* s_asn; uint8_t* s_xmn; uint64_t* s_roff;
     uint32_t* run_flag; uint32_t* n_unmapped;
@@ -310,7 +393,7 @@ __global__ void __launch_bounds__(kT) gather_kernel(const GatherArgs a) {
     const uint64_t key = a.key_sorted[k];
     const uint32_t tid = static_cast<uint32_t>(key >> 33);
     a.tid[k] = tid; a.as0[k] = a.in.as0[i]; a.xm3[k] = a.in.xm3[i]; a.qlen[k] = a.in.qlen[i];
-    if (a.orig_idx) a.orig_idx[k] = static_cast<uint32_t>(i);
+    if (a.orig_idx) a.orig_idx[k] = a.gidx ? a.gidx[i] : static_cast<uint32_t>(i);
     if (a.qhash) { a.qhash[2 * k] = a.in.qh[2 * i]; a.qhash[2 * k + 1] = a.in.qh[2 * i + 1]; }
     a.s_pos[k] = static_cast<int32_t>(((key >> 1) & 0xffffffffull) - 1ull);
     a.s_reflen[k] = a.in.reflen[i]; a.s_bits[k] = a.in.bits[i]; a.s_asn[k] = a.in.asn[i]; a.s_xmn[k] = a.in.xmn[i]; a.s_roff[k] = a.roff[i];
@@ -527,7 +610,7 @@ struct mmlst_dev_bam {
     std::string names_blob, header_text;
     uint64_t n_rec = 0, n_prec = 0, n_plane_words = 0, n_dropped = 0, n_unmapped = 0, n_blocks = 0, comp_bytes = 0, infl_bytes = 0;
     uint32_t n_runs = 0, max_row_words = 0, n_ref = 0, max_depth = 0, repairs = 0;
-    int presorted = 0, minqual = 20, qc = 0;
+    int presorted = 0, minqual = 20, qc = 0, explicit_idx = 0;   // explicit_idx: a shard's streams carry orig_idx even in file order
     double seconds[8] = {0, 0, 0, 0, 0, 0, 0, 0};
 };
 
@@ -557,7 +640,7 @@ extern "C" int mmlst_dev_bam_info(const mmlst_dev_bam* b, mmlst_dev_bam_info_t* 
     if (!b || !o) { mmlst_set_error("mmlst_dev_bam_info: null argument"); return MMLST_E_ARG; }
     memset(o, 0, sizeof(*o));
     o->tid = b->tid.as<uint32_t>(); o->as0 = b->as0.as<int16_t>(); o->xm3 = b->xm3.as<uint8_t>(); o->qlen = b->qlen.as<uint16_t>();
-    o->orig_idx = b->presorted ? nullptr : b->orig_idx.as<uint32_t>();
+    o->orig_idx = (b->presorted && !b->explicit_idx) ? nullptr : b->orig_idx.as<uint32_t>();
     o->qhash = b->qhash.as<uint64_t>();
     o->run_tid = b->run_tid.as<uint32_t>(); o->run_start = b->run_start.as<uint32_t>(); o->chunk_run = b->chunk_run.as<uint32_t>();
     o->chunk_qlen = b->qc ? b->chunk_qlen.as<uint16_t>() : nullptr;
@@ -586,23 +669,14 @@ static int fetch_error(unsigned long long* d_err, cudaStream_t st, const char* w
     return err_class(code);
 }
 
-extern "C" int mmlst_bam_ingest(int device, const uint8_t* bam, size_t n_bytes, const mmlst_unpack_opts* opts_in, void* stream_in, mmlst_dev_bam** out) {
-    if (!bam || !out) { mmlst_set_error("mmlst_bam_ingest: null argument"); return MMLST_E_ARG; }
-    mmlst_unpack_opts o;
-    o.minqual = 20; o.max_depth = 8000; o.sentinel_nodes = 1; o.n_threads = 0; o.pinned = 1; o.assume_sorted = 0; o.want_qhash = 1; o.check_crc = 0; o.lenient_tags = 0;
-    if (opts_in) o = *opts_in;
-    if (o.lenient_tags) { mmlst_set_error("mmlst_bam_ingest: lenient_tags is an option of the host unpacker (mmlst_bam_unpack)"); return MMLST_E_ARG; }
-    CUDA_TRY(cudaSetDevice(device));
-    cudaStream_t st = static_cast<cudaStream_t>(stream_in);
-    g_cur_stream = st;
-    {
-        const int rc = mmlst_de_available(device);
-        if (rc != MMLST_OK) { mmlst_set_error("mmlst_bam_ingest: %s; use mmlst_bam_unpack", mmlst_last_error()); return rc; }
-    }
-    // ---- host: BGZF block table
-    struct Blk { uint64_t coff; uint32_t clen, isize, crc; uint64_t uoff; };
-    std::vector<Blk> blocks;
-    uint64_t usize = 0;
+
+namespace {
+
+struct Blk { uint64_t coff; uint32_t clen, isize, crc; uint64_t uoff; };
+
+// BGZF block table of bam[0, n_bytes): payload offset / size, CRC, ISIZE and inflated offset of every non-empty block
+int scan_blocks(const uint8_t* bam, size_t n_bytes, std::vector<Blk>& blocks, uint64_t& usize) {
+    usize = 0;
     for (size_t p = 0; p < n_bytes;) {
         if (n_bytes - p < 18 || bam[p] != 0x1f || bam[p + 1] != 0x8b || bam[p + 2] != 8 || !(bam[p + 3] & 4)) {
             mmlst_set_error("mmlst_bam_ingest: not a BGZF block at byte %zu (plain gzip / truncated file?)", p);
@@ -630,6 +704,311 @@ extern "C" int mmlst_bam_ingest(int device, const uint8_t* bam, size_t n_bytes, 
         if (b.isize) blocks.push_back(b);
         p += total;
     }
+    return MMLST_OK;
+}
+
+// Device buffers of the inflated stream and its block table
+struct Inflated {
+    DBuf d_comp, d_u, d_act, d_isize, d_uoff, d_crc;
+};
+
+// H2D + hardware inflate of every block, ISIZE check of every block, CRC-32 of the first n_crc blocks (opts.check_crc); failures go to
+// err as (block << 8 | code).  mark() is called after the block table is uploaded (the H2D / inflate split of the phase timer).
+template <class Mark>
+int inflate_blocks(int device, cudaStream_t st, const uint8_t* bam, size_t n_bytes, const std::vector<Blk>& blocks, uint64_t usize, bool check_crc,
+                   uint32_t n_crc, Inflated& I, unsigned long long* err, Mark&& mark) {
+    const uint32_t nb = static_cast<uint32_t>(blocks.size());
+    ING_TRY(I.d_comp.alloc(n_bytes + 64));
+    ING_TRY(I.d_u.alloc(usize + 64));
+    ING_TRY(I.d_act.alloc(static_cast<size_t>(nb) * 4));
+    ING_TRY(I.d_isize.alloc(static_cast<size_t>(nb) * 4));
+    ING_TRY(I.d_uoff.alloc((static_cast<size_t>(nb) + 1) * 8));
+    if (check_crc) ING_TRY(I.d_crc.alloc(static_cast<size_t>(nb) * 4));
+    std::vector<uint32_t> h_isize(nb);
+    std::vector<uint64_t> h_uoff(nb + 1);
+    for (uint32_t b = 0; b < nb; ++b) { h_isize[b] = blocks[b].isize; h_uoff[b] = blocks[b].uoff; }
+    h_uoff[nb] = usize;
+    CUDA_TRY(cudaMemcpyAsync(I.d_isize.p, h_isize.data(), static_cast<size_t>(nb) * 4, cudaMemcpyHostToDevice, st));
+    CUDA_TRY(cudaMemcpyAsync(I.d_uoff.p, h_uoff.data(), (static_cast<size_t>(nb) + 1) * 8, cudaMemcpyHostToDevice, st));
+    std::vector<uint32_t> h_want;
+    if (check_crc) {   // the raw CRC each block must have: trailer ^ crc32(0^isize)
+        static const std::vector<uint32_t> zeros = [] { std::vector<uint32_t> z(65537); bgzf_crc::make_zeros(z.data(), 65536); return z; }();
+        h_want.resize(nb);
+        for (uint32_t b = 0; b < nb; ++b) h_want[b] = blocks[b].crc ^ zeros[blocks[b].isize];
+        CUDA_TRY(cudaMemcpyAsync(I.d_crc.p, h_want.data(), static_cast<size_t>(nb) * 4, cudaMemcpyHostToDevice, st));
+    }
+    mark();
+    if (nb == 0) return MMLST_OK;
+    std::vector<CUmemDecompressParams> prm(nb);
+    memset(prm.data(), 0, sizeof(CUmemDecompressParams) * nb);
+    for (uint32_t b = 0; b < nb; ++b) {
+        prm[b].srcNumBytes = blocks[b].clen;
+        prm[b].dstNumBytes = blocks[b].isize;
+        prm[b].dstActBytes = I.d_act.as<cuuint32_t>() + b;
+        prm[b].src = I.d_comp.as<uint8_t>() + blocks[b].coff;
+        prm[b].dst = I.d_u.as<uint8_t>() + blocks[b].uoff;
+        prm[b].algo = CU_MEM_DECOMPRESS_ALGORITHM_DEFLATE;
+    }
+    // the file goes over in slices on a copy stream while the decompression engine works on the slices that have landed: the copy
+    // engine and the decompression engine are different units, so PCIe time hides behind the inflate (or the other way round)
+    {
+        std::vector<uint64_t> src_off(nb);
+        for (uint32_t b = 0; b < nb; ++b) src_off[b] = blocks[b].coff;
+        ING_TRY(mmlst_h2d_inflate(device, st, I.d_comp.as<uint8_t>(), bam, n_bytes, prm, src_off));
+    }
+    check_isize_kernel<<<(nb + kT - 1) / kT, kT, 0, st>>>(I.d_act.as<uint32_t>(), I.d_isize.as<uint32_t>(), nb, err);
+    CUDA_TRY(cudaGetLastError());
+    if (check_crc && n_crc) {
+        static const CrcArgs proto = [] { CrcArgs c{}; bgzf_crc::make_ops(c.ops); return c; }();
+        CrcArgs ca = proto;
+        ca.u = I.d_u.as<uint8_t>(); ca.uoff = I.d_uoff.as<uint64_t>(); ca.isize = I.d_isize.as<uint32_t>(); ca.want = I.d_crc.as<uint32_t>(); ca.n_blocks = n_crc;
+        int sms = 0, per_sm = 0;
+        CUDA_TRY(cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, device));
+        CUDA_TRY(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, crc_kernel, bgzf_crc::kCrcThreads, 0));
+        const uint32_t grid = std::min<uint32_t>(n_crc, static_cast<uint32_t>(std::max(sms, 1) * std::max(per_sm, 1)));
+        crc_kernel<<<grid, bgzf_crc::kCrcThreads, 0, st>>>(ca, err);
+        CUDA_TRY(cudaGetLastError());
+    }
+    return MMLST_OK;
+}
+
+// K1: guess every block's first record boundary, then verify / repair until nothing changes
+int run_chain(const ChainArgs& ca, uint32_t* d_changed, cudaStream_t st, uint32_t* repairs) {
+    const uint32_t nb = ca.n_blocks;
+    chain_guess_kernel<<<(nb + kT - 1) / kT, kT, 0, st>>>(ca);
+    CUDA_TRY(cudaGetLastError());
+    for (uint32_t sweep = 0;; ++sweep) {
+        CUDA_TRY(cudaMemsetAsync(d_changed, 0, 4, st));
+        chain_repair_kernel<<<(nb + kT - 1) / kT, kT, 0, st>>>(ca, d_changed);
+        CUDA_TRY(cudaGetLastError());
+        uint32_t changed = 0;
+        CUDA_TRY(cudaMemcpyAsync(&changed, d_changed, 4, cudaMemcpyDeviceToHost, st));
+        CUDA_TRY(cudaStreamSynchronize(st));
+        if (!changed) break;
+        *repairs += changed;
+        if (sweep > nb) { mmlst_set_error("mmlst_bam_ingest: record chain did not converge"); return MMLST_E_BAM; }
+    }
+    return MMLST_OK;
+}
+
+// Where the back half stopped: 1 = a record refusal (K2), 2 = --presorted on records out of coordinate order, 3 = plane array too
+// large, 4 = a refusal of a record entering the pileup (K5).  A shard's ranks agree on the least (phase, error word) before raising.
+enum BackPhase { kPhaseRecord = 1, kPhaseUnsorted = 2, kPhasePlanes = 3, kPhasePileup = 4 };
+
+struct BackIn {
+    const uint8_t* u; const uint64_t* roff; const uint32_t* gidx; uint64_t n;   // gidx: file index of record i (shards); nullptr = i
+    int32_t n_ref; const uint32_t* d_reflen;
+    unsigned long long* err; uint32_t* d_flags;
+    int unsorted;   // -1: decide from these records (the whole file); 0 / 1: decided across the shards of the file
+};
+
+const char* kUnsortedText = "mmlst_bam_ingest: --presorted given but records are not coordinate-sorted (htslib: 'The input is not sorted')";
+
+// The records known, everything after: K2 parse -> sort (stable by key, then file index) -> K3 score stream -> K4 depth cap -> K5 plane
+// rows.  The one back half of the whole-file ingest and of a shard's owner.  mark() after K2, the sort, K3, K4 and K5.
+template <class Mark>
+int back_half(const BackIn& in, const mmlst_unpack_opts& o, cudaStream_t st, mmlst_dev_bam* B, Mark&& mark, int* phase, unsigned long long* err_word) {
+    const uint64_t n = in.n;
+    const int32_t n_ref = in.n_ref;
+    unsigned long long* err = in.err;
+    uint32_t* d_flags = in.d_flags;
+    B->explicit_idx = in.gidx ? 1 : 0;
+    // ---- K2: per record
+    DBuf k_key, k_reflen, k_as0, k_asn, k_qlen, k_xm3, k_xmn, k_bits, k_qh;
+    ING_TRY(k_key.alloc(n * 8)); ING_TRY(k_reflen.alloc(n * 2)); ING_TRY(k_as0.alloc(n * 2)); ING_TRY(k_asn.alloc(n * 2)); ING_TRY(k_qlen.alloc(n * 2));
+    ING_TRY(k_xm3.alloc(n)); ING_TRY(k_xmn.alloc(n)); ING_TRY(k_bits.alloc(n));
+    if (o.want_qhash) ING_TRY(k_qh.alloc(n * 16));
+    const ParseOut po{k_key.as<uint64_t>(), k_reflen.as<uint16_t>(), k_as0.as<int16_t>(), k_asn.as<int16_t>(), k_qlen.as<uint16_t>(), k_xm3.as<uint8_t>(),
+                      k_xmn.as<uint8_t>(), k_bits.as<uint8_t>(), o.want_qhash ? k_qh.as<uint64_t>() : nullptr};
+    const unsigned gn = static_cast<unsigned>((n + kT - 1) / kT);
+    if (n) {
+        parse_kernel<<<gn, kT, 0, st>>>(in.u, in.roff, in.gidx, n, n_ref, po, err);
+        CUDA_TRY(cudaGetLastError());
+        check_sorted_kernel<<<gn, kT, 0, st>>>(k_key.as<uint64_t>(), n, d_flags);
+        CUDA_TRY(cudaGetLastError());
+    }
+    uint32_t sflags = 0;
+    CUDA_TRY(cudaMemcpyAsync(&sflags, d_flags, 4, cudaMemcpyDeviceToHost, st));
+    {
+        const int rc = fetch_error(err, st, "mmlst_bam_ingest", err_word);
+        if (rc != MMLST_OK) { *phase = kPhaseRecord; return rc; }
+    }
+    mark();  // 4
+    bool sorted = !(sflags & 1u);
+    if (o.assume_sorted) {
+        if (in.unsorted < 0 ? (sflags & 2u) != 0 : in.unsorted != 0) { mmlst_set_error("%s", kUnsortedText); *phase = kPhaseUnsorted; *err_word = 0; return MMLST_E_UNSORTED; }
+        sorted = true;
+    }
+    B->presorted = sorted ? 1 : 0;
+    const bool keep_idx = !sorted || in.gidx;
+
+    // ---- sort
+    DBuf d_key2, d_ord, d_ord2;
+    const uint64_t* key_sorted = k_key.as<uint64_t>();
+    const uint32_t* order = nullptr;
+    if (!sorted && n) {
+        ING_TRY(d_key2.alloc(n * 8)); ING_TRY(d_ord.alloc(n * 4)); ING_TRY(d_ord2.alloc(n * 4));
+        iota_kernel<<<gn, kT, 0, st>>>(d_ord.as<uint32_t>(), n);
+        CUDA_TRY(cudaGetLastError());
+        int end_bit = 34;
+        while (end_bit < 64 && (static_cast<uint64_t>(n_ref) >> (end_bit - 33)) != 0) ++end_bit;
+        size_t sb = 0;
+        CUDA_TRY(cub::DeviceRadixSort::SortPairs(nullptr, sb, k_key.as<uint64_t>(), d_key2.as<uint64_t>(), d_ord.as<uint32_t>(), d_ord2.as<uint32_t>(),
+                                                 static_cast<int>(n), 0, end_bit, st));
+        DBuf d_sorttmp;
+        ING_TRY(d_sorttmp.alloc(sb));
+        CUDA_TRY(cub::DeviceRadixSort::SortPairs(d_sorttmp.p, sb, k_key.as<uint64_t>(), d_key2.as<uint64_t>(), d_ord.as<uint32_t>(), d_ord2.as<uint32_t>(),
+                                                 static_cast<int>(n), 0, end_bit, st));
+        CUDA_TRY(cudaStreamSynchronize(st));
+        key_sorted = d_key2.as<uint64_t>();
+        order = d_ord2.as<uint32_t>();
+    }
+    mark();  // 5
+
+    // ---- K3: score stream
+    B->n_rec = n;
+    ING_TRY(B->tid.alloc(n * 4)); ING_TRY(B->as0.alloc(n * 2)); ING_TRY(B->xm3.alloc(n)); ING_TRY(B->qlen.alloc(n * 2));
+    if (keep_idx) ING_TRY(B->orig_idx.alloc(n * 4));
+    if (o.want_qhash) ING_TRY(B->qhash.alloc(n * 16));
+    DBuf s_pos, s_reflen, s_bits, s_asn, s_xmn, s_roff, d_runflag, d_runincl;
+    ING_TRY(s_pos.alloc(n * 4)); ING_TRY(s_reflen.alloc(n * 2)); ING_TRY(s_bits.alloc(n)); ING_TRY(s_asn.alloc(n * 2)); ING_TRY(s_xmn.alloc(n)); ING_TRY(s_roff.alloc(n * 8));
+    ING_TRY(d_runflag.alloc(n * 4 + 4)); ING_TRY(d_runincl.alloc(n * 4 + 4));
+    uint32_t n_runs = 0;
+    const uint64_t n_chunks = (n + 255) / 256;
+    ING_TRY(B->chunk_run.alloc(n_chunks * 4)); ING_TRY(B->chunk_qlen.alloc(n_chunks * 2));
+    if (n) {
+        const GatherArgs ga{key_sorted, order, po, in.roff, in.gidx, B->tid.as<uint32_t>(), B->as0.as<int16_t>(), B->xm3.as<uint8_t>(), B->qlen.as<uint16_t>(),
+                            keep_idx ? B->orig_idx.as<uint32_t>() : nullptr, o.want_qhash ? B->qhash.as<uint64_t>() : nullptr,
+                            s_pos.as<int32_t>(), s_reflen.as<uint16_t>(), s_bits.as<uint8_t>(), s_asn.as<int16_t>(), s_xmn.as<uint8_t>(), s_roff.as<uint64_t>(),
+                            d_runflag.as<uint32_t>(), d_flags + 4, n};
+        gather_kernel<<<gn, kT, 0, st>>>(ga);
+        CUDA_TRY(cudaGetLastError());
+        size_t sb = 0;
+        CUDA_TRY(cub::DeviceScan::InclusiveSum(nullptr, sb, d_runflag.as<uint32_t>(), d_runincl.as<uint32_t>(), static_cast<int>(n), st));
+        DBuf d_scantmp;
+        ING_TRY(d_scantmp.alloc(sb));
+        CUDA_TRY(cub::DeviceScan::InclusiveSum(d_scantmp.p, sb, d_runflag.as<uint32_t>(), d_runincl.as<uint32_t>(), static_cast<int>(n), st));
+        CUDA_TRY(cudaMemcpyAsync(&n_runs, d_runincl.as<uint32_t>() + (n - 1), 4, cudaMemcpyDeviceToHost, st));
+        CUDA_TRY(cudaStreamSynchronize(st));
+        ING_TRY(B->run_tid.alloc(static_cast<size_t>(n_runs) * 4)); ING_TRY(B->run_start.alloc((static_cast<size_t>(n_runs) + 1) * 4));
+        runs_kernel<<<gn, kT, 0, st>>>(d_runflag.as<uint32_t>(), d_runincl.as<uint32_t>(), B->tid.as<uint32_t>(), n, B->run_tid.as<uint32_t>(),
+                                       B->run_start.as<uint32_t>(), B->chunk_run.as<uint32_t>());
+        CUDA_TRY(cudaGetLastError());
+        const uint32_t one = 1;
+        CUDA_TRY(cudaMemcpyAsync(d_flags + 2, &one, 4, cudaMemcpyHostToDevice, st));
+        chunk_qlen_kernel<<<static_cast<unsigned>((n_chunks * 32 + kT - 1) / kT), kT, 0, st>>>(B->qlen.as<uint16_t>(), n, B->chunk_qlen.as<uint16_t>(), d_flags + 2);
+        CUDA_TRY(cudaGetLastError());
+    }
+    B->n_runs = n_runs;
+    mark();  // 6
+
+    // ---- K4: depth cap
+    DBuf d_adm, d_admx, d_hsz, d_hoff, d_hist, d_list, d_rw, d_rowoff, d_cs;
+    ING_TRY(d_adm.alloc(n * 4 + 4)); ING_TRY(d_admx.alloc(n * 4 + 4));
+    ING_TRY(d_cs.alloc((static_cast<size_t>(n_ref) + 1) * 8));
+    uint64_t P = 0, total_words = 0;
+    uint32_t fl[8] = {0, 0, 0, 0, 0, 0, 0, 0};
+    B->contig_start.assign(static_cast<size_t>(n_ref) + 1, 0);
+    if (n) {
+        CUDA_TRY(cudaMemsetAsync(d_adm.p, 0, n * 4 + 4, st));
+        ING_TRY(d_hsz.alloc((static_cast<size_t>(n_runs) + 1) * 8)); ING_TRY(d_hoff.alloc((static_cast<size_t>(n_runs) + 1) * 8));
+        CapArgs cap{B->run_tid.as<uint32_t>(), B->run_start.as<uint32_t>(), n_runs, s_pos.as<int32_t>(), s_reflen.as<uint16_t>(), s_bits.as<uint8_t>(),
+                    in.d_reflen, o.max_depth, o.sentinel_nodes, nullptr, nullptr, d_adm.as<uint32_t>()};
+        CUDA_TRY(cudaMemsetAsync(d_hsz.p, 0, (static_cast<size_t>(n_runs) + 1) * 8, st));
+        cap_sizes_kernel<<<(n_runs + kT - 1) / kT, kT, 0, st>>>(cap, d_hsz.as<uint64_t>());
+        CUDA_TRY(cudaGetLastError());
+        size_t sb = 0;
+        CUDA_TRY(cub::DeviceScan::ExclusiveSum(nullptr, sb, d_hsz.as<uint64_t>(), d_hoff.as<uint64_t>(), static_cast<int>(n_runs + 1), st));
+        DBuf t1;
+        ING_TRY(t1.alloc(sb));
+        CUDA_TRY(cub::DeviceScan::ExclusiveSum(t1.p, sb, d_hsz.as<uint64_t>(), d_hoff.as<uint64_t>(), static_cast<int>(n_runs + 1), st));
+        uint64_t hist_words = 0;
+        CUDA_TRY(cudaMemcpyAsync(&hist_words, d_hoff.as<uint64_t>() + n_runs, 8, cudaMemcpyDeviceToHost, st));
+        CUDA_TRY(cudaStreamSynchronize(st));
+        ING_TRY(d_hist.alloc(hist_words * 4 + 16));
+        CUDA_TRY(cudaMemsetAsync(d_hist.p, 0, hist_words * 4 + 16, st));
+        cap.hist_off = d_hoff.as<uint64_t>(); cap.hist = d_hist.as<uint32_t>();
+        cap_kernel<<<static_cast<unsigned>((static_cast<uint64_t>(n_runs) * 32 + kT - 1) / kT), kT, 0, st>>>(cap);
+        CUDA_TRY(cudaGetLastError());
+        // ---- K5: compaction
+        CUDA_TRY(cub::DeviceScan::ExclusiveSum(nullptr, sb, d_adm.as<uint32_t>(), d_admx.as<uint32_t>(), static_cast<int>(n + 1), st));
+        DBuf t2;
+        ING_TRY(t2.alloc(sb));
+        CUDA_TRY(cub::DeviceScan::ExclusiveSum(t2.p, sb, d_adm.as<uint32_t>(), d_admx.as<uint32_t>(), static_cast<int>(n + 1), st));
+        uint32_t P32 = 0;
+        CUDA_TRY(cudaMemcpyAsync(&P32, d_admx.as<uint32_t>() + n, 4, cudaMemcpyDeviceToHost, st));
+        CUDA_TRY(cudaStreamSynchronize(st));
+        P = P32;
+        ING_TRY(d_list.alloc(P * 4)); ING_TRY(d_rw.alloc((P + 1) * 8)); ING_TRY(d_rowoff.alloc((P + 1) * 8));
+        scatter_adm_kernel<<<gn, kT, 0, st>>>(d_adm.as<uint32_t>(), d_admx.as<uint32_t>(), n, d_list.as<uint32_t>());
+        CUDA_TRY(cudaGetLastError());
+        CUDA_TRY(cudaMemsetAsync(d_rw.p, 0, (P + 1) * 8, st));
+        if (P) {
+            row_sizes_kernel<<<static_cast<unsigned>((P + kT - 1) / kT), kT, 0, st>>>(d_list.as<uint32_t>(), P, s_pos.as<int32_t>(), s_reflen.as<uint16_t>(),
+                                                                                     d_rw.as<uint64_t>(), d_flags + 3);
+            CUDA_TRY(cudaGetLastError());
+        }
+        CUDA_TRY(cub::DeviceScan::ExclusiveSum(nullptr, sb, d_rw.as<uint64_t>(), d_rowoff.as<uint64_t>(), static_cast<int>(P + 1), st));
+        DBuf t3;
+        ING_TRY(t3.alloc(sb));
+        CUDA_TRY(cub::DeviceScan::ExclusiveSum(t3.p, sb, d_rw.as<uint64_t>(), d_rowoff.as<uint64_t>(), static_cast<int>(P + 1), st));
+        contig_start_kernel<<<(static_cast<unsigned>(n_ref) + 1 + kT - 1) / kT, kT, 0, st>>>(B->run_tid.as<uint32_t>(), B->run_start.as<uint32_t>(), n_runs,
+                                                                                             d_admx.as<uint32_t>(), P, static_cast<uint32_t>(n_ref), d_cs.as<uint64_t>());
+        CUDA_TRY(cudaGetLastError());
+        CUDA_TRY(cudaMemcpyAsync(&total_words, d_rowoff.as<uint64_t>() + P, 8, cudaMemcpyDeviceToHost, st));
+        CUDA_TRY(cudaMemcpyAsync(fl, d_flags, 32, cudaMemcpyDeviceToHost, st));
+        CUDA_TRY(cudaMemcpyAsync(B->contig_start.data(), d_cs.p, (static_cast<size_t>(n_ref) + 1) * 8, cudaMemcpyDeviceToHost, st));
+        CUDA_TRY(cudaStreamSynchronize(st));
+    }
+    mark();  // 7
+    const uint64_t kSlack = 8;
+    if (total_words + kSlack >= (1ull << 32)) { mmlst_set_error("mmlst_bam_ingest: plane array exceeds 2^32 words"); *phase = kPhasePlanes; *err_word = 0; return MMLST_E_RANGE; }
+    B->n_prec = P; B->n_plane_words = total_words + kSlack; B->max_row_words = fl[3]; B->qc = (n && fl[2]) ? 1 : 0;
+    ING_TRY(B->p_recs.alloc(P * sizeof(mmlst_prec))); ING_TRY(B->planes.alloc((total_words + kSlack) * 4));
+    CUDA_TRY(cudaMemsetAsync(B->planes.as<uint32_t>() + total_words, 0, kSlack * 4, st));
+    if (P) {
+        const PackArgs pa{in.u, d_list.as<uint32_t>(), P, d_rowoff.as<uint64_t>(), s_pos.as<int32_t>(), s_reflen.as<uint16_t>(), s_bits.as<uint8_t>(),
+                          s_asn.as<int16_t>(), s_xmn.as<uint8_t>(), s_roff.as<uint64_t>(), keep_idx ? B->orig_idx.as<uint32_t>() : nullptr, o.minqual,
+                          B->p_recs.as<mmlst_prec>(), B->planes.as<uint32_t>()};
+        pack_kernel<<<static_cast<unsigned>((P * 32 + kT - 1) / kT), kT, 0, st>>>(pa, err);
+        CUDA_TRY(cudaGetLastError());
+    }
+    mark();  // 8
+    {
+        const int rc = fetch_error(err, st, "mmlst_bam_ingest (pileup stream)", err_word);
+        if (rc != MMLST_OK) { *phase = kPhasePileup; return rc; }
+    }
+    B->n_unmapped = fl[4];
+    B->n_dropped = n - fl[4] - P;
+    B->minqual = o.minqual; B->max_depth = o.max_depth;
+    CUDA_TRY(cudaStreamSynchronize(st));
+    return MMLST_OK;
+}
+
+mmlst_unpack_opts ingest_opts(const mmlst_unpack_opts* opts_in) {
+    mmlst_unpack_opts o;
+    o.minqual = 20; o.max_depth = 8000; o.sentinel_nodes = 1; o.n_threads = 0; o.pinned = 1; o.assume_sorted = 0; o.want_qhash = 1; o.check_crc = 0; o.lenient_tags = 0;
+    if (opts_in) o = *opts_in;
+    return o;
+}
+
+}  // namespace
+
+extern "C" int mmlst_bam_ingest(int device, const uint8_t* bam, size_t n_bytes, const mmlst_unpack_opts* opts_in, void* stream_in, mmlst_dev_bam** out) {
+    if (!bam || !out) { mmlst_set_error("mmlst_bam_ingest: null argument"); return MMLST_E_ARG; }
+    const mmlst_unpack_opts o = ingest_opts(opts_in);
+    if (o.lenient_tags) { mmlst_set_error("mmlst_bam_ingest: lenient_tags is an option of the host unpacker (mmlst_bam_unpack)"); return MMLST_E_ARG; }
+    CUDA_TRY(cudaSetDevice(device));
+    cudaStream_t st = static_cast<cudaStream_t>(stream_in);
+    g_cur_stream = st;
+    {
+        const int rc = mmlst_de_available(device);
+        if (rc != MMLST_OK) { mmlst_set_error("mmlst_bam_ingest: %s; use mmlst_bam_unpack", mmlst_last_error()); return rc; }
+    }
+    // ---- host: BGZF block table
+    std::vector<Blk> blocks;
+    uint64_t usize = 0;
+    ING_TRY(scan_blocks(bam, n_bytes, blocks, usize));
     const uint32_t nb = static_cast<uint32_t>(blocks.size());
     if (usize < 12 || nb == 0) { mmlst_set_error("mmlst_bam_ingest: not a BAM file (empty)"); return MMLST_E_BAM; }
 
@@ -640,63 +1019,15 @@ extern "C" int mmlst_bam_ingest(int device, const uint8_t* bam, size_t n_bytes, 
     auto mark = [&]() { cudaEventRecord(ev[evn++], st); };
 
     // ---- H2D + hardware inflate
-    DBuf d_comp, d_u, d_act, d_isize, d_uoff, d_err, d_crc;
-    ING_TRY(d_comp.alloc(n_bytes + 64));
-    ING_TRY(d_u.alloc(usize + 64));
-    ING_TRY(d_act.alloc(static_cast<size_t>(nb) * 4));
-    ING_TRY(d_isize.alloc(static_cast<size_t>(nb) * 4));
-    ING_TRY(d_uoff.alloc((static_cast<size_t>(nb) + 1) * 8));
+    DBuf d_err;
     ING_TRY(d_err.alloc(8 + 32));
-    if (o.check_crc) ING_TRY(d_crc.alloc(static_cast<size_t>(nb) * 4));
     unsigned long long* err = d_err.as<unsigned long long>();
     uint32_t* d_flags = reinterpret_cast<uint32_t*>(err + 1);   // [0] sortedness, [1] repair counter, [2] uniform qlen, [3] max row words, [4] records with the unmapped flag
     CUDA_TRY(cudaMemsetAsync(err, 0xff, 8, st));
     CUDA_TRY(cudaMemsetAsync(d_flags, 0, 32, st));
     mark();  // 0
-    std::vector<uint32_t> h_isize(nb);
-    std::vector<uint64_t> h_uoff(nb + 1);
-    for (uint32_t b = 0; b < nb; ++b) { h_isize[b] = blocks[b].isize; h_uoff[b] = blocks[b].uoff; }
-    h_uoff[nb] = usize;
-    CUDA_TRY(cudaMemcpyAsync(d_isize.p, h_isize.data(), static_cast<size_t>(nb) * 4, cudaMemcpyHostToDevice, st));
-    CUDA_TRY(cudaMemcpyAsync(d_uoff.p, h_uoff.data(), (static_cast<size_t>(nb) + 1) * 8, cudaMemcpyHostToDevice, st));
-    std::vector<uint32_t> h_want;
-    if (o.check_crc) {   // the raw CRC each block must have: trailer ^ crc32(0^isize)
-        static const std::vector<uint32_t> zeros = [] { std::vector<uint32_t> z(65537); bgzf_crc::make_zeros(z.data(), 65536); return z; }();
-        h_want.resize(nb);
-        for (uint32_t b = 0; b < nb; ++b) h_want[b] = blocks[b].crc ^ zeros[blocks[b].isize];
-        CUDA_TRY(cudaMemcpyAsync(d_crc.p, h_want.data(), static_cast<size_t>(nb) * 4, cudaMemcpyHostToDevice, st));
-    }
-    mark();  // 1
-    std::vector<CUmemDecompressParams> prm(nb);
-    memset(prm.data(), 0, sizeof(CUmemDecompressParams) * nb);
-    for (uint32_t b = 0; b < nb; ++b) {
-        prm[b].srcNumBytes = blocks[b].clen;
-        prm[b].dstNumBytes = blocks[b].isize;
-        prm[b].dstActBytes = d_act.as<cuuint32_t>() + b;
-        prm[b].src = d_comp.as<uint8_t>() + blocks[b].coff;
-        prm[b].dst = d_u.as<uint8_t>() + blocks[b].uoff;
-        prm[b].algo = CU_MEM_DECOMPRESS_ALGORITHM_DEFLATE;
-    }
-    // the file goes over in slices on a copy stream while the decompression engine works on the slices that have landed: the copy
-    // engine and the decompression engine are different units, so PCIe time hides behind the inflate (or the other way round)
-    {
-        std::vector<uint64_t> src_off(nb);
-        for (uint32_t b = 0; b < nb; ++b) src_off[b] = blocks[b].coff;
-        ING_TRY(mmlst_h2d_inflate(device, st, d_comp.as<uint8_t>(), bam, n_bytes, prm, src_off));
-    }
-    check_isize_kernel<<<(nb + kT - 1) / kT, kT, 0, st>>>(d_act.as<uint32_t>(), d_isize.as<uint32_t>(), nb, err);
-    CUDA_TRY(cudaGetLastError());
-    if (o.check_crc) {
-        static const CrcArgs proto = [] { CrcArgs c{}; bgzf_crc::make_ops(c.ops); return c; }();
-        CrcArgs ca = proto;
-        ca.u = d_u.as<uint8_t>(); ca.uoff = d_uoff.as<uint64_t>(); ca.isize = d_isize.as<uint32_t>(); ca.want = d_crc.as<uint32_t>(); ca.n_blocks = nb;
-        int sms = 0, per_sm = 0;
-        CUDA_TRY(cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, device));
-        CUDA_TRY(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, crc_kernel, bgzf_crc::kCrcThreads, 0));
-        const uint32_t grid = std::min<uint32_t>(nb, static_cast<uint32_t>(std::max(sms, 1) * std::max(per_sm, 1)));
-        crc_kernel<<<grid, bgzf_crc::kCrcThreads, 0, st>>>(ca, err);
-        CUDA_TRY(cudaGetLastError());
-    }
+    Inflated I;
+    ING_TRY(inflate_blocks(device, st, bam, n_bytes, blocks, usize, o.check_crc != 0, nb, I, err, mark));   // mark 1 inside
     mark();  // 2
     // ---- header (first bytes of the inflated stream come back to the host)
     std::unique_ptr<mmlst_dev_bam> B(new mmlst_dev_bam());
@@ -711,7 +1042,7 @@ extern "C" int mmlst_bam_ingest(int device, const uint8_t* bam, size_t n_bytes, 
             uint8_t* hb = stage_guard.get(want);
             if (!hb) { mmlst_set_error("mmlst_bam_ingest: cudaHostAlloc(%zu) failed", want); return MMLST_E_NOMEM; }
             head = hb;
-            CUDA_TRY(cudaMemcpyAsync(hb, d_u.p, want, cudaMemcpyDeviceToHost, st));
+            CUDA_TRY(cudaMemcpyAsync(hb, I.d_u.p, want, cudaMemcpyDeviceToHost, st));
             {
                 unsigned long long e = kNoErr;
                 const int rc = fetch_error(err, st, "mmlst_bam_ingest (inflate)", &e);
@@ -765,21 +1096,9 @@ extern "C" int mmlst_bam_ingest(int device, const uint8_t* bam, size_t n_bytes, 
     DBuf d_start, d_exit, d_count, d_badw, d_base, d_tmp;
     ING_TRY(d_start.alloc(static_cast<size_t>(nb) * 8)); ING_TRY(d_exit.alloc(static_cast<size_t>(nb) * 8));
     ING_TRY(d_count.alloc(static_cast<size_t>(nb) * 4 + 4)); ING_TRY(d_badw.alloc(static_cast<size_t>(nb) * 4)); ING_TRY(d_base.alloc(static_cast<size_t>(nb) * 4 + 4));
-    const ChainArgs ca{d_u.as<uint8_t>(), usize, d_uoff.as<uint64_t>(), nb, first_record, n_ref, d_reflen.as<uint32_t>(),
-                       d_start.as<uint64_t>(), d_exit.as<uint64_t>(), d_count.as<uint32_t>(), d_badw.as<uint32_t>()};
-    chain_guess_kernel<<<(nb + kT - 1) / kT, kT, 0, st>>>(ca);
-    CUDA_TRY(cudaGetLastError());
-    for (uint32_t sweep = 0;; ++sweep) {
-        CUDA_TRY(cudaMemsetAsync(d_flags + 1, 0, 4, st));
-        chain_repair_kernel<<<(nb + kT - 1) / kT, kT, 0, st>>>(ca, d_flags + 1);
-        CUDA_TRY(cudaGetLastError());
-        uint32_t changed = 0;
-        CUDA_TRY(cudaMemcpyAsync(&changed, d_flags + 1, 4, cudaMemcpyDeviceToHost, st));
-        CUDA_TRY(cudaStreamSynchronize(st));
-        if (!changed) break;
-        B->repairs += changed;
-        if (sweep > nb) { mmlst_set_error("mmlst_bam_ingest: record chain did not converge"); return MMLST_E_BAM; }
-    }
+    const ChainArgs ca{I.d_u.as<uint8_t>(), usize, I.d_uoff.as<uint64_t>(), nb, first_record, n_ref, d_reflen.as<uint32_t>(),
+                       d_start.as<uint64_t>(), d_exit.as<uint64_t>(), d_count.as<uint32_t>(), d_badw.as<uint32_t>(), usize, nullptr};
+    ING_TRY(run_chain(ca, d_flags + 1, st, &B->repairs));
     size_t tmp_bytes = 0;
     CUDA_TRY(cub::DeviceScan::ExclusiveSum(nullptr, tmp_bytes, d_count.as<uint32_t>(), d_base.as<uint32_t>(), nb + 1, st));
     ING_TRY(d_tmp.alloc(tmp_bytes));
@@ -796,170 +1115,310 @@ extern "C" int mmlst_bam_ingest(int device, const uint8_t* bam, size_t n_bytes, 
     CUDA_TRY(cudaGetLastError());
     mark();  // 3
 
-    // ---- K2: per record
-    DBuf k_key, k_reflen, k_as0, k_asn, k_qlen, k_xm3, k_xmn, k_bits, k_qh;
-    ING_TRY(k_key.alloc(n * 8)); ING_TRY(k_reflen.alloc(n * 2)); ING_TRY(k_as0.alloc(n * 2)); ING_TRY(k_asn.alloc(n * 2)); ING_TRY(k_qlen.alloc(n * 2));
-    ING_TRY(k_xm3.alloc(n)); ING_TRY(k_xmn.alloc(n)); ING_TRY(k_bits.alloc(n));
-    if (o.want_qhash) ING_TRY(k_qh.alloc(n * 16));
-    const ParseOut po{k_key.as<uint64_t>(), k_reflen.as<uint16_t>(), k_as0.as<int16_t>(), k_asn.as<int16_t>(), k_qlen.as<uint16_t>(), k_xm3.as<uint8_t>(),
-                      k_xmn.as<uint8_t>(), k_bits.as<uint8_t>(), o.want_qhash ? k_qh.as<uint64_t>() : nullptr};
-    const unsigned gn = static_cast<unsigned>((n + kT - 1) / kT);
-    if (n) {
-        parse_kernel<<<gn, kT, 0, st>>>(d_u.as<uint8_t>(), d_roff.as<uint64_t>(), n, n_ref, po, err);
-        CUDA_TRY(cudaGetLastError());
-        check_sorted_kernel<<<gn, kT, 0, st>>>(k_key.as<uint64_t>(), n, d_flags);
-        CUDA_TRY(cudaGetLastError());
-    }
-    uint32_t sflags = 0;
-    CUDA_TRY(cudaMemcpyAsync(&sflags, d_flags, 4, cudaMemcpyDeviceToHost, st));
-    ING_TRY(fetch_error(err, st, "mmlst_bam_ingest"));
-    mark();  // 4
-    bool sorted = !(sflags & 1u);
-    if (o.assume_sorted) {
-        if (sflags & 2u) { mmlst_set_error("mmlst_bam_ingest: --presorted given but records are not coordinate-sorted (htslib: 'The input is not sorted')"); return MMLST_E_UNSORTED; }
-        sorted = true;
-    }
-    B->presorted = sorted ? 1 : 0;
-
-    // ---- sort
-    DBuf d_key2, d_ord, d_ord2;
-    const uint64_t* key_sorted = k_key.as<uint64_t>();
-    const uint32_t* order = nullptr;
-    if (!sorted && n) {
-        ING_TRY(d_key2.alloc(n * 8)); ING_TRY(d_ord.alloc(n * 4)); ING_TRY(d_ord2.alloc(n * 4));
-        iota_kernel<<<gn, kT, 0, st>>>(d_ord.as<uint32_t>(), n);
-        CUDA_TRY(cudaGetLastError());
-        int end_bit = 34;
-        while (end_bit < 64 && (static_cast<uint64_t>(n_ref) >> (end_bit - 33)) != 0) ++end_bit;
-        size_t sb = 0;
-        CUDA_TRY(cub::DeviceRadixSort::SortPairs(nullptr, sb, k_key.as<uint64_t>(), d_key2.as<uint64_t>(), d_ord.as<uint32_t>(), d_ord2.as<uint32_t>(),
-                                                 static_cast<int>(n), 0, end_bit, st));
-        DBuf d_sorttmp;
-        ING_TRY(d_sorttmp.alloc(sb));
-        CUDA_TRY(cub::DeviceRadixSort::SortPairs(d_sorttmp.p, sb, k_key.as<uint64_t>(), d_key2.as<uint64_t>(), d_ord.as<uint32_t>(), d_ord2.as<uint32_t>(),
-                                                 static_cast<int>(n), 0, end_bit, st));
-        CUDA_TRY(cudaStreamSynchronize(st));
-        key_sorted = d_key2.as<uint64_t>();
-        order = d_ord2.as<uint32_t>();
-    }
-    mark();  // 5
-
-    // ---- K3: score stream
-    B->n_rec = n;
-    ING_TRY(B->tid.alloc(n * 4)); ING_TRY(B->as0.alloc(n * 2)); ING_TRY(B->xm3.alloc(n)); ING_TRY(B->qlen.alloc(n * 2));
-    if (!sorted) ING_TRY(B->orig_idx.alloc(n * 4));
-    if (o.want_qhash) ING_TRY(B->qhash.alloc(n * 16));
-    DBuf s_pos, s_reflen, s_bits, s_asn, s_xmn, s_roff, d_runflag, d_runincl;
-    ING_TRY(s_pos.alloc(n * 4)); ING_TRY(s_reflen.alloc(n * 2)); ING_TRY(s_bits.alloc(n)); ING_TRY(s_asn.alloc(n * 2)); ING_TRY(s_xmn.alloc(n)); ING_TRY(s_roff.alloc(n * 8));
-    ING_TRY(d_runflag.alloc(n * 4 + 4)); ING_TRY(d_runincl.alloc(n * 4 + 4));
-    uint32_t n_runs = 0;
-    const uint64_t n_chunks = (n + 255) / 256;
-    ING_TRY(B->chunk_run.alloc(n_chunks * 4)); ING_TRY(B->chunk_qlen.alloc(n_chunks * 2));
-    if (n) {
-        const GatherArgs ga{key_sorted, order, po, d_roff.as<uint64_t>(), B->tid.as<uint32_t>(), B->as0.as<int16_t>(), B->xm3.as<uint8_t>(), B->qlen.as<uint16_t>(),
-                            sorted ? nullptr : B->orig_idx.as<uint32_t>(), o.want_qhash ? B->qhash.as<uint64_t>() : nullptr,
-                            s_pos.as<int32_t>(), s_reflen.as<uint16_t>(), s_bits.as<uint8_t>(), s_asn.as<int16_t>(), s_xmn.as<uint8_t>(), s_roff.as<uint64_t>(),
-                            d_runflag.as<uint32_t>(), d_flags + 4, n};
-        gather_kernel<<<gn, kT, 0, st>>>(ga);
-        CUDA_TRY(cudaGetLastError());
-        size_t sb = 0;
-        CUDA_TRY(cub::DeviceScan::InclusiveSum(nullptr, sb, d_runflag.as<uint32_t>(), d_runincl.as<uint32_t>(), static_cast<int>(n), st));
-        DBuf d_scantmp;
-        ING_TRY(d_scantmp.alloc(sb));
-        CUDA_TRY(cub::DeviceScan::InclusiveSum(d_scantmp.p, sb, d_runflag.as<uint32_t>(), d_runincl.as<uint32_t>(), static_cast<int>(n), st));
-        CUDA_TRY(cudaMemcpyAsync(&n_runs, d_runincl.as<uint32_t>() + (n - 1), 4, cudaMemcpyDeviceToHost, st));
-        CUDA_TRY(cudaStreamSynchronize(st));
-        ING_TRY(B->run_tid.alloc(static_cast<size_t>(n_runs) * 4)); ING_TRY(B->run_start.alloc((static_cast<size_t>(n_runs) + 1) * 4));
-        runs_kernel<<<gn, kT, 0, st>>>(d_runflag.as<uint32_t>(), d_runincl.as<uint32_t>(), B->tid.as<uint32_t>(), n, B->run_tid.as<uint32_t>(),
-                                       B->run_start.as<uint32_t>(), B->chunk_run.as<uint32_t>());
-        CUDA_TRY(cudaGetLastError());
-        const uint32_t one = 1;
-        CUDA_TRY(cudaMemcpyAsync(d_flags + 2, &one, 4, cudaMemcpyHostToDevice, st));
-        chunk_qlen_kernel<<<static_cast<unsigned>((n_chunks * 32 + kT - 1) / kT), kT, 0, st>>>(B->qlen.as<uint16_t>(), n, B->chunk_qlen.as<uint16_t>(), d_flags + 2);
-        CUDA_TRY(cudaGetLastError());
-    }
-    B->n_runs = n_runs;
-    mark();  // 6
-
-    // ---- K4: depth cap
-    DBuf d_adm, d_admx, d_hsz, d_hoff, d_hist, d_list, d_rw, d_rowoff, d_cs;
-    ING_TRY(d_adm.alloc(n * 4 + 4)); ING_TRY(d_admx.alloc(n * 4 + 4));
-    ING_TRY(d_cs.alloc((static_cast<size_t>(n_ref) + 1) * 8));
-    uint64_t P = 0, total_words = 0;
-    uint32_t fl[8] = {0, 0, 0, 0, 0, 0, 0, 0};
-    B->contig_start.assign(static_cast<size_t>(n_ref) + 1, 0);
-    if (n) {
-        CUDA_TRY(cudaMemsetAsync(d_adm.p, 0, n * 4 + 4, st));
-        ING_TRY(d_hsz.alloc((static_cast<size_t>(n_runs) + 1) * 8)); ING_TRY(d_hoff.alloc((static_cast<size_t>(n_runs) + 1) * 8));
-        CapArgs cap{B->run_tid.as<uint32_t>(), B->run_start.as<uint32_t>(), n_runs, s_pos.as<int32_t>(), s_reflen.as<uint16_t>(), s_bits.as<uint8_t>(),
-                    d_reflen.as<uint32_t>(), o.max_depth, o.sentinel_nodes, nullptr, nullptr, d_adm.as<uint32_t>()};
-        CUDA_TRY(cudaMemsetAsync(d_hsz.p, 0, (static_cast<size_t>(n_runs) + 1) * 8, st));
-        cap_sizes_kernel<<<(n_runs + kT - 1) / kT, kT, 0, st>>>(cap, d_hsz.as<uint64_t>());
-        CUDA_TRY(cudaGetLastError());
-        size_t sb = 0;
-        CUDA_TRY(cub::DeviceScan::ExclusiveSum(nullptr, sb, d_hsz.as<uint64_t>(), d_hoff.as<uint64_t>(), static_cast<int>(n_runs + 1), st));
-        DBuf t1;
-        ING_TRY(t1.alloc(sb));
-        CUDA_TRY(cub::DeviceScan::ExclusiveSum(t1.p, sb, d_hsz.as<uint64_t>(), d_hoff.as<uint64_t>(), static_cast<int>(n_runs + 1), st));
-        uint64_t hist_words = 0;
-        CUDA_TRY(cudaMemcpyAsync(&hist_words, d_hoff.as<uint64_t>() + n_runs, 8, cudaMemcpyDeviceToHost, st));
-        CUDA_TRY(cudaStreamSynchronize(st));
-        ING_TRY(d_hist.alloc(hist_words * 4 + 16));
-        CUDA_TRY(cudaMemsetAsync(d_hist.p, 0, hist_words * 4 + 16, st));
-        cap.hist_off = d_hoff.as<uint64_t>(); cap.hist = d_hist.as<uint32_t>();
-        cap_kernel<<<static_cast<unsigned>((static_cast<uint64_t>(n_runs) * 32 + kT - 1) / kT), kT, 0, st>>>(cap);
-        CUDA_TRY(cudaGetLastError());
-        // ---- K5: compaction
-        CUDA_TRY(cub::DeviceScan::ExclusiveSum(nullptr, sb, d_adm.as<uint32_t>(), d_admx.as<uint32_t>(), static_cast<int>(n + 1), st));
-        DBuf t2;
-        ING_TRY(t2.alloc(sb));
-        CUDA_TRY(cub::DeviceScan::ExclusiveSum(t2.p, sb, d_adm.as<uint32_t>(), d_admx.as<uint32_t>(), static_cast<int>(n + 1), st));
-        uint32_t P32 = 0;
-        CUDA_TRY(cudaMemcpyAsync(&P32, d_admx.as<uint32_t>() + n, 4, cudaMemcpyDeviceToHost, st));
-        CUDA_TRY(cudaStreamSynchronize(st));
-        P = P32;
-        ING_TRY(d_list.alloc(P * 4)); ING_TRY(d_rw.alloc((P + 1) * 8)); ING_TRY(d_rowoff.alloc((P + 1) * 8));
-        scatter_adm_kernel<<<gn, kT, 0, st>>>(d_adm.as<uint32_t>(), d_admx.as<uint32_t>(), n, d_list.as<uint32_t>());
-        CUDA_TRY(cudaGetLastError());
-        CUDA_TRY(cudaMemsetAsync(d_rw.p, 0, (P + 1) * 8, st));
-        if (P) {
-            row_sizes_kernel<<<static_cast<unsigned>((P + kT - 1) / kT), kT, 0, st>>>(d_list.as<uint32_t>(), P, s_pos.as<int32_t>(), s_reflen.as<uint16_t>(),
-                                                                                     d_rw.as<uint64_t>(), d_flags + 3);
-            CUDA_TRY(cudaGetLastError());
-        }
-        CUDA_TRY(cub::DeviceScan::ExclusiveSum(nullptr, sb, d_rw.as<uint64_t>(), d_rowoff.as<uint64_t>(), static_cast<int>(P + 1), st));
-        DBuf t3;
-        ING_TRY(t3.alloc(sb));
-        CUDA_TRY(cub::DeviceScan::ExclusiveSum(t3.p, sb, d_rw.as<uint64_t>(), d_rowoff.as<uint64_t>(), static_cast<int>(P + 1), st));
-        contig_start_kernel<<<(static_cast<unsigned>(n_ref) + 1 + kT - 1) / kT, kT, 0, st>>>(B->run_tid.as<uint32_t>(), B->run_start.as<uint32_t>(), n_runs,
-                                                                                             d_admx.as<uint32_t>(), P, static_cast<uint32_t>(n_ref), d_cs.as<uint64_t>());
-        CUDA_TRY(cudaGetLastError());
-        CUDA_TRY(cudaMemcpyAsync(&total_words, d_rowoff.as<uint64_t>() + P, 8, cudaMemcpyDeviceToHost, st));
-        CUDA_TRY(cudaMemcpyAsync(fl, d_flags, 32, cudaMemcpyDeviceToHost, st));
-        CUDA_TRY(cudaMemcpyAsync(B->contig_start.data(), d_cs.p, (static_cast<size_t>(n_ref) + 1) * 8, cudaMemcpyDeviceToHost, st));
-        CUDA_TRY(cudaStreamSynchronize(st));
-    }
-    mark();  // 7
-    const uint64_t kSlack = 8;
-    if (total_words + kSlack >= (1ull << 32)) { mmlst_set_error("mmlst_bam_ingest: plane array exceeds 2^32 words"); return MMLST_E_RANGE; }
-    B->n_prec = P; B->n_plane_words = total_words + kSlack; B->max_row_words = fl[3]; B->qc = (n && fl[2]) ? 1 : 0;
-    ING_TRY(B->p_recs.alloc(P * sizeof(mmlst_prec))); ING_TRY(B->planes.alloc((total_words + kSlack) * 4));
-    CUDA_TRY(cudaMemsetAsync(B->planes.as<uint32_t>() + total_words, 0, kSlack * 4, st));
-    if (P) {
-        const PackArgs pa{d_u.as<uint8_t>(), d_list.as<uint32_t>(), P, d_rowoff.as<uint64_t>(), s_pos.as<int32_t>(), s_reflen.as<uint16_t>(), s_bits.as<uint8_t>(),
-                          s_asn.as<int16_t>(), s_xmn.as<uint8_t>(), s_roff.as<uint64_t>(), sorted ? nullptr : B->orig_idx.as<uint32_t>(), o.minqual,
-                          B->p_recs.as<mmlst_prec>(), B->planes.as<uint32_t>()};
-        pack_kernel<<<static_cast<unsigned>((P * 32 + kT - 1) / kT), kT, 0, st>>>(pa, err);
-        CUDA_TRY(cudaGetLastError());
-    }
-    mark();  // 8
-    ING_TRY(fetch_error(err, st, "mmlst_bam_ingest (pileup stream)"));
-    B->n_unmapped = fl[4];
-    B->n_dropped = n - fl[4] - P;
-    B->minqual = o.minqual; B->max_depth = o.max_depth; B->n_blocks = nb; B->comp_bytes = n_bytes; B->infl_bytes = usize;
-    CUDA_TRY(cudaStreamSynchronize(st));
+    const BackIn in{I.d_u.as<uint8_t>(), d_roff.as<uint64_t>(), nullptr, n, n_ref, d_reflen.as<uint32_t>(), err, d_flags, -1};
+    int phase = 0;
+    unsigned long long ew = kNoErr;
+    ING_TRY(back_half(in, o, st, B.get(), mark, &phase, &ew));
+    B->n_blocks = nb; B->comp_bytes = n_bytes; B->infl_bytes = usize;
     // phase seconds from the device events: h2d, inflate, chain, parse, sort, score stream, cap + compaction, pack
     for (int i = 0; i + 1 < evn && i < 8; ++i) { float ms = 0; cudaEventElapsedTime(&ms, ev[i], ev[i + 1]); B->seconds[i] = ms * 1e-3; }
     *out = B.release();
     return MMLST_OK;
+}
+
+// ================================================================================================================================
+// One BAM over several ranks.  Front half (per rank): the rank's own BGZF blocks (+ a halo of the next blocks, so that its last
+// record can end there) are inflated, the record chain is walked from an agreed entry, and the records that START in its own blocks
+// are partitioned by owner rank.  The ranks exchange the partitions; the back half (per owner) is back_half() above.
+// ================================================================================================================================
+struct mmlst_ingest_front {
+    int device = 0;
+    cudaStream_t st = nullptr;
+    std::vector<Blk> blocks;
+    uint32_t nb = 0, n_own = 0;
+    uint64_t usize = 0, uend = 0, n_comp = 0;
+    int32_t n_ref = 0;
+    Inflated I;
+    DBuf d_err, d_reflen, d_start, d_exit, d_count, d_badw, d_need, d_base, d_owner, d_roff, d_dest, d_rlen, d_order, d_boff, d_dcount, d_keys;
+    DBuf send, send_len, send_idx;
+    unsigned long long block_err = kNoErr, chain_err = kNoErr;
+    uint64_t entry = kNoEntry, exit = kNoEntry, need = 0, n_rec = 0;
+    uint32_t repairs = 0;
+    int world = 0, unsorted = 0, walked = 0;
+    uint64_t keys[2] = {0, 0};
+    std::vector<uint64_t> dest_records, dest_bytes;
+    double seconds[4] = {0, 0, 0, 0};
+};
+
+namespace {
+double since(std::chrono::steady_clock::time_point t0) { return std::chrono::duration<double>(std::chrono::steady_clock::now() - t0).count(); }
+}
+
+extern "C" int mmlst_ingest_front_open(int device, const uint8_t* comp, size_t n_comp, size_t n_own_bytes, const uint32_t* ref_len, int32_t n_ref,
+                                       int check_crc, void* stream_in, mmlst_ingest_front** out) {
+    if ((!comp && n_comp) || !out || n_own_bytes > n_comp || n_ref < 0 || (n_ref && !ref_len)) { mmlst_set_error("mmlst_ingest_front_open: bad argument"); return MMLST_E_ARG; }
+    CUDA_TRY(cudaSetDevice(device));
+    cudaStream_t st = static_cast<cudaStream_t>(stream_in);
+    g_cur_stream = st;
+    {
+        const int rc = mmlst_de_available(device);
+        if (rc != MMLST_OK) { mmlst_set_error("mmlst_ingest_front_open: %s; use mmlst_bam_unpack", mmlst_last_error()); return rc; }
+    }
+    const auto t0 = std::chrono::steady_clock::now();
+    std::unique_ptr<mmlst_ingest_front> F(new mmlst_ingest_front());
+    F->device = device; F->st = st; F->n_ref = n_ref; F->n_comp = n_comp;
+    ING_TRY(scan_blocks(comp, n_comp, F->blocks, F->usize));
+    F->nb = static_cast<uint32_t>(F->blocks.size());
+    F->uend = F->usize;
+    for (uint32_t b = 0; b < F->nb; ++b) {
+        const uint64_t hdr = F->blocks[b].coff;   // payload offset; the block's header starts before it, inside the same range
+        if (hdr >= n_own_bytes) { F->uend = F->blocks[b].uoff; break; }
+        F->n_own = b + 1;
+    }
+    ING_TRY(F->d_err.alloc(16 + 32));
+    unsigned long long* err = F->d_err.as<unsigned long long>();
+    CUDA_TRY(cudaMemsetAsync(err, 0xff, 16, st));
+    CUDA_TRY(cudaMemsetAsync(err + 2, 0, 32, st));
+    ING_TRY(inflate_blocks(device, st, comp, n_comp, F->blocks, F->usize, check_crc != 0, F->n_own, F->I, err, [] {}));
+    ING_TRY(F->d_reflen.alloc(static_cast<size_t>(n_ref) * 4 + 16));
+    if (n_ref) CUDA_TRY(cudaMemcpyAsync(F->d_reflen.p, ref_len, static_cast<size_t>(n_ref) * 4, cudaMemcpyHostToDevice, st));
+    const size_t nb = F->nb;
+    ING_TRY(F->d_start.alloc(nb * 8)); ING_TRY(F->d_exit.alloc(nb * 8)); ING_TRY(F->d_count.alloc(nb * 4 + 4)); ING_TRY(F->d_badw.alloc(nb * 4));
+    ING_TRY(F->d_need.alloc(nb * 8)); ING_TRY(F->d_base.alloc(nb * 4 + 4));
+    CUDA_TRY(cudaMemcpyAsync(&F->block_err, err, 8, cudaMemcpyDeviceToHost, st));
+    CUDA_TRY(cudaStreamSynchronize(st));
+    F->seconds[0] = since(t0);
+    *out = F.release();
+    return MMLST_OK;
+}
+
+extern "C" int mmlst_ingest_front_walk(mmlst_ingest_front* F, uint64_t entry) {
+    if (!F) { mmlst_set_error("mmlst_ingest_front_walk: null argument"); return MMLST_E_ARG; }
+    CUDA_TRY(cudaSetDevice(F->device));
+    g_cur_stream = F->st;
+    cudaStream_t st = F->st;
+    const auto t0 = std::chrono::steady_clock::now();
+    F->walked = 1; F->need = 0; F->n_rec = 0; F->chain_err = kNoErr;
+    if (F->n_own == 0 || (entry != kNoEntry && entry >= F->uend)) {   // no record starts here: the chain passes through
+        F->entry = entry; F->exit = entry;
+        CUDA_TRY(cudaMemsetAsync(F->d_count.p, 0, 4, st));
+        return MMLST_OK;
+    }
+    const uint32_t n_own = F->n_own;
+    const ChainArgs ca{F->I.d_u.as<uint8_t>(), F->usize, F->I.d_uoff.as<uint64_t>(), n_own, entry, F->n_ref, F->d_reflen.as<uint32_t>(),
+                       F->d_start.as<uint64_t>(), F->d_exit.as<uint64_t>(), F->d_count.as<uint32_t>(), F->d_badw.as<uint32_t>(), F->uend,
+                       F->d_need.as<uint64_t>()};
+    uint32_t* d_changed = reinterpret_cast<uint32_t*>(F->d_err.as<unsigned long long>() + 2);
+    ING_TRY(run_chain(ca, d_changed, st, &F->repairs));
+    std::vector<uint32_t> badw(n_own);
+    std::vector<uint64_t> need(n_own);
+    uint64_t first_start = 0, last_exit = 0;
+    CUDA_TRY(cudaMemcpyAsync(badw.data(), F->d_badw.p, n_own * 4ull, cudaMemcpyDeviceToHost, st));
+    CUDA_TRY(cudaMemcpyAsync(need.data(), F->d_need.p, n_own * 8ull, cudaMemcpyDeviceToHost, st));
+    CUDA_TRY(cudaMemcpyAsync(&first_start, F->d_start.p, 8, cudaMemcpyDeviceToHost, st));
+    CUDA_TRY(cudaMemcpyAsync(&last_exit, F->d_exit.as<uint64_t>() + (n_own - 1), 8, cudaMemcpyDeviceToHost, st));
+    CUDA_TRY(cudaStreamSynchronize(st));
+    F->entry = entry == kNoEntry ? first_start : entry;
+    F->exit = last_exit;
+    for (uint32_t b = 0; b < n_own; ++b) {
+        if (!badw[b]) continue;
+        F->exit = kNoEntry;            // the chain is broken here (a malformed record), unless the halo is only too short
+        if (need[b] > F->usize) F->need = need[b];
+        break;
+    }
+    F->seconds[1] += since(t0);
+    return MMLST_OK;
+}
+
+extern "C" int mmlst_ingest_front_partition(mmlst_ingest_front* F, const int32_t* owner, int world) {
+    if (!F || world < 1 || world > kMaxShardRanks || (F->n_ref && !owner)) { mmlst_set_error("mmlst_ingest_front_partition: bad argument (world <= %d)", kMaxShardRanks); return MMLST_E_ARG; }
+    if (!F->walked || F->need) { mmlst_set_error("mmlst_ingest_front_partition: the record chain has not been walked to its end"); return MMLST_E_ARG; }
+    for (int32_t t = 0; t < F->n_ref; ++t)
+        if (owner[t] < 0 || owner[t] >= world) { mmlst_set_error("mmlst_ingest_front_partition: owner[%d] = %d outside [0, %d)", t, owner[t], world); return MMLST_E_ARG; }
+    CUDA_TRY(cudaSetDevice(F->device));
+    g_cur_stream = F->st;
+    cudaStream_t st = F->st;
+    const auto t0 = std::chrono::steady_clock::now();
+    F->world = world;
+    F->dest_records.assign(world, 0); F->dest_bytes.assign(world, 0);
+    F->unsorted = 0; F->keys[0] = F->keys[1] = 0; F->n_rec = 0; F->chain_err = kNoErr;
+    unsigned long long* err = F->d_err.as<unsigned long long>();
+    uint32_t* d_flags = reinterpret_cast<uint32_t*>(err + 2);
+    ING_TRY(F->send.alloc(16)); ING_TRY(F->send_len.alloc(16)); ING_TRY(F->send_idx.alloc(16));
+    const bool walks = F->n_own && !(F->entry != kNoEntry && F->entry >= F->uend);
+    if (!walks) { F->seconds[2] = since(t0); return MMLST_OK; }
+    const uint32_t nb = F->n_own;
+    const ChainArgs ca{F->I.d_u.as<uint8_t>(), F->usize, F->I.d_uoff.as<uint64_t>(), nb, F->entry, F->n_ref, F->d_reflen.as<uint32_t>(),
+                       F->d_start.as<uint64_t>(), F->d_exit.as<uint64_t>(), F->d_count.as<uint32_t>(), F->d_badw.as<uint32_t>(), F->uend, nullptr};
+    size_t tb = 0;
+    DBuf d_tmp;
+    CUDA_TRY(cub::DeviceScan::ExclusiveSum(nullptr, tb, F->d_count.as<uint32_t>(), F->d_base.as<uint32_t>(), nb + 1, st));
+    ING_TRY(d_tmp.alloc(tb));
+    CUDA_TRY(cudaMemsetAsync(F->d_count.as<uint32_t>() + nb, 0, 4, st));
+    CUDA_TRY(cub::DeviceScan::ExclusiveSum(d_tmp.p, tb, F->d_count.as<uint32_t>(), F->d_base.as<uint32_t>(), nb + 1, st));
+    uint32_t n32 = 0;
+    CUDA_TRY(cudaMemcpyAsync(&n32, F->d_base.as<uint32_t>() + nb, 4, cudaMemcpyDeviceToHost, st));
+    CUDA_TRY(cudaMemsetAsync(err + 1, 0xff, 8, st));
+    CUDA_TRY(cudaMemsetAsync(d_flags, 0, 4, st));
+    CUDA_TRY(cudaStreamSynchronize(st));
+    const uint64_t n = n32;
+    F->n_rec = n;
+    ING_TRY(F->d_roff.alloc(n * 8 + 8));
+    chain_offsets_kernel<<<(nb + kT - 1) / kT, kT, 0, st>>>(ca, F->d_base.as<uint32_t>(), F->d_roff.as<uint64_t>(), err + 1);
+    CUDA_TRY(cudaGetLastError());
+    if (n) {
+        const unsigned gn = static_cast<unsigned>((n + kT - 1) / kT);
+        ING_TRY(F->d_owner.alloc(static_cast<size_t>(F->n_ref) * 4 + 16));
+        if (F->n_ref) CUDA_TRY(cudaMemcpyAsync(F->d_owner.p, owner, static_cast<size_t>(F->n_ref) * 4, cudaMemcpyHostToDevice, st));
+        ING_TRY(F->d_dest.alloc(n * 4)); ING_TRY(F->d_rlen.alloc(n * 4)); ING_TRY(F->d_dcount.alloc(static_cast<size_t>(world) * 8)); ING_TRY(F->d_keys.alloc(16));
+        CUDA_TRY(cudaMemsetAsync(F->d_dcount.p, 0, static_cast<size_t>(world) * 8, st));
+        route_kernel<<<gn, kT, 0, st>>>(F->I.d_u.as<uint8_t>(), F->d_roff.as<uint64_t>(), n, F->n_ref, F->d_owner.as<int32_t>(), world, F->d_dest.as<uint32_t>(),
+                                        F->d_rlen.as<uint32_t>(), F->d_dcount.as<unsigned long long>(), d_flags, F->d_keys.as<uint64_t>());
+        CUDA_TRY(cudaGetLastError());
+        // stable partition by destination: LSD radix sort of (dest, shard index) over the bits a rank number needs
+        DBuf d_iota, d_dest2;
+        ING_TRY(d_iota.alloc(n * 4)); ING_TRY(F->d_order.alloc(n * 4)); ING_TRY(d_dest2.alloc(n * 4));
+        iota_kernel<<<gn, kT, 0, st>>>(d_iota.as<uint32_t>(), n);
+        CUDA_TRY(cudaGetLastError());
+        int end_bit = 1;
+        while ((1 << end_bit) < world) ++end_bit;
+        size_t sb = 0;
+        CUDA_TRY(cub::DeviceRadixSort::SortPairs(nullptr, sb, F->d_dest.as<uint32_t>(), d_dest2.as<uint32_t>(), d_iota.as<uint32_t>(), F->d_order.as<uint32_t>(),
+                                                 static_cast<int>(n), 0, end_bit, st));
+        DBuf d_stmp;
+        ING_TRY(d_stmp.alloc(sb));
+        CUDA_TRY(cub::DeviceRadixSort::SortPairs(d_stmp.p, sb, F->d_dest.as<uint32_t>(), d_dest2.as<uint32_t>(), d_iota.as<uint32_t>(), F->d_order.as<uint32_t>(),
+                                                 static_cast<int>(n), 0, end_bit, st));
+        DBuf d_plen;
+        ING_TRY(d_plen.alloc((n + 1) * 8)); ING_TRY(F->d_boff.alloc((n + 1) * 8));
+        part_len_kernel<<<static_cast<unsigned>((n + 1 + kT - 1) / kT), kT, 0, st>>>(F->d_order.as<uint32_t>(), F->d_rlen.as<uint32_t>(), n, d_plen.as<uint64_t>());
+        CUDA_TRY(cudaGetLastError());
+        CUDA_TRY(cub::DeviceScan::ExclusiveSum(nullptr, sb, d_plen.as<uint64_t>(), F->d_boff.as<uint64_t>(), static_cast<int>(n + 1), st));
+        ING_TRY(d_stmp.alloc(sb));
+        CUDA_TRY(cub::DeviceScan::ExclusiveSum(d_stmp.p, sb, d_plen.as<uint64_t>(), F->d_boff.as<uint64_t>(), static_cast<int>(n + 1), st));
+        uint64_t total = 0;
+        CUDA_TRY(cudaMemcpyAsync(&total, F->d_boff.as<uint64_t>() + n, 8, cudaMemcpyDeviceToHost, st));
+        CUDA_TRY(cudaMemcpyAsync(F->dest_records.data(), F->d_dcount.p, static_cast<size_t>(world) * 8, cudaMemcpyDeviceToHost, st));
+        CUDA_TRY(cudaStreamSynchronize(st));
+        ING_TRY(F->send.alloc(total + 16)); ING_TRY(F->send_len.alloc(n * 4)); ING_TRY(F->send_idx.alloc(n * 4));
+        partition_kernel<<<static_cast<unsigned>((n * 32 + kT - 1) / kT), kT, 0, st>>>(F->I.d_u.as<uint8_t>(), F->d_roff.as<uint64_t>(), F->d_order.as<uint32_t>(),
+                                                                                      F->d_rlen.as<uint32_t>(), F->d_boff.as<uint64_t>(), n, F->send.as<uint8_t>(),
+                                                                                      F->send_len.as<uint32_t>(), F->send_idx.as<uint32_t>());
+        CUDA_TRY(cudaGetLastError());
+        // bytes per destination: boff at the first record of every destination
+        std::vector<uint64_t> first(world + 1, 0);
+        for (int d = 0; d < world; ++d) first[d + 1] = first[d] + F->dest_records[d];
+        std::vector<uint64_t> at(world + 1, 0);
+        for (int d = 0; d <= world; ++d) CUDA_TRY(cudaMemcpyAsync(&at[d], F->d_boff.as<uint64_t>() + first[d], 8, cudaMemcpyDeviceToHost, st));
+        uint32_t fl = 0;
+        CUDA_TRY(cudaMemcpyAsync(&fl, d_flags, 4, cudaMemcpyDeviceToHost, st));
+        CUDA_TRY(cudaMemcpyAsync(F->keys, F->d_keys.p, 16, cudaMemcpyDeviceToHost, st));
+        CUDA_TRY(cudaStreamSynchronize(st));
+        for (int d = 0; d < world; ++d) F->dest_bytes[d] = at[d + 1] - at[d];
+        F->unsorted = fl & 1u;
+    }
+    CUDA_TRY(cudaMemcpyAsync(&F->chain_err, err + 1, 8, cudaMemcpyDeviceToHost, st));
+    CUDA_TRY(cudaStreamSynchronize(st));
+    F->seconds[2] = since(t0);
+    return MMLST_OK;
+}
+
+extern "C" int mmlst_ingest_front_info(const mmlst_ingest_front* F, mmlst_ingest_front_info_t* o) {
+    if (!F || !o) { mmlst_set_error("mmlst_ingest_front_info: null argument"); return MMLST_E_ARG; }
+    memset(o, 0, sizeof(*o));
+    o->n_blocks = F->nb; o->n_own_blocks = F->n_own; o->own_inflated = F->uend; o->inflated = F->usize; o->compressed = F->n_comp;
+    o->block_error = F->block_err; o->entry = F->entry; o->exit = F->exit; o->need = F->need; o->n_rec = F->n_rec; o->chain_error = F->chain_err;
+    o->repairs = F->repairs; o->world = F->world;
+    o->send = F->send.as<uint8_t>(); o->send_len = F->send_len.as<uint32_t>(); o->send_idx = F->send_idx.as<uint32_t>();
+    o->dest_records = F->dest_records.empty() ? nullptr : F->dest_records.data();
+    o->dest_bytes = F->dest_bytes.empty() ? nullptr : F->dest_bytes.data();
+    o->unsorted = F->unsorted; o->first_key = F->keys[0]; o->last_key = F->keys[1];
+    for (int i = 0; i < 3; ++i) o->seconds[i] = F->seconds[i];
+    return MMLST_OK;
+}
+
+extern "C" void mmlst_ingest_front_free(mmlst_ingest_front* F) {
+    if (!F) return;
+    cudaSetDevice(F->device);
+    cudaStreamSynchronize(F->st);
+    delete F;
+}
+
+extern "C" int mmlst_bam_ingest_back(int device, const uint8_t* recs, const uint32_t* rec_len, const uint32_t* file_idx, uint64_t n,
+                                     const mmlst_ingest_back_args* a, const mmlst_unpack_opts* opts_in, void* stream_in, mmlst_dev_bam** out,
+                                     uint64_t* error_out) {
+    if (error_out) *error_out = kNoErr;
+    if (!a || !out || (n && (!recs || !rec_len || !file_idx)) || a->n_ref < 0 || (a->n_ref && !a->ref_len)) {
+        mmlst_set_error("mmlst_bam_ingest_back: bad argument");
+        return MMLST_E_ARG;
+    }
+    const mmlst_unpack_opts o = ingest_opts(opts_in);
+    if (o.lenient_tags) { mmlst_set_error("mmlst_bam_ingest: lenient_tags is an option of the host unpacker (mmlst_bam_unpack)"); return MMLST_E_ARG; }
+    if (n >= 0x7fffff00ull) { mmlst_set_error("mmlst_bam_ingest_back: more than 2^31-257 records in one call"); return MMLST_E_RANGE; }
+    CUDA_TRY(cudaSetDevice(device));
+    cudaStream_t st = static_cast<cudaStream_t>(stream_in);
+    g_cur_stream = st;
+    cudaEvent_t ev[6];
+    for (auto& e : ev) CUDA_TRY(cudaEventCreate(&e));
+    struct EvGuard { cudaEvent_t* e; ~EvGuard() { for (int i = 0; i < 6; ++i) cudaEventDestroy(e[i]); } } evg{ev};
+    int evn = 0;
+    auto mark = [&]() { cudaEventRecord(ev[evn++], st); };
+    std::unique_ptr<mmlst_dev_bam> B(new mmlst_dev_bam());
+    B->device = device;
+    B->n_ref = static_cast<uint32_t>(a->n_ref);
+    B->ref_len.assign(a->ref_len, a->ref_len + a->n_ref);
+    B->names_blob = a->ref_names ? a->ref_names : "";
+    B->header_text = a->header_text ? a->header_text : "";
+    DBuf d_err, d_reflen, d_roff, d_w;
+    ING_TRY(d_err.alloc(8 + 32));
+    unsigned long long* err = d_err.as<unsigned long long>();
+    uint32_t* d_flags = reinterpret_cast<uint32_t*>(err + 1);
+    CUDA_TRY(cudaMemsetAsync(err, 0xff, 8, st));
+    CUDA_TRY(cudaMemsetAsync(d_flags, 0, 32, st));
+    mark();  // 0
+    ING_TRY(d_reflen.alloc(static_cast<size_t>(a->n_ref) * 4 + 16));
+    if (a->n_ref) CUDA_TRY(cudaMemcpyAsync(d_reflen.p, a->ref_len, static_cast<size_t>(a->n_ref) * 4, cudaMemcpyHostToDevice, st));
+    // record offsets in the received bytes: exclusive prefix of the lengths
+    ING_TRY(d_roff.alloc((n + 1) * 8)); ING_TRY(d_w.alloc((n + 1) * 8));
+    widen_kernel<<<static_cast<unsigned>((n + 1 + kT - 1) / kT), kT, 0, st>>>(rec_len, n, d_w.as<uint64_t>());
+    CUDA_TRY(cudaGetLastError());
+    {
+        size_t sb = 0;
+        CUDA_TRY(cub::DeviceScan::ExclusiveSum(nullptr, sb, d_w.as<uint64_t>(), d_roff.as<uint64_t>(), static_cast<int>(n + 1), st));
+        DBuf t;
+        ING_TRY(t.alloc(sb));
+        CUDA_TRY(cub::DeviceScan::ExclusiveSum(t.p, sb, d_w.as<uint64_t>(), d_roff.as<uint64_t>(), static_cast<int>(n + 1), st));
+    }
+    const BackIn in{recs, d_roff.as<uint64_t>(), file_idx, n, a->n_ref, d_reflen.as<uint32_t>(), err, d_flags, a->unsorted ? 1 : 0};
+    int phase = 0;
+    unsigned long long ew = kNoErr;
+    const int rc = back_half(in, o, st, B.get(), mark, &phase, &ew);
+    if (rc != MMLST_OK) {
+        if (error_out && phase) *error_out = (static_cast<uint64_t>(phase) << 56) | (ew == kNoErr ? 0ull : ew);
+        return rc;
+    }
+    B->explicit_idx = 1;   // also for an owner that received no record
+    if (!B->orig_idx.p) ING_TRY(B->orig_idx.alloc(4));
+    // phase seconds: parse, sort, score stream, cap + compaction, pack (slots 3..7 of the whole-file ingest)
+    for (int i = 0; i + 1 < evn && i < 5; ++i) { float ms = 0; cudaEventElapsedTime(&ms, ev[i], ev[i + 1]); B->seconds[3 + i] = ms * 1e-3; }
+    *out = B.release();
+    return MMLST_OK;
+}
+
+// The refusal a shard's ranks agreed on: (phase << 56 | record-or-block << 8 | code), phase 0 = a BGZF block, 1..4 = BackPhase.  Sets
+// the text the whole-file ingest gives for it and returns its code.
+extern "C" int mmlst_ingest_refusal(uint64_t e) {
+    const uint32_t phase = static_cast<uint32_t>(e >> 56), code = static_cast<uint32_t>(e & 0xff);
+    const unsigned long long at = (e & ((1ull << 56) - 1)) >> 8;
+    switch (phase) {
+        case 0:
+            if (code == E_CRC) mmlst_set_error("mmlst_bam_ingest: CRC mismatch in BGZF block %llu", at);
+            else mmlst_set_error("mmlst_bam_ingest: a BGZF block did not inflate to its ISIZE (corrupt file?)");
+            return MMLST_E_BAM;
+        case kPhaseRecord: mmlst_set_error("mmlst_bam_ingest: record %llu: %s", at, err_text(code)); return err_class(code);
+        case kPhaseUnsorted: mmlst_set_error("%s", kUnsortedText); return MMLST_E_UNSORTED;
+        case kPhasePlanes: mmlst_set_error("mmlst_bam_ingest: plane array exceeds 2^32 words"); return MMLST_E_RANGE;
+        case kPhasePileup: mmlst_set_error("mmlst_bam_ingest (pileup stream): record %llu: %s", at, err_text(code)); return err_class(code);
+        default: mmlst_set_error("mmlst_ingest_refusal: unknown phase %u", phase); return MMLST_E_ARG;
+    }
 }

@@ -184,6 +184,14 @@ EXPORTS = {
     "mmlst_bam_ingest": (C.c_int, [C.c_int, C.c_void_p, C.c_size_t, C.c_void_p, C.c_void_p, C.POINTER(C.c_void_p)]),
     "mmlst_dev_bam_info": (C.c_int, [C.c_void_p, C.c_void_p]),
     "mmlst_dev_bam_free": (None, [C.c_void_p]),
+    "mmlst_ingest_front_open": (C.c_int, [C.c_int, C.c_void_p, C.c_size_t, C.c_size_t, C.c_void_p, C.c_int32, C.c_int, C.c_void_p, C.POINTER(C.c_void_p)]),
+    "mmlst_ingest_front_walk": (C.c_int, [C.c_void_p, C.c_uint64]),
+    "mmlst_ingest_front_partition": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int]),
+    "mmlst_ingest_front_info": (C.c_int, [C.c_void_p, C.c_void_p]),
+    "mmlst_ingest_front_free": (None, [C.c_void_p]),
+    "mmlst_bam_ingest_back": (C.c_int, [C.c_int, C.c_void_p, C.c_void_p, C.c_void_p, C.c_uint64, C.c_void_p, C.c_void_p, C.c_void_p,
+                                        C.POINTER(C.c_void_p), C.POINTER(C.c_uint64)]),
+    "mmlst_ingest_refusal": (C.c_int, [C.c_uint64]),
     "mmlst_index_upload": (C.c_int, [C.c_void_p, C.c_void_p]),
     "mmlst_sample": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p]),
 }

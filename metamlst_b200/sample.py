@@ -248,14 +248,25 @@ class SampleTyper:
         """Host half of phase 1, safe on a prefetch thread: ingest="host" -> the unpacked streams (C++ threads); ingest="device" -> the
         file's bytes in page-locked memory (the GPU does the rest: `ingest`)."""
         if self.ingest == "device" and self.engine == "device":
+            if self._world() > 1:   # every rank reads only its share of the file (bam.ingest_bam_sharded)
+                return bam_path
             return bam.read_pinned(bam_path, bam.POOL)
         return self.unpack(bam_path)
+
+    def _world(self) -> int:
+        import torch
+        if torch.distributed.is_available() and torch.distributed.is_initialized():
+            return torch.distributed.get_world_size(self.group)
+        return 1
 
     def ingest_loaded(self, loaded, want_qhash: bool = False):
         """Device half of phase 1 for ingest="device": compressed bytes cross PCIe; inflate / parse / sort / depth cap / packing happen
         in HBM (csrc/ingest.cu).  A host-unpacked sample passes through."""
         if hasattr(loaded, "c_struct"):
             return loaded
+        if isinstance(loaded, str):   # one file over the ranks of the group: this rank's owned loci
+            return bam.ingest_bam_sharded(loaded, self.device, group=self.group, presorted=self.presorted, want_qhash=want_qhash,
+                                          check_crc=self.check_crc)
         st = bam.ingest_bam(loaded, self.device, presorted=self.presorted, want_qhash=want_qhash, check_crc=self.check_crc)
         bam.POOL.put(loaded)  # the call is synchronous: the staging buffer has been consumed
         return st
@@ -287,20 +298,23 @@ class SampleTyper:
         dist_on = torch.distributed.is_available() and torch.distributed.is_initialized() and torch.distributed.get_world_size(self.group) > 1
         rank = torch.distributed.get_rank(self.group) if dist_on else 0
         world = torch.distributed.get_world_size(self.group) if dist_on else 1
-        if isinstance(soa, streams.DeviceStreams):  # already resident (bam.ingest_bam)
+        exchange = "allreduce"
+        if isinstance(soa, streams.DeviceStreams):  # already resident (bam.ingest_bam / bam.ingest_bam_sharded)
+            if world > 1 and getattr(soa, "shard", None) is None:
+                raise ValueError("a sample ingested by one GPU is typed by that GPU; ingest it with bam.ingest_bam_sharded to type it on several")
             if world > 1:
-                raise ValueError("a device-ingested sample is typed by one GPU; shard a host-unpacked sample (ingest='host') over several")
+                exchange = "gather"   # owner mode: this rank holds the records of its own loci
             st = soa
         else:
             st = streams.DeviceStreams.from_soa(soa, dev, rank=rank, world=world, mode="ranges", want_qhash=want_qhash)
-        key = (tuple(soa.ref_names), np.asarray(soa.ref_lens).tobytes())
+        key = (tuple(soa.ref_names), np.asarray(soa.ref_lens).tobytes(), exchange)
         if self._pipe is None or self._pipe_key != key:
             index = api.AlleleIndex(soa.ref_names)
             table = self._allele_table()
             genes_in_db = {sp: len(self._genes(sp)) for sp in dict.fromkeys(index.species)}
             self._pipe = pipeline.DevicePipeline(st, index, lambda t: table.get(index.ref_names[t]) or "", minscore=self.minscore, max_xM=self.max_xM,
                                                  min_read_len=self.min_read_len, penalty=self.penalty, species_filter=self.species_filter,
-                                                 nloci=self.nloci, genes_in_db=genes_in_db, exchange="allreduce", group=self.group)
+                                                 nloci=self.nloci, genes_in_db=genes_in_db, exchange=exchange, group=self.group)
             self._pipe_key = key
         else:
             self._pipe.rebind(st)
