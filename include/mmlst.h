@@ -537,6 +537,12 @@ typedef struct {
 } mmlst_contig_stats_out;
 int mmlst_contig_stats(mmlst_ctx* ctx, const mmlst_soa* soa, const uint32_t* tid, uint32_t n, const uint32_t* col_off, int minscore,
                        int max_xm, const mmlst_contig_stats_params* prm, mmlst_contig_stats_out* out);
+/* The same call over a pileup stream RESIDENT in HBM (mmlst_bam_ingest, a DeviceStreams): d_recs / d_planes are the stream's DEVICE
+ * records and plane rows (16-byte aligned), max_row_words its widest row, contig_start its HOST [n_ref+1] record ranges.  Nothing is
+ * uploaded but the chunk list (records of the batch's contigs, plane_delta = 0) and col_off; same checks, refusals and outputs. */
+int mmlst_contig_stats_resident(mmlst_ctx* ctx, const mmlst_prec* d_recs, const uint32_t* d_planes, uint32_t max_row_words,
+                                const uint64_t* contig_start, uint32_t n_ref, const uint32_t* tid, uint32_t n, const uint32_t* col_off,
+                                int minscore, int max_xm, const mmlst_contig_stats_params* prm, mmlst_contig_stats_out* out);
 
 /* seam S3 (metamlst-merge.py:177-181): DB planes stay resident in the context across calls / samples. */
 int mmlst_db_upload(mmlst_ctx* ctx, const uint32_t* db_hi, const uint32_t* db_lo, const uint16_t* row_len,
@@ -635,10 +641,10 @@ typedef struct mmlst_bam mmlst_bam;
 typedef struct {
     int minqual; uint32_t max_depth; uint32_t sentinel_nodes; int n_threads; int pinned; int assume_sorted;
     int want_qhash; int check_crc;
-    /* HOST unpacker only (mmlst_bam_ingest refuses it).  0 = MetaMLST's own crash rules: a record whose 1st / 4th aux field is missing or not an integer,
+    /* Both unpackers (mmlst_bam_unpack, mmlst_bam_ingest and its sharded back half mmlst_bam_ingest_back).  0 = MetaMLST's own crash rules: a record whose 1st / 4th aux field is missing or not an integer,
      * or a pileup record without integer AS:i / XM:i tags, is MMLST_E_BAM.  1 = what a cmseq user without a tag filter gets from pysam: such records are
      * kept -- positional fields read as -32768 / 255 (no stage-1 filter ever passes them; the Python side refuses to SCORE a stream unpacked this way),
-     * missing named tags read as 0 and are counted in mmlst_bam_info_t.n_untagged, so that a caller who DOES pass a tag filter can raise the reference's
+     * missing named tags read as 0 and are counted in mmlst_bam_info_t.n_untagged (mmlst_dev_bam_info_t.n_untagged), so that a caller who DOES pass a tag filter can raise the reference's
      * KeyError (cmseq/cmseq.py:545) instead of filtering on invented values.  Proper-pair mates stay refused (H2). */
     int lenient_tags;
 } mmlst_unpack_opts;
@@ -685,6 +691,7 @@ typedef struct {
     uint64_t n_dropped_by_cap, n_unmapped_flag, n_bgzf_blocks, compressed_bytes, inflated_bytes;
     int presorted, minqual; uint32_t max_depth; int boundary_repairs;
     double seconds[8];              /* device time: H2D, inflate, record chain, parse, sort, score stream, depth cap + compaction, pack */
+    uint64_t n_untagged;            /* opts.lenient_tags: pileup records without integer AS:i / XM:i (0 otherwise: they are refused) */
 } mmlst_dev_bam_info_t;
 int mmlst_bam_ingest(int device, const uint8_t* bam, size_t n_bytes, const mmlst_unpack_opts* opts, void* stream, mmlst_dev_bam** out);
 int mmlst_dev_bam_info(const mmlst_dev_bam* bam, mmlst_dev_bam_info_t* info);

@@ -99,7 +99,7 @@ class DevBamInfo(C.Structure):
                 ("contig_start", C.c_void_p), ("ref_len", C.c_void_p), ("ref_names", C.c_char_p), ("header_text", C.c_char_p), ("n_ref", C.c_uint32),
                 ("n_dropped_by_cap", C.c_uint64), ("n_unmapped_flag", C.c_uint64), ("n_bgzf_blocks", C.c_uint64), ("compressed_bytes", C.c_uint64),
                 ("inflated_bytes", C.c_uint64), ("presorted", C.c_int), ("minqual", C.c_int), ("max_depth", C.c_uint32), ("boundary_repairs", C.c_int),
-                ("seconds", C.c_double * 8)]
+                ("seconds", C.c_double * 8), ("n_untagged", C.c_uint64)]
 
 
 class _DevHandle:
@@ -174,13 +174,14 @@ def read_pinned(path: str, pool: Optional[PinnedPool] = None):
 
 
 def ingest_bam(source, device=0, minqual: int = packing.DEFAULT_MINQUAL, max_depth: Optional[int] = packing.DEFAULT_MAX_DEPTH,
-               presorted: bool = False, want_qhash: bool = True, sentinel_nodes: int = 1, check_crc: bool = False):
+               presorted: bool = False, want_qhash: bool = True, sentinel_nodes: int = 1, check_crc: bool = False, lenient_tags: bool = False):
     """BAM -> streams.DeviceStreams WITHOUT the sample ever being unpacked on the host: the compressed file crosses PCIe, the
     hardware decompression engine inflates the BGZF blocks, kernels chain / parse / sort / depth-cap / pack the records
     (csrc/ingest.cu).  `source`: a path, or a uint8 torch tensor / numpy array holding the file's bytes (page-locked for an
     asynchronous copy: `read_pinned`).  Same streams, same refusals as `unpack_bam`; raises MmlstError(MMLST_E_CUDA) on a device
     without hardware DEFLATE.  `check_crc`: also check every BGZF block's CRC32 against its trailer on the device, as `unpack_bam`
-    always does (MmlstError(MMLST_E_BAM) "CRC mismatch in BGZF block k"); without it the DEFLATE stream and ISIZE are still checked."""
+    always does (MmlstError(MMLST_E_BAM) "CRC mismatch in BGZF block k"); without it the DEFLATE stream and ISIZE are still checked.
+    `lenient_tags`: as `unpack_bam` -- the streams are marked `lenient` (they cannot be scored) and carry `n_untagged`."""
     import torch
     dev = torch.device("cuda", device) if isinstance(device, int) else torch.device(device)
     data = read_pinned(source) if isinstance(source, str) else source
@@ -188,15 +189,15 @@ def ingest_bam(source, device=0, minqual: int = packing.DEFAULT_MINQUAL, max_dep
     nbytes = int(data.numel() if hasattr(data, "numel") else data.size)
     lib = native.lib()
     o = UnpackOpts(int(minqual), int(max_depth or 0), int(sentinel_nodes), 0, 1, 1 if presorted else 0, 1 if want_qhash else 0,
-                  1 if check_crc else 0, 0)
+                  1 if check_crc else 0, 1 if lenient_tags else 0)
     h = C.c_void_p()
     with torch.cuda.device(dev):
         stream = torch.cuda.current_stream(dev).cuda_stream
         native.check(lib.mmlst_bam_ingest(dev.index or 0, addr, nbytes, C.byref(o), stream, C.byref(h)))
-    return _dev_streams(_DevHandle(h), dev, want_qhash)
+    return _dev_streams(_DevHandle(h), dev, want_qhash, lenient_tags)
 
 
-def _dev_streams(keep, dev, want_qhash: bool):
+def _dev_streams(keep, dev, want_qhash: bool, lenient_tags: bool = False):
     """streams.DeviceStreams over the arrays of an mmlst_dev_bam handle (no copy: the handle stays alive with the streams)."""
     import torch
     from . import streams
@@ -233,21 +234,25 @@ def _dev_streams(keep, dev, want_qhash: bool):
     s.ingest_seconds = dict(zip(("h2d", "inflate", "chain", "parse", "sort", "score_stream", "cap_compact", "pack"), [float(x) for x in info.seconds]))
     s.ingest_stats = {"bgzf_blocks": int(info.n_bgzf_blocks), "compressed_bytes": int(info.compressed_bytes), "inflated_bytes": int(info.inflated_bytes),
                       "boundary_repairs": int(info.boundary_repairs), "unmapped_flag": int(info.n_unmapped_flag)}
+    if lenient_tags:   # pileup only: DevicePipeline refuses to score it, as the host score seams refuse a lenient SoaHost
+        s.lenient, s.n_untagged = True, int(info.n_untagged)
     return s
 
 
 def ingest_bam_sharded(path: str, device=0, group=None, locus_of=None, minqual: int = packing.DEFAULT_MINQUAL,
                        max_depth: Optional[int] = packing.DEFAULT_MAX_DEPTH, presorted: bool = False, want_qhash: bool = True,
-                       sentinel_nodes: int = 1, check_crc: bool = False):
+                       sentinel_nodes: int = 1, check_crc: bool = False, lenient_tags: bool = False):
     """One BAM ingested by every rank of a torch.distributed group (metamlst_b200/shard.py): this rank inflates and parses a 1/W share
     of the BGZF blocks and returns its streams.DeviceStreams, the records of the loci it owns (locus_of[tid] % W == rank; default:
     the loci of api.AlleleIndex over the header's reference names) -- what `DeviceStreams.from_soa(unpack_bam(path), mode="loci")`
     gives, with orig_idx the explicit file index and the pileup stream of the owned contigs only.  Same options and the same refusals
-    as `ingest_bam`: every rank raises the refusal the whole file gives, after the ranks agreed on it."""
+    as `ingest_bam`: every rank raises the refusal the whole file gives, after the ranks agreed on it.  With `lenient_tags` each rank's
+    `n_untagged` counts the untagged pileup records of its own contigs (their sum over the ranks is the file's)."""
     from . import shard
     coll = shard.TorchCollective(group)
     return coll.run(shard.ingest_steps(path, device, coll.rank, coll.world, locus_of=locus_of, minqual=minqual, max_depth=max_depth,
-                                       presorted=presorted, want_qhash=want_qhash, sentinel_nodes=sentinel_nodes, check_crc=check_crc))
+                                       presorted=presorted, want_qhash=want_qhash, sentinel_nodes=sentinel_nodes, check_crc=check_crc,
+                                       lenient_tags=lenient_tags))
 
 
 def ingest_bam_local(path: str, world: int, device=0, **kw):

@@ -21,6 +21,12 @@ the contigs into batches under a column budget; per batch ONE library call (`mml
 them and selects / compacts the columns on the device, and only the compacted columns come back.  The per-contig methods and these
 share one host definition of the reference's arithmetic (`_column_stats`, `_base_stats_dict`, `_poly_dict`, `_breadth_tuple`).
 
+Two ingest routes (`BamFile(..., ingest=)`): "host" (the default) unpacks on the host and uploads each batch; "device" ingests the
+compressed file on the GPU (`bam.ingest_bam`, lenient_tags, CRC checked) and keeps the streams in HBM, where `mmlst_contig_stats_resident`
+counts them without any upload.  With a `group` of W >= 2 ranks the device route is sharded by contig (`bam.ingest_bam_sharded`): rank r
+owns the contigs of a contiguous header range balanced by the sum of their lengths (`owner_map`), its `contigs` are the kept contigs it
+owns, so every `*_all` method returns this rank's share; `merge_rank_results` / `BamFile.gather` put the shares back together.
+
 Not carried over (each raises, nothing degrades silently): `trimReads` (the bit-planes carry no read coordinate),
 `BAM_tagFilter` entries other than `('AS','loc_gte',x)` / `('XM','loc_lte',y)` (the only ones MetaMLST passes,
 `metaMLST_functions.py:259`), `stepper='all'`, the GFF/codon functions (`parse_gff`, `baseline_PSR`,
@@ -89,10 +95,8 @@ class _BatchStats(NamedTuple):
 _WIDTH = {native.STATS_COLUMNS: 5, native.STATS_DEPTH: 1, native.STATS_LOWDOM: 2}
 
 
-def _bulk_stats(ctx: native.Context, soa, tids: Sequence[int], col_off: np.ndarray, minscore: int, max_xm: int,
-                prm: native.ContigStatsParams, want_cons: bool) -> _BatchStats:
-    """Pileup + column selection of a batch of contigs (tids ascending) in one library call.  The bulk seam the CPU tests answer with
-    the oracle's counts and a numpy restatement of the column rule."""
+def _stats_call(call, tids: Sequence[int], col_off: np.ndarray, prm: native.ContigStatsParams, want_cons: bool) -> _BatchStats:
+    """Output buffers of `mmlst_contig_stats[_resident]` for a batch; call(tid array, ContigStatsOut) makes the library call."""
     n, total = len(tids), int(col_off[-1])
     width = _WIDTH[prm.mode]
     sel_off, low_off, depth_off = np.zeros(n + 1, np.uint32), np.zeros(n + 1, np.uint32), np.zeros(n + 1, np.uint64)
@@ -100,12 +104,71 @@ def _bulk_stats(ctx: native.Context, soa, tids: Sequence[int], col_off: np.ndarr
     cons = np.empty(max(total, 1), np.uint8) if want_cons else None
     out = native.ContigStatsOut(native.ptr(sel_off), native.ptr(low_off), native.ptr(depth_off), native.ptr(cols), native.ptr(vals),
                                 native.ptr(cons), total, 0)
-    tid_arr = np.asarray(tids, dtype=np.uint32)
-    cs = soa.c_struct()
-    native.check(native.lib().mmlst_contig_stats(ctx.handle, C.byref(cs), native.ptr(tid_arr), n, native.ptr(col_off), int(minscore), int(max_xm),
-                                                 C.byref(prm), C.byref(out)))
+    native.check(call(np.asarray(tids, dtype=np.uint32), out))
     k = int(out.n_out)
     return _BatchStats(sel_off, low_off, depth_off, cols[:k], vals[:k], cons[:total] if want_cons else None)
+
+
+def _bulk_stats(ctx: native.Context, soa, tids: Sequence[int], col_off: np.ndarray, minscore: int, max_xm: int,
+                prm: native.ContigStatsParams, want_cons: bool) -> _BatchStats:
+    """Pileup + column selection of a batch of contigs (tids ascending) in one library call.  The bulk seam the CPU tests answer with
+    the oracle's counts and a numpy restatement of the column rule."""
+    cs = soa.c_struct()
+    return _stats_call(lambda tid_arr, out: native.lib().mmlst_contig_stats(ctx.handle, C.byref(cs), native.ptr(tid_arr), len(tids), native.ptr(col_off),
+                                                                            int(minscore), int(max_xm), C.byref(prm), C.byref(out)),
+                       tids, col_off, prm, want_cons)
+
+
+def _resident_stats(ctx: native.Context, streams, tids: Sequence[int], col_off: np.ndarray, minscore: int, max_xm: int,
+                    prm: native.ContigStatsParams, want_cons: bool) -> _BatchStats:
+    """`_bulk_stats` over device-resident streams (`bam.ingest_bam`): `mmlst_contig_stats_resident`, nothing uploaded.  The bulk seam of the
+    device route."""
+    cs = np.ascontiguousarray(streams.contig_start, dtype=np.uint64)
+    return _stats_call(lambda tid_arr, out: native.lib().mmlst_contig_stats_resident(
+        ctx.handle, native.ptr(streams.p_recs), native.ptr(streams.planes), int(streams.max_row_words), native.ptr(cs), len(cs) - 1,
+        native.ptr(tid_arr), len(tids), native.ptr(col_off), int(minscore), int(max_xm), C.byref(prm), C.byref(out)), tids, col_off, prm, want_cons)
+
+
+def _resident_counts(ctx: native.Context, streams, tid: int, minscore: int, max_xm: int) -> np.ndarray:
+    """counts[len][5] of one contig of device-resident streams: the columns with A+C+G+T >= 1 from `_resident_stats`, zeros elsewhere.  Exact
+    for every per-contig method, which reads only columns with A+C+G+T >= mincov >= 1.  The per-contig seam of the device route."""
+    ln = int(streams.ref_lens[tid])
+    prm = native.ContigStatsParams(native.STATS_COLUMNS, 1, 0, 0, 0.0)
+    r = _resident_stats(ctx, streams, [tid], np.array([0, ln], np.uint32), minscore, max_xm, prm, False)
+    counts = np.zeros((ln, 5), np.uint32)
+    counts[np.asarray(r.cols, dtype=np.int64)] = r.vals
+    return counts
+
+
+def _reads_per_contig(tid, n_ref: int) -> np.ndarray:
+    """Score-stream records per contig (minimumReadsAligning): counted on the device for device streams."""
+    if hasattr(tid, "is_cuda"):   # a torch tensor
+        import torch
+        return torch.bincount(tid.to(torch.int64), minlength=n_ref).cpu().numpy()
+    return np.bincount(np.asarray(tid, dtype=np.int64), minlength=n_ref)
+
+
+def owner_map(lengths: Sequence[int], world: int) -> np.ndarray:
+    """owner[tid] of a contig-sharded BamFile: rank r owns the contigs whose first column, as a prefix of LN in header order, lies in
+    [r * sum(LN) / W, (r + 1) * sum(LN) / W) -- contiguous header ranges of about equal length; a rank may own nothing."""
+    ln = np.asarray(lengths, dtype=np.int64)
+    start = np.concatenate([[0], np.cumsum(ln)[:-1]]) if ln.size else ln
+    total = int(ln.sum())
+    return ((start * int(world)) // max(total, 1)).astype(np.int32)
+
+
+def merge_rank_results(results: Sequence[dict], references: Sequence[str]) -> dict:
+    """The ranks' results of one `*_all` call of a contig-sharded BamFile as one dict: the disjoint union, in header order."""
+    merged = {}
+    for r in results:
+        for k, v in r.items():
+            if k in merged:
+                raise ValueError("contig %r appears in the results of two ranks" % (k,))
+            merged[k] = v
+    out = {name: merged[name] for name in references if name in merged}
+    if len(out) != len(merged):
+        raise KeyError("contigs not in the header: %r" % (sorted(set(merged) - set(out))[:5],))
+    return out
 
 
 # ---- the reference's host arithmetic, one definition for the per-contig and the whole-BAM methods ----------------------------------
@@ -250,7 +313,8 @@ class BamContig:
         self._check_stepper()
         h = self.bam_handle
         soa, minscore, max_xm = h._stream(min_base_quality, BAM_tagFilter)
-        return np.asarray(_contig_counts(h.ctx, soa, h._tid[self.name], minscore, max_xm))
+        counts_of = _resident_counts if h.ingest == "device" else _contig_counts
+        return np.asarray(counts_of(h.ctx, soa, h._tid[self.name], minscore, max_xm))
 
     def get_base_stats(self, min_read_depth=CMSEQ_DEFAULTS.mincov, min_base_quality=CMSEQ_DEFAULTS.minqual, error_rate=CMSEQ_DEFAULTS.poly_error_rate,
                        dominant_frq_thrsh=CMSEQ_DEFAULTS.poly_dominant_frq_thrsh, BAM_tagFilter=None, trimReads=None):
@@ -339,43 +403,97 @@ DEFAULT_COL_BUDGET = 1 << 26   # columns per batch: 1.3 GB of counts on the devi
 
 class BamFile:
     """cmseq/cmseq.py:35-88.  `sort` / `index` are accepted and need nothing: the unpacker puts the records in
-    `samtools sort` order in memory and the pileup needs no `.bai` (no `.sorted` / `.bai` files are written)."""
+    `samtools sort` order in memory and the pileup needs no `.bai` (no `.sorted` / `.bai` files are written).
+
+    ingest="host" unpacks the file on the host once per base-quality threshold; ingest="device" ingests it on the GPU (hardware DEFLATE,
+    MmlstError(MMLST_E_CUDA) on a device without it) and keeps the streams in HBM.  group: a torch.distributed group of W ranks (device
+    route only) -- the file is ingested sharded by contig (module text); every rank calls the `*_all` methods, `prepare` and `gather` with
+    the same arguments, since a threshold not yet resident is a collective ingest."""
     bam_handle = None
     bamFile = None
     contigs = {}
 
     def __init__(self, bamFile, sort=False, index=False, stepper='nofilter', minlen=CMSEQ_DEFAULTS.minlen, filterInputList=None,
-                 minimumReadsAligning=None, ctx: Optional[native.Context] = None, device: int = 0, minqual: int = CMSEQ_DEFAULTS.minqual):
+                 minimumReadsAligning=None, ctx: Optional[native.Context] = None, device: int = 0, minqual: int = CMSEQ_DEFAULTS.minqual,
+                 ingest: str = "host", group=None):
         if not os.path.isfile(bamFile):
             raise Exception(bamFile + ' is not accessible, or is not a file')
+        if ingest not in ("host", "device"):
+            raise ValueError("ingest must be 'host' or 'device'")
+        shards = group if isinstance(group, _LocalRank) else (_TorchShards(group) if group is not None else None)
+        if shards is not None and shards.world < 2:
+            shards = None
+        if shards is not None and ingest != "device":
+            raise ValueError("a group of %d ranks needs ingest='device'" % shards.world)
         self.bamFile = bamFile
         self.bam_handle = self
+        self.ingest, self.device, self._shards = ingest, int(device), shards
+        self.rank, self.world = (shards.rank, shards.world) if shards is not None else (0, 1)
         self._own_ctx = ctx is None
         self.ctx = ctx if ctx is not None else native.Context(device)
         self._soas: Dict[int, object] = {}
-        first = self._soa(int(minqual))  # header + the streams of the most likely threshold
+        self._untagged: Dict[int, int] = {}   # threshold -> pileup records of the FILE without AS:i / XM:i
+        self._reads: Optional[np.ndarray] = None
+        if shards is not None:
+            from . import shard
+            self._owner = owner_map(shard.read_header(bamFile)[2], self.world)
+        first = self._soa(int(minqual), collective=True)  # header + the streams of the most likely threshold
         self.references = tuple(first.ref_names)
         self.lengths = tuple(int(x) for x in first.ref_lens)
         self._tid = {r: i for i, r in enumerate(self.references)}
         keep = _wanted_contigs(filterInputList)  # upstream scans a list per reference (O(n_ref x n)); a set gives the same answer
-        n_on = np.bincount(np.asarray(first.tid, dtype=np.int64), minlength=len(self.references)) if minimumReadsAligning else None
-        self.contigs = dict((r, BamContig(self, r, l, stepper)) for i, (r, l) in enumerate(zip(self.references, self.lengths))
-                            if l > minlen and (keep is None or r in keep) and (not minimumReadsAligning or int(n_on[i]) >= minimumReadsAligning))
+        n_on = None
+        if minimumReadsAligning:
+            n_on = self._reads if self._reads is not None else _reads_per_contig(first.tid, len(self.references))
+        kept = [(r, l) for i, (r, l) in enumerate(zip(self.references, self.lengths))
+                if l > minlen and (keep is None or r in keep) and (not minimumReadsAligning or int(n_on[i]) >= minimumReadsAligning)]
+        self._kept = {r for r, _l in kept}
+        self.contigs = dict((r, BamContig(self, r, l, stepper)) for r, l in kept if self.owner_of(r) == self.rank)
 
-    def _stream(self, min_base_quality, BAM_tagFilter=None):
+    def owner_of(self, name: str) -> int:
+        """The rank that owns contig `name` (0 without a group)."""
+        return int(self._owner[self._tid[name]]) if self._shards is not None else 0
+
+    def prepare(self, *minquals) -> None:
+        """Ingest these base-quality thresholds now (a collective with a group; per-contig calls need their threshold resident)."""
+        for q in minquals:
+            self._soa(int(q), collective=True)
+
+    def gather(self, result: dict) -> dict:
+        """The union of every rank's result of one `*_all` call, in header order (merge_rank_results over an all-gather)."""
+        if self._shards is None:
+            return result
+        return merge_rank_results(self._shards.allgather(result), self.references)
+
+    def _stream(self, min_base_quality, BAM_tagFilter=None, collective=False):
         """(pileup stream at min_base_quality, minscore, max_xm) of a call with this tag filter."""
         minscore, max_xm = _tag_filter(BAM_tagFilter)
-        soa = self._soa(int(min_base_quality))
-        if BAM_tagFilter and getattr(soa, "n_untagged", 0):
+        q = int(min_base_quality)
+        soa = self._soa(q, collective)
+        if BAM_tagFilter and self._untagged[q]:
             # pysam's get_tag raises for the first read without the tag (cmseq/cmseq.py:545); the unpacker counts such reads per FILE, so this is
             # raised for any contig of a file that holds one -- stricter than upstream, never silently different
-            raise KeyError("tag 'AS' / 'XM' not present in %d pileup records of %s: a BAM_tagFilter cannot be evaluated (cmseq/cmseq.py:545)" % (soa.n_untagged, self.bamFile))
+            raise KeyError("tag 'AS' / 'XM' not present in %d pileup records of %s: a BAM_tagFilter cannot be evaluated (cmseq/cmseq.py:545)" % (self._untagged[q], self.bamFile))
         return soa, minscore, max_xm
 
-    def _soa(self, minqual: int):
+    def _soa(self, minqual: int, collective: bool = False):
         s = self._soas.get(minqual)
-        if s is None:
-            s = self._soas[minqual] = bam_mod.unpack_bam(self.bamFile, minqual=minqual, want_qhash=False, lenient_tags=True)
+        if s is not None:
+            return s
+        if self._shards is not None:
+            if not collective and not self._shards.resident(minqual):
+                raise RuntimeError("base quality %d is not resident on this rank of a sharded BamFile: call prepare(%d) on every rank first"
+                                   % (minqual, minqual))
+            s, self._untagged[minqual], reads = self._shards.ingest(self.bamFile, self.device, self._owner, minqual)
+            if self._reads is None:
+                self._reads = reads
+        elif self.ingest == "device":
+            s = bam_mod.ingest_bam(self.bamFile, self.device, minqual=minqual, want_qhash=False, lenient_tags=True, check_crc=True)
+            self._untagged[minqual] = int(s.n_untagged)
+        else:
+            s = bam_mod.unpack_bam(self.bamFile, minqual=minqual, want_qhash=False, lenient_tags=True)
+            self._untagged[minqual] = int(getattr(s, "n_untagged", 0))
+        self._soas[minqual] = s
         return s
 
     def get_contigs(self):
@@ -395,14 +513,15 @@ class BamFile:
         if contigs is None:
             chosen = list(self.contigs.values())
         else:
-            missing = [c for c in contigs if c not in self.contigs]
+            missing = [c for c in contigs if c not in self._kept]
             if missing:
                 raise KeyError("contigs not kept by this BamFile: %r" % (missing[:5],))
             wanted = set(contigs)
-            chosen = [c for name, c in self.contigs.items() if name in wanted]
+            chosen = [c for name, c in self.contigs.items() if name in wanted]   # with a group: those this rank owns
         for c in chosen:
             c._check_stepper()
-        soa, minscore, max_xm = self._stream(min_base_quality, BAM_tagFilter)
+        soa, minscore, max_xm = self._stream(min_base_quality, BAM_tagFilter, collective=True)
+        stats_of = _resident_stats if self.ingest == "device" else _bulk_stats
         prm = native.ContigStatsParams(mode, min(int(math.ceil(mincov)), 0xFFFFFFFF), int(trunc), none_char, float(dominant_frq_thrsh))
         width = _WIDTH[mode]
         empty = (0, np.zeros(0, np.int64), np.zeros((0, width), np.uint32), None)
@@ -418,7 +537,7 @@ class BamFile:
             if int(sum(c.length for c in batch)) > native.CONTIG_STATS_MAX_COLS:
                 raise native.MmlstError(native.E_RANGE, "contig %s has %d columns, one batch holds at most %d (5 * column in 32 bits)"
                                         % (batch[0].name, batch[0].length, native.CONTIG_STATS_MAX_COLS))
-            r = _bulk_stats(self.ctx, soa, tids, col_off, minscore, max_xm, prm, want_cons)
+            r = stats_of(self.ctx, soa, tids, col_off, minscore, max_xm, prm, want_cons)
             out_off = r.low_off if mode == native.STATS_LOWDOM else r.sel_off
             for i, c in enumerate(batch):
                 a, b = int(out_off[i]), int(out_off[i + 1])
@@ -526,3 +645,78 @@ class BamFile:
             self.ctx.close()
         self.ctx = None
         self._soas.clear()
+
+
+# ---- contig-sharded device route ----------------------------------------------------------------------------------------------------
+def _ingest_kw(owner, minqual):
+    return dict(locus_of=owner, minqual=minqual, want_qhash=False, lenient_tags=True, check_crc=True)
+
+
+def _file_totals(streams, n_ref: int) -> np.ndarray:
+    """[records per contig..., untagged pileup records] of one rank's streams, int64 on the streams' device (summed over the ranks)."""
+    import torch
+    t = torch.bincount(streams.tid.to(torch.int64), minlength=n_ref)
+    return torch.cat([t, torch.tensor([int(streams.n_untagged)], dtype=torch.int64, device=t.device)])
+
+
+class _TorchShards:
+    """One rank of a torch.distributed group: collective ingest (bam.ingest_bam_sharded) and all-gather."""
+
+    def __init__(self, group):
+        import torch.distributed as dist
+        self.group = group
+        self.rank, self.world = dist.get_rank(group), dist.get_world_size(group)
+
+    def ingest(self, path, device, owner, minqual):
+        import torch.distributed as dist
+        s = bam_mod.ingest_bam_sharded(path, device, self.group, **_ingest_kw(owner, minqual))
+        tot = _file_totals(s, len(s.ref_names))
+        dist.all_reduce(tot, group=self.group)
+        tot = tot.cpu().numpy()
+        return s, int(tot[-1]), tot[:-1]
+
+    def resident(self, minqual):
+        return False
+
+    def allgather(self, obj):
+        import torch.distributed as dist
+        out = [None] * self.world
+        dist.all_gather_object(out, obj, group=self.group)
+        return out
+
+
+class _LocalGroup:
+    """The W ranks of one file in one process (open_local): a threshold any rank needs is ingested for every rank at once (shard.run_local)."""
+
+    def __init__(self, world: int):
+        self.world = world
+        self.ingested: Dict[int, tuple] = {}   # threshold -> (every rank's streams, untagged records of the file, records per contig)
+
+
+class _LocalRank:
+    def __init__(self, g: _LocalGroup, rank: int):
+        self.g, self.rank, self.world = g, rank, g.world
+
+    def ingest(self, path, device, owner, minqual):
+        got = self.g.ingested.get(minqual)
+        if got is None:
+            from . import shard
+            ranks = shard.run_local([shard.ingest_steps(path, device, r, self.world, **_ingest_kw(owner, minqual)) for r in range(self.world)])
+            tot = sum(_file_totals(s, len(s.ref_names)) for s in ranks).cpu().numpy()
+            got = self.g.ingested[minqual] = [ranks, int(tot[-1]), tot[:-1]]
+        s = got[0][self.rank]
+        got[0][self.rank] = None   # the rank's handle keeps its streams; the group forgets them
+        return s, got[1], got[2]
+
+    def resident(self, minqual):
+        return minqual in self.g.ingested
+
+    def allgather(self, obj):
+        raise ValueError("the ranks of open_local run in turn in one process: merge their results with merge_rank_results")
+
+
+def open_local(path: str, world: int, device: int = 0, **kw) -> List[BamFile]:
+    """Every rank of a `world`-rank contig-sharded BamFile(ingest="device") in this process on one device, for tests: the W handles.  They
+    share one local group, so a threshold that any of them needs is ingested for all ranks at once."""
+    g = _LocalGroup(int(world))
+    return [BamFile(path, device=device, ingest="device", group=_LocalRank(g, r), **kw) for r in range(int(world))]

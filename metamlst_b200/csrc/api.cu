@@ -685,9 +685,10 @@ extern "C" int mmlst_pileup_consensus(mmlst_ctx* c, const mmlst_soa* soa, const 
     return MMLST_OK;
 }
 
-extern "C" int mmlst_contig_stats(mmlst_ctx* c, const mmlst_soa* soa, const uint32_t* tid, uint32_t n, const uint32_t* col_off, int minscore,
-                                  int max_xm, const mmlst_contig_stats_params* prm, mmlst_contig_stats_out* out) {
-    if (!soa || !tid || !col_off || !prm || !out || !out->sel_off || !out->low_off || !out->depth_off) { mmlst_set_error("mmlst_contig_stats: null pointer"); return MMLST_E_ARG; }
+// The checks of mmlst_contig_stats / mmlst_contig_stats_resident, before anything else: *width = u32 per compacted column.
+static int contig_stats_check(const uint32_t* tid, uint32_t n, const uint32_t* col_off, const mmlst_contig_stats_params* prm,
+                              mmlst_contig_stats_out* out, uint32_t* width) {
+    if (!tid || !col_off || !prm || !out || !out->sel_off || !out->low_off || !out->depth_off) { mmlst_set_error("mmlst_contig_stats: null pointer"); return MMLST_E_ARG; }
     if (col_off[0] != 0) { mmlst_set_error("mmlst_contig_stats: col_off[0] = %u, not 0", col_off[0]); return MMLST_E_ARG; }
     for (uint32_t i = 0; i < n; ++i) {
         if (col_off[i + 1] < col_off[i]) { mmlst_set_error("mmlst_contig_stats: col_off not ascending at %u", i); return MMLST_E_ARG; }
@@ -699,15 +700,20 @@ extern "C" int mmlst_contig_stats(mmlst_ctx* c, const mmlst_soa* soa, const uint
         return MMLST_E_RANGE;
     }
     if (prm->mode > MMLST_STATS_LOWDOM || prm->mincov == 0 || prm->none_char > 255) { mmlst_set_error("mmlst_contig_stats: mode %u / mincov %u / none_char %u out of range", prm->mode, prm->mincov, prm->none_char); return MMLST_E_ARG; }
-    const uint32_t width = prm->mode == MMLST_STATS_COLUMNS ? 5u : prm->mode == MMLST_STATS_DEPTH ? 1u : 2u;
+    *width = prm->mode == MMLST_STATS_COLUMNS ? 5u : prm->mode == MMLST_STATS_DEPTH ? 1u : 2u;
     if (out->capacity && (!out->out_col || !out->out_val)) { mmlst_set_error("mmlst_contig_stats: null pointer"); return MMLST_E_ARG; }
     out->n_out = 0;
-    if (n == 0) { out->sel_off[0] = 0; out->low_off[0] = 0; out->depth_off[0] = 0; return MMLST_OK; }
-    CTX_ENTER(c);
+    if (n == 0) { out->sel_off[0] = 0; out->low_off[0] = 0; out->depth_off[0] = 0; }
+    return MMLST_OK;
+}
+
+// The device half of both: pileup of the batch's chunks (already in c->chunks) over recs / planes -> mmlst_contig_stats_dev -> the
+// prefixes, then the compacted columns they size, back to the host.
+static int contig_stats_batch(mmlst_ctx* c, const mmlst_prec* recs, const uint32_t* planes, uint32_t n_chunks, uint32_t max_row_words, uint32_t n,
+                              const uint32_t* col_off, int minscore, int max_xm, const mmlst_contig_stats_params* prm, uint32_t width,
+                              mmlst_contig_stats_out* out) {
     cudaStream_t s = c->stream;
-    mmlst_trace_mark("enter");
-    std::vector<mmlst_chunk> chunks;
-    TRY(upload_chosen_contigs(c, soa, tid, n, col_off, chunks, false, true));
+    const uint32_t total_cols = col_off[n];
     TRY(h2d(c->col_off, col_off, (size_t)n + 1, s));
     const size_t scratch = mmlst_contig_stats_scratch_bytes(total_cols);
     TRY(c->counts.reserve((size_t)total_cols * 20 + 16)); TRY(c->cs_scratch.reserve(scratch));
@@ -717,8 +723,7 @@ extern "C" int mmlst_contig_stats(mmlst_ctx* c, const mmlst_soa* soa, const uint
     uint64_t* d_dep = reinterpret_cast<uint64_t*>(c->cs_off.as<uint8_t>() + (((size_t)n + 1) * 8 + 15) / 16 * 16);
     uint32_t* d_col = c->cs_out.as<uint32_t>(); uint32_t* d_val = d_col + total_cols;
     CUDA_TRY(cudaMemsetAsync(c->counts.p, 0, (size_t)total_cols * 20, s));
-    TRY(mmlst_pileup_dev(c->p_recs.as<mmlst_prec>(), c->planes.as<uint32_t>(), c->chunks.as<mmlst_chunk>(), (uint32_t)chunks.size(),
-                         soa->max_row_words, minscore, max_xm, c->counts.as<uint32_t>(), total_cols, 0, s));
+    TRY(mmlst_pileup_dev(recs, planes, c->chunks.as<mmlst_chunk>(), n_chunks, max_row_words, minscore, max_xm, c->counts.as<uint32_t>(), total_cols, 0, s));
     TRY(mmlst_contig_stats_dev(c->counts.as<uint32_t>(), c->col_off.as<uint32_t>(), n, total_cols, prm, c->cs_scratch.p, scratch, d_sel, d_low, d_dep,
                                d_col, d_val, out->cons ? c->cons.as<uint8_t>() : nullptr, 0, s));
     CUDA_TRY(cudaMemcpyAsync(out->sel_off, d_sel, ((size_t)n + 1) * 4, cudaMemcpyDeviceToHost, s));
@@ -738,6 +743,58 @@ extern "C" int mmlst_contig_stats(mmlst_ctx* c, const mmlst_soa* soa, const uint
     mmlst_trace_mark("sync");
     mmlst_trace_flush("mmlst_contig_stats");
     return MMLST_OK;
+}
+
+extern "C" int mmlst_contig_stats(mmlst_ctx* c, const mmlst_soa* soa, const uint32_t* tid, uint32_t n, const uint32_t* col_off, int minscore,
+                                  int max_xm, const mmlst_contig_stats_params* prm, mmlst_contig_stats_out* out) {
+    if (!soa) { mmlst_set_error("mmlst_contig_stats: null pointer"); return MMLST_E_ARG; }
+    uint32_t width = 0;
+    TRY(contig_stats_check(tid, n, col_off, prm, out, &width));
+    if (n == 0) return MMLST_OK;
+    CTX_ENTER(c);
+    mmlst_trace_mark("enter");
+    std::vector<mmlst_chunk> chunks;
+    TRY(upload_chosen_contigs(c, soa, tid, n, col_off, chunks, false, true));
+    return contig_stats_batch(c, c->p_recs.as<mmlst_prec>(), c->planes.as<uint32_t>(), (uint32_t)chunks.size(), soa->max_row_words, n, col_off,
+                              minscore, max_xm, prm, width, out);
+}
+
+extern "C" int mmlst_contig_stats_resident(mmlst_ctx* c, const mmlst_prec* d_recs, const uint32_t* d_planes, uint32_t max_row_words,
+                                           const uint64_t* contig_start, uint32_t n_ref, const uint32_t* tid, uint32_t n, const uint32_t* col_off,
+                                           int minscore, int max_xm, const mmlst_contig_stats_params* prm, mmlst_contig_stats_out* out) {
+    if (!contig_start) { mmlst_set_error("mmlst_contig_stats_resident: null pointer"); return MMLST_E_ARG; }
+    uint32_t width = 0;
+    TRY(contig_stats_check(tid, n, col_off, prm, out, &width));
+    if (n == 0) return MMLST_OK;
+    uint64_t n_rec = 0;
+    for (uint32_t i = 0; i < n; ++i) {
+        if (tid[i] >= n_ref) { mmlst_set_error("mmlst_contig_stats_resident: tid[%u]=%u out of range", i, tid[i]); return MMLST_E_ARG; }
+        if (contig_start[tid[i] + 1] < contig_start[tid[i]] || contig_start[tid[i] + 1] > 0xffffffffull) {
+            mmlst_set_error("mmlst_contig_stats_resident: contig_start of contig %u is not a record range", tid[i]);
+            return MMLST_E_ARG;
+        }
+        n_rec += contig_start[tid[i] + 1] - contig_start[tid[i]];
+    }
+    if (n_rec && (!d_recs || !d_planes)) { mmlst_set_error("mmlst_contig_stats_resident: null pointer"); return MMLST_E_ARG; }
+    CTX_ENTER(c);
+    mmlst_trace_mark("enter");
+    // the chunk rule of upload_chosen_contigs over the stream's own record indices: the rows are where the stream keeps them
+    std::vector<mmlst_chunk> chunks;
+    const uint32_t kChunkRecords = mmlst_chunk_records(n_rec);
+    for (uint32_t i = 0; i < n; ++i) {
+        const uint64_t q0 = contig_start[tid[i]], q1 = contig_start[tid[i] + 1];
+        for (uint64_t b = q0; b < q1; b += kChunkRecords) {
+            mmlst_chunk ck{};
+            ck.rec_begin = (uint32_t)b;
+            ck.rec_end = (uint32_t)std::min<uint64_t>(q1, b + kChunkRecords);
+            ck.col_base = col_off[i];
+            ck.contig_len = col_off[i + 1] - col_off[i];
+            ck.plane_delta = 0;
+            chunks.push_back(ck);
+        }
+    }
+    TRY(h2d(c->chunks, chunks.data(), chunks.size(), c->stream));
+    return contig_stats_batch(c, d_recs, d_planes, (uint32_t)chunks.size(), max_row_words, n, col_off, minscore, max_xm, prm, width, out);
 }
 
 // ---------------------------------------------------------------------------------------------------------------

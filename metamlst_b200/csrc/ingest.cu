@@ -348,12 +348,12 @@ struct ParseOut {
 
 // gidx (shards): file index of record i, for the refusal text; nullptr = i
 __global__ void __launch_bounds__(kT) parse_kernel(const uint8_t* u, const uint64_t* roff, const uint32_t* gidx, uint64_t n, int32_t n_ref, ParseOut o,
-                                                   unsigned long long* err) {
+                                                   bool lenient, unsigned long long* err) {
     const uint64_t i = static_cast<uint64_t>(blockIdx.x) * kT + threadIdx.x;
     if (i >= n) return;
     Core c;
     uint64_t qh[2];
-    const uint32_t e = parse_record(u, roff[i], n_ref, &c, o.qh ? qh : nullptr);
+    const uint32_t e = parse_record(u, roff[i], n_ref, &c, o.qh ? qh : nullptr, lenient);
     if (e != E_NONE) { report(err, gidx ? gidx[i] : i, e); o.key[i] = ~0ull; return; }
     o.key[i] = c.key; o.reflen[i] = static_cast<uint16_t>(c.reflen); o.as0[i] = c.as0; o.asn[i] = c.asn; o.qlen[i] = c.qlen;
     o.xm3[i] = c.xm3; o.xmn[i] = c.xmn; o.bits[i] = c.bits;
@@ -526,6 +526,7 @@ struct PackArgs {
     const uint8_t* u; const uint32_t* list; uint64_t P; const uint64_t* rowoff;
     const int32_t* s_pos; const uint16_t* s_reflen; const uint8_t* s_bits; const int16_t* s_asn; const uint8_t* s_xmn; const uint64_t* s_roff;
     const uint32_t* orig_idx; int minqual; mmlst_prec* recs; uint32_t* planes;
+    int lenient; uint32_t* n_untagged;   // opts.lenient_tags: records without integer AS:i / XM:i are packed and counted here
 };
 
 // one WARP per admitted record: lane = contig column inside the 32-column word being built; every lane finds the query base aligned to
@@ -551,8 +552,9 @@ __global__ void __launch_bounds__(kT) pack_kernel(const PackArgs a, unsigned lon
     const uint8_t* seq = cig + 4ull * n_cig;
     const uint8_t* qual = seq + (static_cast<uint64_t>(l_seq) + 1) / 2;
     uint32_t e = E_NONE;
-    if (!(a.s_bits[k] & 2u)) e = E_NAMED;
+    if (!(a.s_bits[k] & 2u) && !a.lenient) e = E_NAMED;
     else if (l_seq && qual[0] == 0xff) e = E_NOQUAL;
+    else if (!(a.s_bits[k] & 2u) && lane == 0) atomicAdd(a.n_untagged, 1u);
     if (e != E_NONE) {
         for (uint32_t w = lane; w < rw; w += 32) row[w] = 0;
         if (lane == 0) report(err, a.orig_idx ? a.orig_idx[k] : k, e);
@@ -608,7 +610,7 @@ struct mmlst_dev_bam {
     std::vector<uint64_t> contig_start;
     std::vector<uint32_t> ref_len;
     std::string names_blob, header_text;
-    uint64_t n_rec = 0, n_prec = 0, n_plane_words = 0, n_dropped = 0, n_unmapped = 0, n_blocks = 0, comp_bytes = 0, infl_bytes = 0;
+    uint64_t n_rec = 0, n_prec = 0, n_plane_words = 0, n_dropped = 0, n_unmapped = 0, n_blocks = 0, comp_bytes = 0, infl_bytes = 0, n_untagged = 0;
     uint32_t n_runs = 0, max_row_words = 0, n_ref = 0, max_depth = 0, repairs = 0;
     int presorted = 0, minqual = 20, qc = 0, explicit_idx = 0;   // explicit_idx: a shard's streams carry orig_idx even in file order
     double seconds[8] = {0, 0, 0, 0, 0, 0, 0, 0};
@@ -653,6 +655,7 @@ extern "C" int mmlst_dev_bam_info(const mmlst_dev_bam* b, mmlst_dev_bam_info_t* 
     o->compressed_bytes = b->comp_bytes; o->inflated_bytes = b->infl_bytes;
     o->presorted = b->presorted; o->minqual = b->minqual; o->max_depth = b->max_depth; o->boundary_repairs = static_cast<int>(b->repairs);
     for (int i = 0; i < 8; ++i) o->seconds[i] = b->seconds[i];
+    o->n_untagged = b->n_untagged;
     return MMLST_OK;
 }
 
@@ -822,7 +825,7 @@ int back_half(const BackIn& in, const mmlst_unpack_opts& o, cudaStream_t st, mml
                       k_xmn.as<uint8_t>(), k_bits.as<uint8_t>(), o.want_qhash ? k_qh.as<uint64_t>() : nullptr};
     const unsigned gn = static_cast<unsigned>((n + kT - 1) / kT);
     if (n) {
-        parse_kernel<<<gn, kT, 0, st>>>(in.u, in.roff, in.gidx, n, n_ref, po, err);
+        parse_kernel<<<gn, kT, 0, st>>>(in.u, in.roff, in.gidx, n, n_ref, po, o.lenient_tags != 0, err);
         CUDA_TRY(cudaGetLastError());
         check_sorted_kernel<<<gn, kT, 0, st>>>(k_key.as<uint64_t>(), n, d_flags);
         CUDA_TRY(cudaGetLastError());
@@ -969,15 +972,18 @@ int back_half(const BackIn& in, const mmlst_unpack_opts& o, cudaStream_t st, mml
     if (P) {
         const PackArgs pa{in.u, d_list.as<uint32_t>(), P, d_rowoff.as<uint64_t>(), s_pos.as<int32_t>(), s_reflen.as<uint16_t>(), s_bits.as<uint8_t>(),
                           s_asn.as<int16_t>(), s_xmn.as<uint8_t>(), s_roff.as<uint64_t>(), keep_idx ? B->orig_idx.as<uint32_t>() : nullptr, o.minqual,
-                          B->p_recs.as<mmlst_prec>(), B->planes.as<uint32_t>()};
+                          B->p_recs.as<mmlst_prec>(), B->planes.as<uint32_t>(), o.lenient_tags != 0, d_flags + 5};
         pack_kernel<<<static_cast<unsigned>((P * 32 + kT - 1) / kT), kT, 0, st>>>(pa, err);
         CUDA_TRY(cudaGetLastError());
     }
     mark();  // 8
+    uint32_t n_untagged = 0;
+    CUDA_TRY(cudaMemcpyAsync(&n_untagged, d_flags + 5, 4, cudaMemcpyDeviceToHost, st));
     {
         const int rc = fetch_error(err, st, "mmlst_bam_ingest (pileup stream)", err_word);
         if (rc != MMLST_OK) { *phase = kPhasePileup; return rc; }
     }
+    B->n_untagged = n_untagged;
     B->n_unmapped = fl[4];
     B->n_dropped = n - fl[4] - P;
     B->minqual = o.minqual; B->max_depth = o.max_depth;
@@ -997,7 +1003,6 @@ mmlst_unpack_opts ingest_opts(const mmlst_unpack_opts* opts_in) {
 extern "C" int mmlst_bam_ingest(int device, const uint8_t* bam, size_t n_bytes, const mmlst_unpack_opts* opts_in, void* stream_in, mmlst_dev_bam** out) {
     if (!bam || !out) { mmlst_set_error("mmlst_bam_ingest: null argument"); return MMLST_E_ARG; }
     const mmlst_unpack_opts o = ingest_opts(opts_in);
-    if (o.lenient_tags) { mmlst_set_error("mmlst_bam_ingest: lenient_tags is an option of the host unpacker (mmlst_bam_unpack)"); return MMLST_E_ARG; }
     CUDA_TRY(cudaSetDevice(device));
     cudaStream_t st = static_cast<cudaStream_t>(stream_in);
     g_cur_stream = st;
@@ -1022,7 +1027,8 @@ extern "C" int mmlst_bam_ingest(int device, const uint8_t* bam, size_t n_bytes, 
     DBuf d_err;
     ING_TRY(d_err.alloc(8 + 32));
     unsigned long long* err = d_err.as<unsigned long long>();
-    uint32_t* d_flags = reinterpret_cast<uint32_t*>(err + 1);   // [0] sortedness, [1] repair counter, [2] uniform qlen, [3] max row words, [4] records with the unmapped flag
+    uint32_t* d_flags = reinterpret_cast<uint32_t*>(err + 1);   // [0] sortedness, [1] repair counter, [2] uniform qlen, [3] max row words, [4] records with the unmapped flag,
+                                                                //  [5] untagged pileup records (lenient_tags)
     CUDA_TRY(cudaMemsetAsync(err, 0xff, 8, st));
     CUDA_TRY(cudaMemsetAsync(d_flags, 0, 32, st));
     mark();  // 0
@@ -1353,7 +1359,6 @@ extern "C" int mmlst_bam_ingest_back(int device, const uint8_t* recs, const uint
         return MMLST_E_ARG;
     }
     const mmlst_unpack_opts o = ingest_opts(opts_in);
-    if (o.lenient_tags) { mmlst_set_error("mmlst_bam_ingest: lenient_tags is an option of the host unpacker (mmlst_bam_unpack)"); return MMLST_E_ARG; }
     if (n >= 0x7fffff00ull) { mmlst_set_error("mmlst_bam_ingest_back: more than 2^31-257 records in one call"); return MMLST_E_RANGE; }
     CUDA_TRY(cudaSetDevice(device));
     cudaStream_t st = static_cast<cudaStream_t>(stream_in);

@@ -134,8 +134,9 @@ ING_HD uint64_t hash64b(const uint8_t* s, uint32_t n) {
 }
 
 // One record at u + off (off from the record chain, so block_size is sane).  Returns E_NONE or the first refusal, in the order
-// bam_unpack.cpp tests them.  qh: 2 x u64 or nullptr.
-ING_HD uint32_t parse_record(const uint8_t* u, uint64_t off, int32_t n_ref, Core* out, uint64_t* qh) {
+// bam_unpack.cpp tests them.  qh: 2 x u64 or nullptr.  lenient (opts.lenient_tags, bam_unpack.cpp's rule): a record whose 1st / 4th
+// aux field is missing, not an integer, outside int16 / negative keeps as0 = -32768, xm3 = 255 instead of E_AUXPOS / E_AS0 / E_XM3.
+ING_HD uint32_t parse_record(const uint8_t* u, uint64_t off, int32_t n_ref, Core* out, uint64_t* qh, bool lenient = false) {
     const uint8_t* r = u + off;
     const uint32_t bs = rd32(r);
     const uint8_t* end = r + 4 + bs;
@@ -180,9 +181,13 @@ ING_HD uint32_t parse_record(const uint8_t* u, uint64_t off, int32_t n_ref, Core
         if (isint && a2[0] == 'X' && a2[1] == 'M' && !okxm) { okxm = true; vxm = v; }
         a2 = val + sz;
     }
-    if (field < 4 || !ok0 || !ok3) return E_AUXPOS;
-    if (v0 < -32768 || v0 > 32767) return E_AS0;
-    if (v3 < 0) return E_XM3;
+    if (lenient && (field < 4 || !ok0 || !ok3 || v0 < -32768 || v0 > 32767 || v3 < 0)) {
+        v0 = -32768; v3 = 255;   // values no stage-1 filter passes: a lenient stream is never scored
+    } else {
+        if (field < 4 || !ok0 || !ok3) return E_AUXPOS;
+        if (v0 < -32768 || v0 > 32767) return E_AS0;
+        if (v3 < 0) return E_XM3;
+    }
     c.as0 = static_cast<int16_t>(v0);
     c.xm3 = static_cast<uint8_t>(v3 < 255 ? v3 : 255);
     const bool named_ok = okas && okxm && vas >= -32768 && vas <= 32767 && vxm >= 0;
@@ -202,11 +207,12 @@ ING_HD uint32_t row_words(uint32_t nw) {  // 3 planes, padded to an odd word cou
 
 // The record's plane row (include/mmlst.h: word-interleaved [V, B1, B0] per 32 contig columns, aligned to the contig's words).
 // `row` (rw words) is written completely.  Returns E_NONE, E_NAMED or E_NOQUAL (the record is in the pileup: what pysam would
-// raise on, cmseq/cmseq.py:538,545).
-ING_HD uint32_t pack_record(const uint8_t* u, uint64_t off, uint32_t pos, uint32_t reflen, bool named_ok, int minqual, uint32_t* row, uint32_t rw) {
+// raise on, cmseq/cmseq.py:538,545).  lenient: a record without integer AS:i / XM:i is packed like any other (the caller counts it).
+ING_HD uint32_t pack_record(const uint8_t* u, uint64_t off, uint32_t pos, uint32_t reflen, bool named_ok, int minqual, uint32_t* row, uint32_t rw,
+                            bool lenient = false) {
     for (uint32_t w = 0; w < rw; ++w) row[w] = 0;
     if (reflen == 0) return E_NONE;
-    if (!named_ok) return E_NAMED;
+    if (!named_ok && !lenient) return E_NAMED;
     const uint8_t* r = u + off;
     const uint32_t l_name = r[12], n_cig = rd16(r + 16), l_seq = rd32(r + 20);
     const uint8_t* cig = r + 36 + l_name;

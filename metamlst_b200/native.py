@@ -140,6 +140,8 @@ EXPORTS = {
                                + [C.c_void_p] * 6 + [C.c_uint32, C.c_void_p]),
     "mmlst_contig_stats": (C.c_int, [C.c_void_p, C.POINTER(Soa), C.c_void_p, C.c_uint32, C.c_void_p, C.c_int, C.c_int,
                                      C.POINTER(ContigStatsParams), C.POINTER(ContigStatsOut)]),
+    "mmlst_contig_stats_resident": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_uint32, C.c_void_p, C.c_uint32, C.c_void_p, C.c_uint32,
+                                              C.c_void_p, C.c_int, C.c_int, C.POINTER(ContigStatsParams), C.POINTER(ContigStatsOut)]),
     "mmlst_xchg_publish_dev": (C.c_int, [C.c_void_p, C.c_uint32, C.c_void_p, C.c_uint32, C.c_uint32, C.c_uint64, C.c_uint64, C.c_uint64,
                                          C.c_void_p, C.c_void_p]),
     "mmlst_xchg_await_dev": (C.c_int, [C.c_void_p, C.c_uint32, C.c_uint32, C.c_uint64, C.c_uint64, C.c_uint64, C.c_void_p, C.c_void_p,

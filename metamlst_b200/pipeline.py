@@ -38,6 +38,7 @@ class DevicePipeline:
         each rank finishes its own loci and ONE all-gather of the result blocks ends the pass (dist.merge_owner_blocks);
         "p2p" = owner mode with the all-gather done by our own kernels over NVLink peer memory (csrc/exchange.cu): the
         block is stored straight into every peer's symmetric buffer, no NCCL call inside the pass."""
+        api.refuse_lenient(streams)
         self.s = streams
         self._use_runs_arg, self._idx_base_arg = use_runs, idx_base
         self.index = index
@@ -148,6 +149,7 @@ class DevicePipeline:
         A captured CUDA graph is dropped (it holds the old streams' addresses)."""
         if list(streams.ref_names) != self.index.ref_names or not np.array_equal(np.asarray(streams.ref_lens), np.asarray(self.s.ref_lens)):
             raise ValueError("rebind: the sample was aligned against a different reference set")
+        api.refuse_lenient(streams)
         self.s = streams
         self.use_runs = getattr(streams, "run_tid", None) is not None if self._use_runs_arg is None else bool(self._use_runs_arg)
         self.use_qc = self.use_runs and getattr(streams, "chunk_qlen", None) is not None

@@ -318,7 +318,8 @@ def _local(fn):
 
 
 def ingest_steps(path: str, device, rank: int, world: int, locus_of=None, minqual: int = 20, max_depth: Optional[int] = 8000,
-                 presorted: bool = False, want_qhash: bool = True, sentinel_nodes: int = 1, check_crc: bool = False, halo_blocks: int = 1):
+                 presorted: bool = False, want_qhash: bool = True, sentinel_nodes: int = 1, check_crc: bool = False, halo_blocks: int = 1,
+                 lenient_tags: bool = False):
     """Generator of rank `rank`'s ingest (module text); returns its streams.DeviceStreams."""
     import torch
     from . import bam
@@ -513,7 +514,8 @@ def ingest_steps(path: str, device, rank: int, world: int, locus_of=None, minqua
     t0 = time.perf_counter()
 
     # ---- back half
-    o = bam.UnpackOpts(int(minqual), int(max_depth or 0), int(sentinel_nodes), 0, 1, 1 if presorted else 0, 1 if want_qhash else 0, 0, 0)
+    o = bam.UnpackOpts(int(minqual), int(max_depth or 0), int(sentinel_nodes), 0, 1, 1 if presorted else 0, 1 if want_qhash else 0, 0,
+                       1 if lenient_tags else 0)
     names_b = "\n".join(names).encode("latin-1")
     text_b = text.encode("latin-1")
     a = BackArgs(ref_len.ctypes.data if n_ref else None, names_b, text_b, n_ref, 1 if unsorted else 0)
@@ -535,7 +537,7 @@ def ingest_steps(path: str, device, rank: int, world: int, locus_of=None, minqua
     errs = yield ("gather", err)
     _agree(errs)
     secs["back"] = time.perf_counter() - t0
-    s = bam._dev_streams(keep, dev, want_qhash)
+    s = bam._dev_streams(keep, dev, want_qhash, lenient_tags)
     s.ingest_stats.update({"bgzf_blocks": own_blocks, "compressed_bytes": c1 - c0, "inflated_bytes": own_inflated})
     s.shard = {"rank": rank, "world": world, "records_parsed": n, "records_received": nrec, "file_index_base": base[rank],
                "bytes_sent": int(nbytes), "bytes_received": int(sum(recv_bytes)), "seconds": secs}
