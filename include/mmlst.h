@@ -113,13 +113,27 @@ int mmlst_score_runs_qc_dev(const uint32_t* run_tid, const uint32_t* run_start, 
                             uint64_t n_rec, uint64_t idx_base, const uint8_t* allow, uint32_t n_ref,
                             int minscore, int max_xm, int min_read_len,
                             int64_t* sum_as, uint32_t* n_hit, uint32_t* first_idx, uint64_t* counters, void* stream);
+/* Compact score stream of a resident run-length sample with len(SEQ) per chunk (device; the one definition of the format, see
+ * csrc/score_runs_kernels.cuh): code[n_rec] = one u16 per record, 0x8400 | (15 - min(xm3, 15)) << 11 | clamp(as0 - top_c + 1023, 0, 1023);
+ * head[ceil(n_rec/256)] = u16(top_c) | chunk_qlen[c] << 16, top_c = max as0 over chunk c.  as0 / code 16-byte aligned, xm3 8. */
+int mmlst_score_pack16_dev(const int16_t* as0, const uint8_t* xm3, const uint16_t* chunk_qlen, uint64_t n_rec, uint16_t* code,
+                           uint32_t* head, void* stream);
+/* mmlst_score_runs_qc_dev with the compact stream of mmlst_score_pack16_dev beside the resident as0 / xm3 (no file-order index): under
+ * form 7 it reads 2 B per record, and a chunk whose code 0 could pass (minscore <= top_c - 1023) from as0 / xm3; another form, max_xm >= 15
+ * or code / head NULL make it the 3-byte call.  Same tables as mmlst_score_runs_qc_dev in every case. */
+int mmlst_score_runs16_dev(const uint32_t* run_tid, const uint32_t* run_start, uint32_t n_runs, const uint32_t* chunk_run,
+                           const uint16_t* chunk_qlen, const int16_t* as0, const uint8_t* xm3, const uint16_t* code, const uint32_t* head,
+                           uint64_t n_rec, uint64_t idx_base, const uint8_t* allow, uint32_t n_ref,
+                           int minscore, int max_xm, int min_read_len,
+                           int64_t* sum_as, uint32_t* n_hit, uint32_t* first_idx, uint64_t* counters, void* stream);
 /* Kernel form used by mmlst_score_runs_dev / mmlst_score_runs_qc_dev (identical results): 0 = register-staged, 1 = register-
  * staged and software-pipelined, 2 = per-warp shared-memory ring filled by TMA bulk copies (records without orig_idx only;
  * other inputs take form 0), 3..5 = the ring with other stage sizes / depths (4 chunks x 3 stages, 8 x 2, 4 x 2),
- * 6 = form 5 with pairs of chunks reduced together (per-chunk len(SEQ) streams; others take form 5): the default since
- * round 2 (B200, configs[1]: 26.7 us against 28.8 us for form 5, profiles/r2a_bench_auto.json).  Returns the previous value; a value outside 0..6 only queries.  The environment variable
+ * 6 = form 5 with pairs of chunks reduced together (per-chunk len(SEQ) streams; others take form 5), 7 = form 6 over the compact
+ * 2 B / record stream of mmlst_score_pack16_dev, through mmlst_score_runs16_dev (the 3-byte entries take form 6 under it): the
+ * default (DESIGN.md section 4).  Returns the previous value; a value outside 0..7 only queries.  The environment variable
  * MMLST_SCORE_VARIANT presets it. */
-#define MMLST_SCORE_VARIANT_DEFAULT 6
+#define MMLST_SCORE_VARIANT_DEFAULT 7
 int mmlst_set_score_variant(int variant);
 /* Ring forms only: L2 residency hints (score stream evict-first; forms 2..5 also read run arrays, allow[] and chunk_qlen[] evict-last).  The stream
  * is read once per pass, so marking it evict-first leaves the L2 to what the REST of the pass reads -- the selection tables, the chosen contigs'

@@ -16,18 +16,20 @@
 
 // Which form of the run-length kernel a launch takes: 0 = registers, two chunks in flight per warp; 1 = registers,
 // software-pipelined (the next pair is requested before the current one is reduced); 2 = per-warp shared-memory ring fed
-// by TMA bulk copies (3..5: the same with other stage sizes / depths, see ring_config).  Same arithmetic, same results; MMLST_SCORE_VARIANT presets it, mmlst_set_score_variant changes it.
+// by TMA bulk copies (3..5: the same with other stage sizes / depths, see ring_config); 6 = form 5 with pairs of chunks reduced together; 7 = form 6
+// over the compact 2 B / record stream (mmlst_score_runs16_dev; the 3-byte entries take form 6 under it).  Same arithmetic, same results;
+// MMLST_SCORE_VARIANT presets it, mmlst_set_score_variant changes it.
 static int g_score_variant = -1;
 static int score_variant() {
     if (g_score_variant < 0) {
         const char* e = getenv("MMLST_SCORE_VARIANT");
-        g_score_variant = (e && e[0] >= '0' && e[0] <= '6' && !e[1]) ? e[0] - '0' : MMLST_SCORE_VARIANT_DEFAULT;
+        g_score_variant = (e && e[0] >= '0' && e[0] <= '7' && !e[1]) ? e[0] - '0' : MMLST_SCORE_VARIANT_DEFAULT;
     }
     return g_score_variant;
 }
 extern "C" int mmlst_set_score_variant(int v) {
     const int prev = score_variant();
-    if (v >= 0 && v <= 6) g_score_variant = v;
+    if (v >= 0 && v <= 7) g_score_variant = v;
     return prev;
 }
 
@@ -85,7 +87,7 @@ static int score_runs_launch(const uint32_t* run_tid, const uint32_t* run_start,
     const int variant = score_variant();
     const cudaStream_t st = static_cast<cudaStream_t>(stream);
     const bool tma_ok = !orig_idx && !(reinterpret_cast<uintptr_t>(xm3) & 15);  // cp.async.bulk wants 16-byte aligned sources
-    if (variant == 6 && tma_ok && chunk_qlen) {  // experimental: form 5's ring with pairs of chunks reduced together
+    if (variant >= 6 && tma_ok && chunk_qlen) {  // form 5's ring with pairs of chunks reduced together (form 7 without its compact stream)
         static int pair_resident_by_device[MMLST_MAX_DEVICES] = {0};
         int& pair_resident = pair_resident_by_device[mmlst_current_device()];
         const size_t smem = (kThreads / 32) * 2u * (4u * 768u + sizeof(uint64_t));
@@ -109,7 +111,7 @@ static int score_runs_launch(const uint32_t* run_tid, const uint32_t* run_start,
         int (&ring_resident)[4][8] = ring_resident_by_device[mmlst_current_device()];
         const int hint = a.l2_hints ? 1 : 0;
         const int q = (chunk_qlen ? 1 : 0) + 2 * hint;
-        const int rv = variant == 6 ? 5 : variant;  // form 6 exists for the per-chunk len(SEQ) stream only
+        const int rv = variant >= 6 ? 5 : variant;  // forms 6 and 7 exist for the per-chunk len(SEQ) stream only
         const RingCfg cfg = chunk_qlen ? (hint ? ring_config<true, true>(rv) : ring_config<true, false>(rv))
                                        : (hint ? ring_config<false, true>(rv) : ring_config<false, false>(rv));
         const size_t smem = (kThreads / 32) * static_cast<size_t>(cfg.ns) * (cfg.ch * (chunk_qlen ? 768u : 1280u) + sizeof(uint64_t));
@@ -164,6 +166,62 @@ extern "C" int mmlst_score_runs_qc_dev(const uint32_t* run_tid, const uint32_t* 
     if (n_rec && !chunk_qlen) { mmlst_set_error("mmlst_score_runs_qc_dev: null pointer"); return MMLST_E_ARG; }
     return score_runs_launch(run_tid, run_start, n_runs, chunk_run, as0, xm3, nullptr, chunk_qlen, orig_idx, n_rec, idx_base, allow, n_ref,
                              minscore, max_xm, min_read_len, sum_as, n_hit, first_idx, counters, stream);
+}
+
+// Form 7: the run-length stream with len(SEQ) per chunk, scored from its compact form (code[], head[] of mmlst_score_pack16_dev).  as0[] /
+// xm3[] stay resident: the chunks whose code 0 would be ambiguous (minscore <= top - 1023) and the partial last chunk are reduced from
+// them.  Another form selected, max_xm >= 15 (outside the 4-bit XM field) or no compact stream: the 3-byte call, same tables.
+extern "C" int mmlst_score_runs16_dev(const uint32_t* run_tid, const uint32_t* run_start, uint32_t n_runs, const uint32_t* chunk_run,
+                                      const uint16_t* chunk_qlen, const int16_t* as0, const uint8_t* xm3, const uint16_t* code, const uint32_t* head,
+                                      uint64_t n_rec, uint64_t idx_base, const uint8_t* allow, uint32_t n_ref, int minscore, int max_xm,
+                                      int min_read_len, int64_t* sum_as, uint32_t* n_hit, uint32_t* first_idx, uint64_t* counters, void* stream) {
+    if (n_rec && !chunk_qlen) { mmlst_set_error("mmlst_score_runs16_dev: null pointer"); return MMLST_E_ARG; }
+    const bool compact = code && head && !(reinterpret_cast<uintptr_t>(code) & 15) && !(reinterpret_cast<uintptr_t>(xm3) & 15);
+    if (score_variant() != 7 || !compact || max_xm >= 15 || n_rec < 256)
+        return score_runs_launch(run_tid, run_start, n_runs, chunk_run, as0, xm3, nullptr, chunk_qlen, nullptr, n_rec, idx_base, allow, n_ref,
+                                 minscore, max_xm, min_read_len, sum_as, n_hit, first_idx, counters, stream);
+    if (!run_tid || !run_start || !chunk_run || !n_runs || !as0 || !xm3 || !allow || !sum_as || !n_hit || !first_idx || !counters) {
+        mmlst_set_error("mmlst_score_runs16_dev: null pointer");
+        return MMLST_E_ARG;
+    }
+    if (n_rec >= 0xffffff00ull) { mmlst_set_error("mmlst_score_runs16_dev: %llu records do not fit 32-bit run offsets", (unsigned long long)n_rec); return MMLST_E_RANGE; }
+    if (reinterpret_cast<uintptr_t>(as0) & 15) { mmlst_set_error("mmlst_score_runs16_dev: as0 / xm3 / code must be 16-byte aligned"); return MMLST_E_ARG; }
+    RunArgs a{run_tid, run_start, chunk_run, n_runs, as0, xm3, nullptr, nullptr, chunk_qlen, n_rec, idx_base, allow, n_ref, minscore, max_xm,
+              min_read_len, reinterpret_cast<long long*>(sum_as), n_hit, first_idx, reinterpret_cast<unsigned long long*>(counters), score_l2_hints(),
+              code, head};
+    static int resident_by_device[MMLST_MAX_DEVICES] = {0};
+    int& resident = resident_by_device[mmlst_current_device()];
+    const size_t smem = (kThreads / 32) * 3u * (4u * 512u + sizeof(uint64_t));  // 3 stages of 4 chunks per warp
+    if (!resident) {
+        CUDA_TRY(cudaFuncSetAttribute(score_runs_ring_pair16_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, static_cast<int>(smem)));
+        CUDA_TRY(cudaFuncSetAttribute(score_runs_ring_pair16_kernel, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared));
+        int r = 0;
+        if (cudaOccupancyMaxActiveBlocksPerMultiprocessor(&r, score_runs_ring_pair16_kernel, kThreads, smem) != cudaSuccess || r < 1) r = 1;
+        resident = r;
+    }
+    uint64_t want = ((n_rec >> 8) + 15) / 16;  // CTAs if every warp took two chunks
+    const uint64_t cap = static_cast<uint64_t>(mmlst_num_sms()) * resident * score_grid8() / 8;
+    if (want > cap) want = cap;
+    if (want < 1) want = 1;
+    score_runs_ring_pair16_kernel<<<static_cast<unsigned>(want), kThreads, smem, static_cast<cudaStream_t>(stream)>>>(a);
+    CUDA_TRY(cudaGetLastError());
+    return MMLST_OK;
+}
+
+extern "C" int mmlst_score_pack16_dev(const int16_t* as0, const uint8_t* xm3, const uint16_t* chunk_qlen, uint64_t n_rec, uint16_t* code,
+                                      uint32_t* head, void* stream) {
+    if (n_rec == 0) return MMLST_OK;
+    if (!as0 || !xm3 || !chunk_qlen || !code || !head) { mmlst_set_error("mmlst_score_pack16_dev: null pointer"); return MMLST_E_ARG; }
+    if ((reinterpret_cast<uintptr_t>(as0) & 15) || (reinterpret_cast<uintptr_t>(xm3) & 7) || (reinterpret_cast<uintptr_t>(code) & 15)) {
+        mmlst_set_error("mmlst_score_pack16_dev: as0 / code must be 16-byte aligned, xm3 8");
+        return MMLST_E_ARG;
+    }
+    uint64_t blocks = (((n_rec + 255) >> 8) + 7) / 8;  // one warp per chunk
+    const uint64_t cap = static_cast<uint64_t>(mmlst_num_sms()) * 16;
+    if (blocks > cap) blocks = cap;
+    score_pack16_kernel<<<static_cast<unsigned>(blocks), 256, 0, static_cast<cudaStream_t>(stream)>>>(as0, xm3, chunk_qlen, n_rec, code, head);
+    CUDA_TRY(cudaGetLastError());
+    return MMLST_OK;
 }
 
 // qlen[i] of every record from the per-chunk form (the coverage kernel wants it per record)

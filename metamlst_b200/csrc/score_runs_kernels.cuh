@@ -17,6 +17,8 @@ struct RunArgs {
     int minscore, max_xm, min_read_len;
     long long* sum_as; uint32_t* n_hit; uint32_t* first_idx; unsigned long long* counters;
     int l2_hints;  // ring forms: streams evict-first, run tables / allow[] / chunk_qlen evict-last in the L2
+    const uint16_t* code;  // form 7: the compact stream of score_pack16_kernel (one word per record) ...
+    const uint32_t* head;  // ... and its per-chunk word (top AS | len(SEQ) << 16)
 };
 
 __device__ __forceinline__ void flush_run(const RunArgs& a, uint32_t key, long long s, uint32_t c, uint32_t mn) {
@@ -615,6 +617,293 @@ __global__ void __launch_bounds__(kThreads, 4) score_runs_ring_pair_kernel(const
     if (lane == 0 && tot) {
         atomicAdd(a.counters + 0, static_cast<unsigned long long>(tot));
         atomicAdd(a.counters + 1, static_cast<unsigned long long>(ign));
+    }
+}
+
+// ---- form 7: form 6 over the COMPACT score stream, 2 B per record instead of 3.  Only the as0 of a record that passes enters a
+// result, and the records of one 256-record chunk of a sorted sample lie within a few hundred AS of each other, so a record is
+// stored relative to its chunk's largest score.  score_pack16_kernel is the one definition of the format:
+//   head[c] = u16(top_c) | len(SEQ)_c << 16,  top_c = max as0 over chunk c,  base_c = top_c - 1023
+//   code[i] = 0x8400 | x' << 11 | a   (bit 15 and bit 10: guard bits, always 1)
+//     a  = clamp(as0 - base_c, 0, 1023): 1..1023 exact, 0 = "as0 <= base_c"
+//     x' = 15 - min(xm3, 15):            xm3 <= 14 exact, 0 = "xm3 >= 15"
+// Both filters are "field >= threshold", so one subtraction of T = A | (15 - max_xm) << 11 (A = minscore - base_c, per chunk)
+// tests both fields of both records of a 32-bit word: a field passes iff the guard bit above it survives.  A passing record's
+// as0 is base_c + a = minscore + (a - A), and a - A is what the subtraction leaves in bits 0..9: the sum over a lane's hits is
+// the sum of those fields plus minscore times the hit count, whatever the chunk.  The code is exact except where a = 0 can pass,
+// i.e. minscore <= base_c: such a chunk (decided per chunk, warp-uniformly) is reduced from the resident as0[] / xm3[] as form 6
+// does.  max_xm >= 15 never reaches this kernel (the launcher sends the call to form 6), max_xm < 0 puts 16 in the x' threshold
+// and min(A, 1024) = 1024 (minscore above top_c, or a chunk shorter than min_read_len) makes the c threshold fail every record.
+__device__ __forceinline__ uint32_t half_masks(uint32_t p) {  // 0xffff in each 16-bit half whose top bit is set
+#ifdef MMLST_HOST_EMUL
+    return ((p & 0x8000u) ? 0x0000ffffu : 0u) | ((p & 0x80000000u) ? 0xffff0000u : 0u);
+#else
+    uint32_t m;  // PRMT sign-replicate of bytes 1 and 3 (not __byte_perm: the intrinsic ignores the sign bit of each selector nibble)
+    asm("prmt.b32 %0, %1, 0, 0xbb99;" : "=r"(m) : "r"(p));
+    return m;
+#endif
+}
+
+// the lane's two records of word `w`: per half, 0xffff iff the record passes (m) and its a - A (v)
+__device__ __forceinline__ void pass16(uint32_t w, uint32_t T, uint32_t& m, uint32_t& v) {
+    const uint32_t d = w - T;  // no borrow leaves a field: every field of w is >= the matching field of T, guards included
+    m = half_masks(d & (d << 5));  // bit 10 (a >= A) moved onto bit 15 (x' >= 15 - max_xm)
+    v = d & m & 0x03ff03ffu;
+}
+
+// number of 0xffff halves in a sum of half masks (n_lo, n_hi <= 0x7fff): -sum = n_lo + (n_hi - n_lo) << 16 (mod 2^32)
+__device__ __forceinline__ uint32_t halves_set(uint32_t sm) {
+    const uint32_t u = 0u - sm;
+    return ((u & 0xffffu) * 2u + (u >> 16)) & 0xffffu;
+}
+
+// index of the lane's first passing record among its 8 (half masks of words 0..3), 0xffffffff if none
+__device__ __forceinline__ uint32_t first_pass16(const uint32_t m[4], uint32_t idx0) {
+    uint32_t b = 0;
+#pragma unroll
+    for (int j = 0; j < 4; ++j) b |= (m[j] & 0x00010001u) << (2 * j);  // record 2j at bit 2j, record 2j + 1 at bit 16 + 2j
+    b = (b & 0x55u) | ((b >> 15) & 0xaau);
+    return b ? idx0 + static_cast<uint32_t>(__ffs(b)) - 1u : 0xffffffffu;
+}
+
+// threshold word of chunk c for the compact stream; fb = the chunk has to be reduced from the 3-byte arrays
+__device__ __forceinline__ uint32_t chunk_thr16(uint32_t head, int ms, uint32_t tx, int min_read_len, bool& fb) {
+    int A = ms + 1023 - static_cast<int>(static_cast<int16_t>(head & 0xffffu));  // minscore - base_c
+    if (static_cast<int>(head >> 16) < min_read_len) A = 1024;                    // the whole chunk is too short
+    A = min(A, 1024);
+    fb = A <= 0;
+    return (static_cast<uint32_t>(A) | tx) * 0x00010001u;
+}
+
+// one compact chunk (lane: records base + 8 lane .. + 7 in q), run boundaries inside it allowed
+__device__ __forceinline__ void reduce_chunk16(const RunArgs& a, WarpRunPF& w, const uint4& q, uint32_t T, int ms, uint32_t base, uint32_t lane,
+                                               uint32_t& tot, uint32_t& ign) {
+    const uint32_t idx0 = static_cast<uint32_t>(a.idx_base) + base + (lane << 3);
+    const uint32_t wv[4] = {q.x, q.y, q.z, q.w};
+    uint32_t m[4], v[4];
+#pragma unroll
+    for (int j = 0; j < 4; ++j) pass16(wv[j], T, m[j], v[j]);
+    const uint32_t chunk_end = base + 256u;
+    if (chunk_end <= w.end) {  // the whole chunk lies inside the open run
+        if (w.al) {
+            const uint32_t acc = v[0] + v[1] + v[2] + v[3];
+            const uint32_t n = halves_set(m[0] + m[1] + m[2] + m[3]);
+            const int s = static_cast<int>((acc & 0xffffu) + (acc >> 16)) + ms * static_cast<int>(n);
+            tot += 8u;
+            ign += 8u - n;
+            w.s += __reduce_add_sync(FULL, s);
+            w.c += __reduce_add_sync(FULL, n);
+            if (w.mn == 0xffffffffu) w.mn = __reduce_min_sync(FULL, first_pass16(m, idx0));
+        }
+        if (chunk_end == w.end) next_run_pf<false>(a, w, lane, 0ull);
+        return;
+    }
+    const int lane0 = static_cast<int>(lane << 3);
+    uint32_t lo = base;
+    while (lo < chunk_end) {  // segment [lo, hi) of the chunk belongs to the open run
+        const uint32_t hi = min(w.end, chunk_end);
+        if (w.al) {
+            const int klo = min(max(static_cast<int>(lo - base) - lane0, 0), 8);
+            const int khi = min(max(static_cast<int>(hi - base) - lane0, 0), 8);
+            uint32_t mm[4], acc = 0, sm = 0;
+#pragma unroll
+            for (int j = 0; j < 4; ++j) {  // records 2j, 2j + 1 of the lane inside [klo, khi)
+                const uint32_t sel = ((2 * j >= klo && 2 * j < khi) ? 0x0000ffffu : 0u) | ((2 * j + 1 >= klo && 2 * j + 1 < khi) ? 0xffff0000u : 0u);
+                mm[j] = m[j] & sel;
+                acc += v[j] & sel;
+                sm += mm[j];
+            }
+            const uint32_t n = halves_set(sm);
+            const int s = static_cast<int>((acc & 0xffffu) + (acc >> 16)) + ms * static_cast<int>(n);
+            const uint32_t in = static_cast<uint32_t>(khi - klo);  // hi > lo, so khi >= klo
+            tot += in;
+            ign += in - n;
+            w.s += __reduce_add_sync(FULL, s);
+            w.c += __reduce_add_sync(FULL, n);
+            if (w.mn == 0xffffffffu) w.mn = __reduce_min_sync(FULL, first_pass16(mm, idx0));
+        }
+        if (hi == w.end) next_run_pf<false>(a, w, lane, 0ull);
+        lo = hi;
+    }
+}
+
+// two compact chunks, neither of which falls back
+__device__ __forceinline__ void reduce_pair16(const RunArgs& a, WarpRunPF& w, const uint4& qa, const uint4& qb, uint32_t Ta, uint32_t Tb, int ms,
+                                              uint32_t base, uint32_t lane, uint32_t& tot, uint32_t& ign) {
+    if (base + 512u > w.end) {  // a run ends inside the pair: chunk by chunk
+        reduce_chunk16(a, w, qa, Ta, ms, base, lane, tot, ign);
+        reduce_chunk16(a, w, qb, Tb, ms, base + 256u, lane, tot, ign);
+        return;
+    }
+    if (w.al) {
+        const uint32_t wa[4] = {qa.x, qa.y, qa.z, qa.w}, wb[4] = {qb.x, qb.y, qb.z, qb.w};
+        uint32_t ma[4], mb[4], va[4], vb[4];
+#pragma unroll
+        for (int j = 0; j < 4; ++j) { pass16(wa[j], Ta, ma[j], va[j]); pass16(wb[j], Tb, mb[j], vb[j]); }
+        const uint32_t acc = (va[0] + va[1] + va[2] + va[3]) + (vb[0] + vb[1] + vb[2] + vb[3]);  // <= 8 x 1022 per half
+        const uint32_t n = halves_set((ma[0] + ma[1] + ma[2] + ma[3]) + (mb[0] + mb[1] + mb[2] + mb[3]));
+        const int s = static_cast<int>((acc & 0xffffu) + (acc >> 16)) + ms * static_cast<int>(n);  // |s| <= 16 x 32768 per lane
+        tot += 16u;
+        ign += 16u - n;
+        w.s += __reduce_add_sync(FULL, s);
+        w.c += __reduce_add_sync(FULL, n);
+        if (w.mn == 0xffffffffu) {  // indices ascend inside a run: the first chunk's hits come first
+            const uint32_t idx0 = static_cast<uint32_t>(a.idx_base) + base + (lane << 3);
+            const uint32_t fa = first_pass16(ma, idx0);
+            w.mn = __reduce_min_sync(FULL, fa != 0xffffffffu ? fa : first_pass16(mb, idx0 + 256u));
+        }
+    }
+    if (base + 512u == w.end) next_run_pf<false>(a, w, lane, 0ull);
+}
+
+// a chunk whose code 0 would be ambiguous: form 6's chunk reduction over the resident 3-byte arrays
+__device__ __forceinline__ void reduce_chunk_fallback(const RunArgs& a, const Thr& thr, WarpRunPF& w, uint32_t head, uint32_t base, uint32_t lane,
+                                                      uint32_t& tot, uint32_t& ign) {
+    Loaded<false> L;
+    L.a8 = ld_stream_u4(a.as0 + base + (lane << 3));
+    L.x8 = ld_stream_u2(a.xm3 + base + (lane << 3));
+    L.q8 = make_uint4(0, 0, 0, 0);
+    L.cq = head >> 16;
+    reduce_chunk_pf<true, false>(a, thr, w, L, base, lane, tot, ign, 0ull);
+}
+
+__global__ void __launch_bounds__(kThreads, 4) score_runs_ring_pair16_kernel(const RunArgs a) {
+    pdl_launch_dependents();  // the selection kernel may take its (few) CTAs now; it waits for this grid to finish before it reads the tables
+    extern __shared__ __align__(128) uint8_t ring_raw[];
+    constexpr int NS = 3;
+    constexpr uint32_t CH = 4, CH_B = 512u, STAGE_B = CH * CH_B;
+    constexpr int NW = kThreads / 32;
+    const uint32_t lane = threadIdx.x & 31u, wid = threadIdx.x >> 5;
+    uint8_t* const my = ring_raw + wid * (NS * STAGE_B);
+    uint64_t* const bars = reinterpret_cast<uint64_t*>(ring_raw + NW * NS * STAGE_B) + wid * NS;
+    if (threadIdx.x == 0) {
+        uint64_t* all = reinterpret_cast<uint64_t*>(ring_raw + NW * NS * STAGE_B);
+        for (int i = 0; i < NW * NS; ++i) mbar_init(all + i, 1);
+        fence_mbar_init();
+    }
+    __syncthreads();
+
+    const uint64_t warp = (static_cast<uint64_t>(blockIdx.x) * blockDim.x + threadIdx.x) >> 5;
+    const uint64_t nwarps = (static_cast<uint64_t>(gridDim.x) * blockDim.x) >> 5;
+    const uint64_t nchunks = a.n_rec >> 8;
+    const uint64_t per = (nchunks + nwarps - 1) / nwarps;
+    const uint64_t c0 = warp * per;
+    const uint64_t c1 = (c0 + per < nchunks) ? c0 + per : nchunks;
+    uint32_t tot = 0, ign = 0;
+    const Thr thr = make_thr(a);
+    const int ms = min(max(a.minscore, -32768), 32768);                               // same filter on an int16 as0
+    const uint32_t tx = static_cast<uint32_t>(a.max_xm < 0 ? 16 : 15 - a.max_xm) << 11;  // 0 <= max_xm <= 14, or nothing passes
+
+    if (c0 < c1) {
+        const uint32_t ngroups = static_cast<uint32_t>((c1 - c0 + CH - 1) / CH);
+        auto issue = [&](uint32_t g, int stage) {  // lane 0: request group g (1..CH chunks) into `stage`
+            const uint64_t ch = c0 + static_cast<uint64_t>(g) * CH;
+            const uint32_t nch = (c1 - ch < CH) ? static_cast<uint32_t>(c1 - ch) : CH;
+            uint8_t* st = my + stage * STAGE_B;
+            mbar_expect_tx(bars + stage, nch * CH_B);
+            if (a.l2_hints) bulk_g2s_hint(st, a.code + (ch << 8), nch * CH_B, bars + stage, l2_policy(1));  // read once: evict-first
+            else bulk_g2s(st, a.code + (ch << 8), nch * CH_B, bars + stage);
+        };
+        if (lane == 0) {
+            const uint32_t pre = ngroups < static_cast<uint32_t>(NS) ? ngroups : static_cast<uint32_t>(NS);
+            for (uint32_t g = 0; g < pre; ++g) issue(g, static_cast<int>(g));
+        }
+        WarpRunPF w;
+        open_run_pf<false>(a, w, __ldg(a.chunk_run + c0), 0ull);
+        uint32_t phase = 0;
+        int stage = 0;
+        for (uint32_t g = 0; g < ngroups; ++g) {
+            const uint64_t ch = c0 + static_cast<uint64_t>(g) * CH;
+            const uint32_t nch = (c1 - ch < CH) ? static_cast<uint32_t>(c1 - ch) : CH;
+            mbar_wait(bars + stage, (phase >> stage) & 1u);
+            phase ^= 1u << stage;
+            const uint8_t* st = my + stage * STAGE_B;
+#pragma unroll
+            for (uint32_t k = 0; k < CH; k += 2) {
+                if (k < nch) {  // warp-uniform
+                    const bool two = k + 1u < nch;
+                    const uint32_t ha = __ldg(a.head + ch + k), hb = two ? __ldg(a.head + ch + k + 1u) : 0u;
+                    const uint4 qa = *reinterpret_cast<const uint4*>(st + k * CH_B + lane * 16u);
+                    const uint4 qb = two ? *reinterpret_cast<const uint4*>(st + (k + 1u) * CH_B + lane * 16u) : qa;
+                    if (k + 2u >= nch) {
+                        __syncwarp();  // every lane has the stage's last records in registers: the stage may be refilled
+                        if (lane == 0 && g + NS < ngroups) issue(g + NS, stage);
+                    }
+                    bool fa, fb;
+                    const uint32_t Ta = chunk_thr16(ha, ms, tx, a.min_read_len, fa), Tb = chunk_thr16(hb, ms, tx, a.min_read_len, fb);
+                    const uint32_t base = static_cast<uint32_t>((ch + k) << 8);
+                    if (two && !fa && !fb) {
+                        reduce_pair16(a, w, qa, qb, Ta, Tb, ms, base, lane, tot, ign);
+                    } else {
+                        if (fa) reduce_chunk_fallback(a, thr, w, ha, base, lane, tot, ign);
+                        else reduce_chunk16(a, w, qa, Ta, ms, base, lane, tot, ign);
+                        if (two) {
+                            if (fb) reduce_chunk_fallback(a, thr, w, hb, base + 256u, lane, tot, ign);
+                            else reduce_chunk16(a, w, qb, Tb, ms, base + 256u, lane, tot, ign);
+                        }
+                    }
+                }
+            }
+            stage = (stage + 1 == NS) ? 0 : stage + 1;
+        }
+        if (lane == 0 && w.al) flush_run(a, w.key, w.s, w.c, w.mn);
+    }
+
+    if (warp == nwarps - 1 && (a.n_rec & 255u)) score_tail<true>(a, nchunks, lane, tot, ign);
+    tot = __reduce_add_sync(FULL, tot);
+    ign = __reduce_add_sync(FULL, ign);
+    if (lane == 0 && tot) {
+        atomicAdd(a.counters + 0, static_cast<unsigned long long>(tot));
+        atomicAdd(a.counters + 1, static_cast<unsigned long long>(ign));
+    }
+}
+
+// the compact stream of form 7 (format above) from the resident 3-byte form: one warp per 256-record chunk, every chunk
+// including the partial last one (the kernel reduces that one from the 3-byte arrays)
+__global__ void __launch_bounds__(256) score_pack16_kernel(const int16_t* __restrict__ as0, const uint8_t* __restrict__ xm3,
+                                                           const uint16_t* __restrict__ chunk_qlen, uint64_t n_rec, uint16_t* __restrict__ code,
+                                                           uint32_t* __restrict__ head) {
+    const uint32_t lane = threadIdx.x & 31u;
+    const uint64_t nwarps = (static_cast<uint64_t>(gridDim.x) * blockDim.x) >> 5;
+    const uint64_t nch = (n_rec + 255u) >> 8;
+    for (uint64_t c = (static_cast<uint64_t>(blockIdx.x) * blockDim.x + threadIdx.x) >> 5; c < nch; c += nwarps) {
+        const uint64_t i0 = (c << 8) + (lane << 3);
+        const bool full = (c << 8) + 256u <= n_rec;  // warp-uniform
+        int as[8];
+        uint32_t xm[8];
+        if (full) {
+            const uint4 a8 = ld_stream_u4(as0 + i0);
+            const uint2 x8 = ld_stream_u2(xm3 + i0);
+            const uint32_t aw[4] = {a8.x, a8.y, a8.z, a8.w};
+#pragma unroll
+            for (int k = 0; k < 8; ++k) {
+                as[k] = static_cast<int16_t>((aw[k >> 1] >> (16 * (k & 1))) & 0xffffu);
+                xm[k] = ((k < 4 ? x8.x : x8.y) >> (8 * (k & 3))) & 0xffu;
+            }
+        } else {
+#pragma unroll
+            for (int k = 0; k < 8; ++k) {
+                const bool in = i0 + k < n_rec;
+                as[k] = in ? static_cast<int>(as0[i0 + k]) : -32768;  // outside the stream: raises no maximum, stored nowhere
+                xm[k] = in ? static_cast<uint32_t>(xm3[i0 + k]) : 255u;
+            }
+        }
+        int mx = as[0];
+#pragma unroll
+        for (int k = 1; k < 8; ++k) mx = max(mx, as[k]);
+        const int top = static_cast<int>(__reduce_max_sync(FULL, static_cast<uint32_t>(mx + 32768))) - 32768;
+        const int base = top - 1023;
+        uint32_t w16[8];
+#pragma unroll
+        for (int k = 0; k < 8; ++k) w16[k] = 0x8400u | ((15u - min(xm[k], 15u)) << 11) | static_cast<uint32_t>(max(as[k] - base, 0));
+        if (full) {
+            *reinterpret_cast<uint4*>(code + i0) = make_uint4(w16[0] | (w16[1] << 16), w16[2] | (w16[3] << 16), w16[4] | (w16[5] << 16), w16[6] | (w16[7] << 16));
+        } else {
+#pragma unroll
+            for (int k = 0; k < 8; ++k)
+                if (i0 + k < n_rec) code[i0 + k] = static_cast<uint16_t>(w16[k]);
+        }
+        if (lane == 0) head[c] = (static_cast<uint32_t>(top) & 0xffffu) | (static_cast<uint32_t>(__ldg(chunk_qlen + c)) << 16);
     }
 }
 

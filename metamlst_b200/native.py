@@ -100,6 +100,9 @@ EXPORTS = {
     "mmlst_chunk_qlen": (C.c_int, [C.c_void_p, C.c_uint64, C.c_void_p, C.POINTER(C.c_int)]),
     "mmlst_score_runs_qc_dev": (C.c_int, [C.c_void_p, C.c_void_p, C.c_uint32] + [C.c_void_p] * 5 + [C.c_uint64, C.c_uint64, C.c_void_p, C.c_uint32,
                                           C.c_int, C.c_int, C.c_int, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p]),
+    "mmlst_score_pack16_dev": (C.c_int, [C.c_void_p] * 3 + [C.c_uint64] + [C.c_void_p] * 3),
+    "mmlst_score_runs16_dev": (C.c_int, [C.c_void_p, C.c_void_p, C.c_uint32] + [C.c_void_p] * 6 + [C.c_uint64, C.c_uint64, C.c_void_p, C.c_uint32,
+                                         C.c_int, C.c_int, C.c_int, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p]),
     "mmlst_expand_chunk_qlen_dev": (C.c_int, [C.c_void_p, C.c_uint64, C.c_void_p, C.c_void_p]),
     "mmlst_inflate_raw": (C.c_int, [C.c_void_p, C.c_size_t, C.c_void_p, C.c_size_t, C.POINTER(C.c_size_t)]),
     "mmlst_set_score_variant": (C.c_int, [C.c_int]),

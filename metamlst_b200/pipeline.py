@@ -155,11 +155,37 @@ class DevicePipeline:
         self.use_qc = self.use_runs and getattr(streams, "chunk_qlen", None) is not None
         self.idx_base = int(self._idx_base_arg) if self._idx_base_arg else int(getattr(streams, "idx_base", 0) or 0)
         self.contig_start_d.copy_(torch.from_numpy(np.asarray(streams.contig_start, dtype=np.uint64).view(np.int64)), non_blocking=False)
+        self._pack16()
         need = int(streams.n_prec) // 512 + self.index.n_loci + 8
         if need > self.max_chunks:
             self.max_chunks = need
             self.chunks_d = torch.zeros(self.max_chunks * 8, dtype=torch.int32, device=self.dev)
         self.graph = None
+
+    def _pack16(self):
+        """The compact score stream (2 B / record, mmlst_score_pack16_dev) of a run-length sample with len(SEQ) per chunk and no
+        file-order index: code[] / head[] derived from the resident as0 / xm3 / chunk_qlen, which stay resident (the chunks the compact
+        code cannot decide, the partial last chunk, the coverage column and to_host() read them).  Derived again for every sample bound."""
+        s = self.s
+        self.code16 = self.head16 = None
+        n = int(s.as0.shape[0])
+        if not self.use_qc or getattr(s, "orig_idx", None) is not None or n == 0:
+            return
+        nch = (n + 255) // 256
+        self.code16 = torch.empty(nch * 256, dtype=torch.int16, device=self.dev)  # whole chunks: the kernel's bulk copies read 512 B per chunk
+        self.head16 = torch.empty(nch, dtype=torch.int32, device=self.dev)
+        native.check(self.lib.mmlst_score_pack16_dev(native.ptr(s.as0), native.ptr(s.xm3), native.ptr(s.chunk_qlen), n, native.ptr(self.code16),
+                                                     native.ptr(self.head16), self._stream()))
+
+    def compact_fallback_chunks(self) -> int:
+        """Full chunks of the bound sample that form 7 reduces from the 3-byte arrays at this pipeline's minscore (code 0, "as0 <= top - 1023",
+        could pass there); -1 without a compact stream."""
+        if self.code16 is None:
+            return -1
+        n = int(self.s.as0.shape[0])
+        top = (self.head16[: n // 256] & 0xFFFF).to(torch.int32)
+        top = top - ((top & 0x8000) << 1)  # u16 -> int16
+        return int((top - 1023 >= self.minscore).sum().item())
 
     def _timed(self, name: str, fn):
         if self.timers is None:
@@ -181,14 +207,20 @@ class DevicePipeline:
         self._clean = True
 
     def _score_call(self):
-        """Stage 1 over the resident score stream: the run-length form when the streams carry it (3 B / record with
-        len(SEQ) per chunk, else 5 B / record), else the explicit-tid form (9 B / record)."""
+        """Stage 1 over the resident score stream: the run-length form when the streams carry it (2 B / record compact or 3 B / record
+        with len(SEQ) per chunk, else 5 B / record), else the explicit-tid form (9 B / record)."""
         s = self.s
         n = int(s.as0.shape[0])
         oi = native.ptr(getattr(s, "orig_idx", None))  # file-order index per record (BAM that was not coordinate-sorted, locus shards); NULL = identity + idx_base
         if n == 0:
             return
-        if self.use_runs and self.use_qc:
+        if self.use_runs and self.use_qc and self.code16 is not None:  # the library picks form 7 or the 3-byte call (another form, max_xM >= 15)
+            native.check(self.lib.mmlst_score_runs16_dev(native.ptr(s.run_tid), native.ptr(s.run_start), int(s.run_tid.shape[0]), native.ptr(s.chunk_run),
+                                                         native.ptr(s.chunk_qlen), native.ptr(s.as0), native.ptr(s.xm3), native.ptr(self.code16),
+                                                         native.ptr(self.head16), n, self.idx_base, native.ptr(self.allow), self.n_ref, self.minscore,
+                                                         self.max_xM, self.min_read_len, native.ptr(self.sum_as), native.ptr(self.n_hit),
+                                                         native.ptr(self.first_idx), native.ptr(self.counters), self._stream()))
+        elif self.use_runs and self.use_qc:
             native.check(self.lib.mmlst_score_runs_qc_dev(native.ptr(s.run_tid), native.ptr(s.run_start), int(s.run_tid.shape[0]), native.ptr(s.chunk_run),
                                                           native.ptr(s.chunk_qlen), native.ptr(s.as0), native.ptr(s.xm3), oi, n, self.idx_base,
                                                           native.ptr(self.allow), self.n_ref, self.minscore, self.max_xM, self.min_read_len,
@@ -493,6 +525,8 @@ class DevicePipeline:
         keys = ["0", "1", "2", "3", "4", "5", "2h", "3h", "4h", "5h"]  # "h": ring form with the L2 residency hints
         if self.use_qc:
             keys += ["6", "6h", "6g10", "6g12"]  # pair-fused ring (per-chunk len(SEQ) streams only); gNN: grid of NN/8 resident waves
+        if self.code16 is not None:
+            keys += ["7", "7h"]  # form 6 over the compact 2 B / record stream
         grid0 = self.lib.mmlst_set_score_grid_scale(-1)
         for key in keys:
             v = int(key[0])
